@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark: Msamples/s segmented (threshold + SpeedyStatSplit).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c1|c2|c3|c4|c5]
+                    [--dump-outputs DIR]
 
 A step is one pass of the hot path (lambda_event_parser threshold scan + rule selection -> [Event.filter] ->
 SpeedyStatSplit prefix sums / split search -> segment table -> segment statistics) over one batch of synthetic
@@ -56,7 +57,7 @@ CONFIGS = {
     "c4": dict(kind="long", events=20, length=10_000_000, scaling="strong", steps=3,
                what="BASELINE configs[3]: long-event regime, 20 events of 10 M samples each (200 M samples), "
                     "SpeedyStatSplit(max_width=1e6)"),
-    "c5": dict(kind="batch", files=1000, scaling="strong", steps=2,
+    "c5": dict(kind="batch", files=1000, scaling="strong", steps=10,
                what="BASELINE configs[4]: batch of 1000 files of 2.49 M samples at 250 kHz (2.49 G samples), "
                     "Event.filter(order=1, cutoff=2000) + SpeedyStatSplit(prior_segments_per_second=10, "
                     "sampling_freq=2.5e5, cutoff_freq=2000) through Experiment.parse(batch=FileBatch)"),
@@ -329,6 +330,35 @@ def parity_rows(ev_rows, seg_rows, fixture, key, what):
         return {"error": "%s: %s" % (type(exc).__name__, exc)}
 
 
+DUMP_BYTES = 60_000_000     # --dump-outputs: array bytes in all, so that the files with their headers stay under 64 MB
+
+
+def device_tables(ctx, res):
+    """The event and segment tables a step left on the device, as a caller of the pipeline reads them, in float64
+    (row indices and sample positions are below 2**53: exact)."""
+    ev_start, ev_len = ctx.events(res["events"])
+    seg = ctx.segments(res["segments"])
+    tables = {"event": {"start": ev_start, "length": ev_len},
+              "segment": {k: seg[k] for k in ("event", "start", "end", "mean", "std", "min", "max")}}
+    return {t: {k: np.asarray(v, np.float64) for k, v in cols.items()} for t, cols in tables.items()}
+
+
+def dump_outputs(out_dir, tables):
+    """Writes column k of table t as out_dir/<t>_<k>.npy.  A table larger than its share of DUMP_BYTES is cut to a
+    fixed, seeded sample of its rows (the same rows for the same row count), whose indices go to <t>_row.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES
+    for i, (name, cols) in enumerate(tables.items()):
+        n = len(next(iter(cols.values())))
+        share = budget // (len(tables) - i)
+        if 8 * n * len(cols) > share:
+            rows = np.sort(np.random.default_rng(0).choice(n, share // (8 * (len(cols) + 1)), replace=False))
+            cols = dict({k: v[rows] for k, v in cols.items()}, row=rows.astype(np.float64))
+        for k, v in cols.items():
+            np.save(os.path.join(out_dir, "%s_%s.npy" % (name, k)), v)
+            budget -= v.nbytes
+
+
 def ncu_traffic(kernel="k3_split", metrics=("dram__bytes_read.sum", "dram__bytes_write.sum")):
     """dram__bytes_read.sum + dram__bytes_write.sum per launch of `kernel` from the newest committed `ncu --set full`
     capture of the default command (profiles/*_ncu_summary.csv), plus whether that capture is of THIS state of the
@@ -558,6 +588,7 @@ def run_trace(args):
     sampler.start()
     ms, res = timer.run(step_resident, args.steps, closing=closing)
     res = drain_resident() if shard is not None else res
+    dumped = device_tables(ctx, res) if args.dump_outputs else None
     launches = ctx.launch_count - launches0
     stage = ctx.stage_ms() if shard is None else dict(shard.stage_ms)
     counters = ctx.split_counters()
@@ -708,6 +739,8 @@ def run_trace(args):
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline_line(cfg)
         print(json.dumps(line), flush=True)
+    if dumped:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -802,6 +835,7 @@ def run_long(args):
     launches0 = ctx.launch_count
     sampler.start()
     ms, res = timer.run(lambda: step(False), args.steps)
+    dumped = device_tables(ctx, res) if args.dump_outputs else None
     launches = ctx.launch_count - launches0
     stage = ctx.stage_ms()
     counters = ctx.split_counters()
@@ -835,6 +869,8 @@ def run_long(args):
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline_line(cfg)
         print(json.dumps(line), flush=True)
+    if dumped:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -897,9 +933,9 @@ def run_batch(args):
     sampler = ClockSampler(local)
     sampler.start()
     launches0 = host.launch_count
-    r_steps = max(args.steps, 10)
-    ms_res, res = rtimer.run(step_resident, r_steps)
-    launches = (host.launch_count - launches0) * args.steps // r_steps
+    ms_res, res = rtimer.run(step_resident, args.steps)
+    dumped = device_tables(host, res) if args.dump_outputs else None
+    launches = host.launch_count - launches0
     stage = host.stage_ms()
     counters = host.split_counters()
     step_e2e()                                   # warm-up batch: every worker context's buffers grown
@@ -916,8 +952,8 @@ def run_batch(args):
         t_e2e = float(tt.item())
     if rank == 0:
         tb = exp.tables
-        value = len(resident) * world / (ms_res / 1e3 / r_steps) / 1e6
-        line = base_line(args, cfg, world, value, ms_res * args.steps / r_steps, n_total / (t_e2e / args.steps) / 1e6,
+        value = len(resident) * world / (ms_res / 1e3 / args.steps) / 1e6
+        line = base_line(args, cfg, world, value, ms_res, n_total / (t_e2e / args.steps) / 1e6,
                          4 * n_total, 56 * tb.n_segments + 48 * tb.n_events, launches, clocks)
         line["value_note"] = ("device-resident leg: one grouped pass of %d files (%d samples) per GPU, whole pipeline "
                               "incl. the Bessel filtfilt, CUDA events; e2e: the %d-file batch through "
@@ -938,6 +974,8 @@ def run_batch(args):
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline_line(cfg)
         print(json.dumps(line), flush=True)
+    if dumped:
+        dump_outputs(args.dump_outputs, dumped)
     batch.close()
     host.close()
     if world > 1:
@@ -962,9 +1000,17 @@ def main():
                     help="N > 1, end to end: equal chunks per GPU instead of chunks proportional to the measured upload rates")
     ap.add_argument("--split-kernel", default=None, choices=["flow", "level"],
                     help="development: force k3_flow / k3_split (default: the library's default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the event and segment tables of the last one as DIR/<name>.npy "
+                         "(float64; a fixed, seeded sample of the rows above 64 MB), to compare two builds output for "
+                         "output; one GPU and --impl ours only")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = CONFIGS[args.config]["steps"] if args.impl == "ours" else 3
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs needs --impl ours and --gpus 1")
     if args.impl == "reference":
         run_reference_arm(args)
     else:
