@@ -107,8 +107,24 @@ int pp_trace_upload(pp_ctx *ctx, const float *host, int64_t n, int64_t extra_cap
 /* Same for a float64 trace -- what the reference's own loader produces (PyPore/read_abf.py:208-210: int16 ADC counts
  * times a float64 scale factor).  The trace stays float64 on the device (8 B per sample): the threshold scan
  * compares the doubles themselves, run extrema are the doubles' own, and the later stages read the events out of
- * it like out of a float32 trace.  pp_trace_append / pp_trace_extend / the streamed host pipeline are float32-only. */
+ * it like out of a float32 trace.  pp_trace_append / pp_trace_extend are float32-only, and the streamed host pipeline
+ * takes float32 or int16 ADC input. */
 int pp_trace_upload_f64(pp_ctx *ctx, const double *host, int64_t n);
+/* Same for int16 ADC counts, 2 B per sample over the link and in the scan: every stage behaves as if it had been
+ * handed the float64 trace decode(c) = fl(fl(c * scale) + offset) (two roundings, no FMA: what NumPy computes for
+ * counts.astype(np.float64) * scale + offset).  The threshold scan compares integer keys (pp_adc16_key_threshold),
+ * the run extrema are decoded from the extreme keys, the later stages decode samples where they read them.
+ * PP_ERR_ARG unless scale is finite and non-zero, offset finite and every count decodes to a finite value.
+ * pp_trace_append / extend / prefetch / adopt and the pp_shard_* calls are float32-only: PP_ERR_STATE while an ADC
+ * trace is resident. */
+int pp_trace_upload_adc16(pp_ctx *ctx, const int16_t *host, int64_t n, double scale, double offset);
+/* PP_OK if (scale, offset) is a valid ADC decoding (see above), PP_ERR_ARG otherwise.  No context, no device. */
+int pp_adc16_check(double scale, double offset);
+/* The threshold scan's view of `current < threshold` for ADC counts: with kxor = -1 for a negative scale and 0
+ * otherwise, the decoded current is non-decreasing in the key k = c ^ kxor, and decode(c) < threshold holds exactly
+ * when k < *key (*key = 32768: for every count; -32768: for none, a NaN threshold included).  No context, no
+ * device; PP_ERR_ARG for an invalid decoding. */
+int pp_adc16_key_threshold(double scale, double offset, double threshold, int32_t *key, int32_t *kxor);
 /* Back-to-back traces: pp_trace_prefetch starts the copy of the NEXT float32 trace (ideally from page-locked memory)
  * into another device buffer on the context's copy stream and returns at once -- it runs under whatever the
  * context's stream is doing with the current trace; pp_trace_swap makes the oldest prefetched trace the resident one
@@ -254,6 +270,12 @@ typedef struct pp_host_tables {
 } pp_host_tables;
 int pp_pipeline_host_tables(pp_ctx *ctx, const float *host, int64_t n, int64_t chunk_samples,
                             const pp_pipeline_params *p, const pp_host_tables *tables, int64_t out[4]);
+/* pp_pipeline_host / pp_pipeline_host_tables (tables == NULL: device tables only) for int16 ADC counts decoded with
+ * `scale` and `offset` (pp_trace_upload_adc16): 2 B per sample over the link, same chunked copy / compute overlap,
+ * the same tables the float64 trace decode(counts) gives. */
+int pp_pipeline_host_adc16(pp_ctx *ctx, const int16_t *host, int64_t n, double scale, double offset,
+                           int64_t chunk_samples, const pp_pipeline_params *p,
+                           const pp_host_tables *tables /* NULL: device tables only */, int64_t out[4]);
 
 /* ---- multi-GPU: one context per rank, contiguous trace chunks (SURVEY 8e) -------------
  * The exchange itself (NCCL all-gathers of the records / tables, point-to-point halos) is

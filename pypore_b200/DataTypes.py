@@ -18,6 +18,7 @@ from functools import lru_cache
 import numpy as np
 
 from . import _lib, wire
+from .adc import AdcTrace
 from .core import MetaSegment, Segment
 from .parsers import SpeedyStatSplit, lambda_event_parser, parser, _run_pipeline, _upload_trace
 
@@ -179,7 +180,9 @@ class File(Segment):
     """A trace and the events detected in it (DataTypes.py:567-602).
 
     Only the ``current=`` / ``timestep=`` constructor is supported: there is no
-    .abf data offline and the ABF reader is out of scope.
+    .abf data offline and the ABF reader is out of scope.  ``current`` may be an ``AdcTrace`` (int16 counts with
+    their scale and offset): the parsers then work on the counts, and ``file.current`` is the decoded float64
+    current, built on first access.
     """
 
     def __init__(self, filename=None, current=None, timestep=None, **kwargs):
@@ -188,6 +191,26 @@ class File(Segment):
                 raise NotImplementedError("reading .abf files is out of scope; pass current= and timestep=")
             raise SyntaxError("Must provide current and timestep, or filename corresponding to a valid abf file.")
         super(File, self).__init__(current=current, filename="", second=1000. / timestep, events=[], sample=None)
+        if isinstance(current, AdcTrace):
+            self.__dict__["_adc"] = self.__dict__.pop("current")
+
+    def __getattr__(self, name):
+        # only reached when `current` is not set: the AdcTrace's decoding, once
+        adc = self.__dict__.get("_adc")
+        if name != "current" or adc is None:
+            raise AttributeError(name)
+        current = self.__dict__["current"] = adc.decode()
+        return current
+
+    def __setattr__(self, name, value):
+        if name == "current":
+            self.__dict__.pop("_adc", None)   # other samples than the counts
+        super(File, self).__setattr__(name, value)
+
+    def _samples(self):
+        """What the device parsers work on: the AdcTrace given as current=, else the current array."""
+        adc = self.__dict__.get("_adc")
+        return adc if adc is not None else np.asarray(self.current)
 
     __getitem__ = lambda self, index: self.events[index]     # noqa: E731
     n = property(lambda self: len(self.events))
@@ -211,8 +234,7 @@ class File(Segment):
             return
         if not isinstance(parser, lambda_event_parser):
             raise TypeError("the device-resident pipeline needs a pypore_b200 lambda_event_parser")
-        self._parse_resident(context or _lib.default_context(), np.asarray(self.current), parser, segmenter,
-                             filter_params)
+        self._parse_resident(context or _lib.default_context(), self._samples(), parser, segmenter, filter_params)
 
     # ------------------------------------------------------------------
     def _parse_resident(self, ctx, host, parser, segmenter, filter_params):
@@ -325,6 +347,7 @@ class File(Segment):
     def to_meta(self):
         """Drop the ionic current of the file and of everything under it (DataTypes.py:683-693)."""
         self.__dict__.pop("current", None)
+        self.__dict__.pop("_adc", None)
         if self._tables_current():
             self._tables.meta = True
             self._attach(self._tables)
@@ -362,7 +385,7 @@ class File(Segment):
         return f
 
     def delete(self):
-        for name in ("current", "event_parser", "_tables"):
+        for name in ("current", "_adc", "event_parser", "_tables"):
             self.__dict__.pop(name, None)
         if isinstance(self.events, _LazyList):
             self.events = []

@@ -9,6 +9,8 @@ import os
 
 import numpy as np
 
+from .adc import AdcTrace
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("PYPORE_B200_LIB") or os.path.join(HERE, "libpypore_b200.so")  # override: development variants only
 
@@ -71,6 +73,9 @@ SIGNATURES = {
     "pp_stage_ms": (_c.c_int, [_c.c_void_p, _c.c_int, _c.POINTER(_c.c_float)]),
     "pp_trace_upload": (_c.c_int, [_c.c_void_p, _c.c_void_p, _i64, _i64]),
     "pp_trace_upload_f64": (_c.c_int, [_c.c_void_p, _c.c_void_p, _i64]),
+    "pp_trace_upload_adc16": (_c.c_int, [_c.c_void_p, _c.c_void_p, _i64, _c.c_double, _c.c_double]),
+    "pp_adc16_check": (_c.c_int, [_c.c_double, _c.c_double]),
+    "pp_adc16_key_threshold": (_c.c_int, [_c.c_double, _c.c_double, _c.c_double, _i32p, _i32p]),
     "pp_trace_prefetch": (_c.c_int, [_c.c_void_p, _c.c_void_p, _i64, _i64]),
     "pp_trace_swap": (_c.c_int, [_c.c_void_p]),
     "pp_trace_adopt": (_c.c_int, [_c.c_void_p, _c.c_void_p, _i64, _i64]),
@@ -122,6 +127,8 @@ SIGNATURES = {
     "pp_pipeline_host": (_c.c_int, [_c.c_void_p, _f32p, _i64, _i64, _c.POINTER(PipelineParams), _i64p]),
     "pp_pipeline_host_tables": (_c.c_int, [_c.c_void_p, _f32p, _i64, _i64, _c.POINTER(PipelineParams),
                                            _c.POINTER(HostTables), _i64p]),
+    "pp_pipeline_host_adc16": (_c.c_int, [_c.c_void_p, _c.c_void_p, _i64, _c.c_double, _c.c_double, _i64,
+                                          _c.POINTER(PipelineParams), _c.POINTER(HostTables), _i64p]),
     "pp_pipeline": (_c.c_int, [_c.c_void_p, _c.POINTER(PipelineParams), _i64p]),
 }
 
@@ -251,6 +258,15 @@ class Context(object):
         self.sync()
         self._keep = []
         return x64.shape[0]
+
+    def upload_trace_adc16(self, trace):
+        """An AdcTrace, kept as int16 counts on the device (pp_trace_upload_adc16)."""
+        self._keep = [trace.counts]
+        self._ck(self._L.pp_trace_upload_adc16(self._h, trace.counts.ctypes.data, len(trace), trace.scale,
+                                               trace.offset))
+        self.sync()
+        self._keep = []
+        return len(trace)
 
     def upload_trace_any(self, x):
         """float32 arrays go up as they are, float64 ones as float32 when that loses nothing (half the bytes,
@@ -498,7 +514,7 @@ class Context(object):
     def pipeline(self, threshold, rule_mask, duration_gt, duration_lt, min_gt, max_lt, min_width,
                  max_width, window_width, min_gain, filter_ba=None, prefix_mode=PREFIX_AUTO,
                  with_stats=True, host_trace=None, chunk_samples=0, export=False):
-        """Whole pipeline on the resident trace, or -- with `host_trace` (float32, ideally pinned) --
+        """Whole pipeline on the resident trace, or -- with `host_trace` (float32 or an AdcTrace, ideally pinned) --
         streamed from host memory in chunks that overlap the copy with the computation.  With `export=True`
         the event and segment tables also arrive in page-locked host memory chunk by chunk (keys `event_table`,
         `segment_table` of the result: views of the context's pinned arena, valid until its next pinned use)."""
@@ -509,7 +525,9 @@ class Context(object):
         if host_trace is None:
             self._ck(self._L.pp_pipeline(self._h, _c.byref(p), _ptr(out, _i64p)))
         else:
-            x = np.ascontiguousarray(host_trace, np.float32)
+            adc = isinstance(host_trace, AdcTrace)
+            x = host_trace.counts if adc else np.ascontiguousarray(host_trace, np.float32)
+            t = None
             if export:
                 # upper bounds: an event is a run (>= 1 sample each, in practice far fewer); a segment is at least
                 # min_width samples unless it is a whole event
@@ -527,15 +545,20 @@ class Context(object):
                                                        views["end"].ctypes.data)
                 if with_stats:
                     t.mean, t.std, t.min, t.max = (views[k].ctypes.data for k in ("mean", "std", "min", "max"))
+            if adc:
+                r = self._L.pp_pipeline_host_adc16(self._h, x.ctypes.data, x.shape[0], host_trace.scale,
+                                                   host_trace.offset, int(chunk_samples), _c.byref(p),
+                                                   _c.byref(t) if t is not None else None, _ptr(out, _i64p))
+            elif export:
                 r = self._L.pp_pipeline_host_tables(self._h, _ptr(x, _f32p), x.shape[0], int(chunk_samples),
                                                     _c.byref(p), _c.byref(t), _ptr(out, _i64p))
-                if r == PP_ERR_CAPACITY and int(out[3]) > 0:
-                    views = None   # the host tables were too small: the device tables are complete, fetch them
-                else:
-                    self._ck(r)
             else:
-                self._ck(self._L.pp_pipeline_host(self._h, _ptr(x, _f32p), x.shape[0], int(chunk_samples),
-                                                  _c.byref(p), _ptr(out, _i64p)))
+                r = self._L.pp_pipeline_host(self._h, _ptr(x, _f32p), x.shape[0], int(chunk_samples),
+                                             _c.byref(p), _ptr(out, _i64p))
+            if export and r == PP_ERR_CAPACITY and int(out[3]) > 0:
+                views = None   # the host tables were too small: the device tables are complete, fetch them
+            else:
+                self._ck(r)
         del keep
         res = dict(runs=int(out[0]), events=int(out[1]), event_samples=int(out[2]), segments=int(out[3]))
         if export and host_trace is not None:

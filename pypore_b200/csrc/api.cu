@@ -42,7 +42,7 @@ struct pp_ctx {
     char err[512] = {0};
     int64_t launches = 0;
 
-    // trace: float32 (trace) or float64 (trace64) samples, one of the two
+    // trace: float32 (trace), float64 (trace64) or int16 ADC (trace16, decoded with adc) samples, one of the three
     DevBuf trace_buf;
     // pp_trace_prefetch: up to two float32 traces on their way up while the resident one is processed (oldest first);
     // trace_spare is the buffer the last swap retired
@@ -55,6 +55,8 @@ struct pp_ctx {
     DevBuf trace_spare;
     const float *trace = nullptr;
     const double *trace64 = nullptr;
+    const int16_t *trace16 = nullptr;
+    PPAdc adc = {1.0, 0.0};
     int64_t n = 0, trace_cap = 0;
     bool adopted = false;
 
@@ -198,11 +200,29 @@ PPSource make_source(pp_ctx *ctx)
     PPSource s;
     s.trace = ctx->trace;
     s.trace64 = ctx->trace64;
+    s.trace16 = ctx->trace16;
+    s.adc = ctx->adc;
     s.flat = (const double *)ctx->flat64.p;
     s.ev_start = (const int64_t *)ctx->ev_start.p;
     s.ev_off = (const int64_t *)ctx->ev_off.p;
     s.kind = ctx->src_kind;
     return s;
+}
+
+bool has_trace(const pp_ctx *ctx) { return ctx->trace || ctx->trace64 || ctx->trace16; }
+
+// event source of events that are views of the resident trace
+int trace_kind(const pp_ctx *ctx)
+{
+    return ctx->trace64 ? PP_SRC_TRACE64 : ctx->trace16 ? PP_SRC_ADC16 : PP_SRC_TRACE32;
+}
+
+// the resident trace is the buffer `p` of `elem`-byte samples (4: float32, 8: float64, 2: int16 ADC counts)
+void point_trace(pp_ctx *ctx, void *p, size_t elem)
+{
+    ctx->trace = elem == sizeof(float) ? (const float *)p : nullptr;
+    ctx->trace64 = elem == sizeof(double) ? (const double *)p : nullptr;
+    ctx->trace16 = elem == sizeof(int16_t) ? (const int16_t *)p : nullptr;
 }
 
 // float64 samples of the current events and the table that locates an event in them
@@ -276,7 +296,8 @@ int begin_threshold(pp_ctx *ctx, int64_t scan_len)
 }
 
 template <typename T>
-int launch_threshold_tiles(pp_ctx *ctx, const T *x, T thr, int64_t upto, int64_t tile_begin, int64_t ntiles)
+int launch_threshold_tiles(pp_ctx *ctx, const T *x, typename K1Key<T>::V thr, int kxor, int64_t upto,
+                           int64_t tile_begin, int64_t ntiles)
 {
     const size_t smem = sizeof(K1Smem<T>);
     static int per_sm = 0;   // per instantiation: resident CTAs per SM (the kernel is persistent: one wave exactly)
@@ -289,13 +310,13 @@ int launch_threshold_tiles(pp_ctx *ctx, const T *x, T thr, int64_t upto, int64_t
     int64_t grid = (int64_t)ctx->sm_count * per_sm;
     if (grid > ntiles) grid = ntiles;
     k1_scan_tiles<T><<<(unsigned)grid, K1_CTA_THREADS, smem, ctx->stream>>>(
-        x, upto, thr, tile_begin, ntiles, (K1Record *)ctx->k1_rec.p, (K1Staged *)ctx->k1_staged.p);
+        x, upto, thr, kxor, tile_begin, ntiles, (K1Record *)ctx->k1_rec.p, (K1Staged *)ctx->k1_staged.p);
     LAUNCHED(ctx);
     const int64_t rec_begin = tile_begin * K1_WARPS, rec_end = (tile_begin + ntiles) * K1_WARPS;
     const int64_t nblk = (rec_end - rec_begin + K1B_THREADS - 1) / K1B_THREADS;
     CK(cudaMemsetAsync(ctx->k1_blk.p, 0, sizeof(unsigned long long) * nblk, ctx->stream));
     k1_stitch<T><<<(unsigned)nblk, K1B_THREADS, 0, ctx->stream>>>(
-        x, upto, thr, rec_begin, rec_end, (const K1Record *)ctx->k1_rec.p, (const K1Staged *)ctx->k1_staged.p,
+        x, upto, thr, kxor, rec_begin, rec_end, (const K1Record *)ctx->k1_rec.p, (const K1Staged *)ctx->k1_staged.p,
         (unsigned long long *)ctx->k1_blk.p, ctx->ctr, ctx->k1_flip, (int64_t *)ctx->run_start.p,
         (unsigned long long *)ctx->run_minkey.p, (unsigned long long *)ctx->run_maxkey.p, ctx->cap_runs);
     LAUNCHED(ctx);
@@ -310,26 +331,31 @@ int enqueue_threshold_tiles(pp_ctx *ctx, double threshold, int64_t upto, int64_t
     StageRange nvtx_range("pypore:threshold");
     if (ntiles > 0) {
         if (ctx->trace64) {
-            CKR(launch_threshold_tiles<double>(ctx, ctx->trace64, threshold, upto, ctx->k1_tiles_done, ntiles));
+            CKR(launch_threshold_tiles<double>(ctx, ctx->trace64, threshold, 0, upto, ctx->k1_tiles_done, ntiles));
+        } else if (ctx->trace16) {
+            int32_t key = 0, kxor = 0;
+            pp_adc16_key_threshold(ctx->adc.scale, ctx->adc.offset, threshold, &key, &kxor);
+            CKR(launch_threshold_tiles<int16_t>(ctx, ctx->trace16, key, kxor, upto, ctx->k1_tiles_done, ntiles));
         } else {
             // smallest float32 >= threshold: double(x) < thr  <=>  x < thr_up for every float32 x
             float thr_f = (float)threshold;
             if ((double)thr_f < threshold) thr_f = nextafterf(thr_f, INFINITY);
-            CKR(launch_threshold_tiles<float>(ctx, ctx->trace, thr_f, upto, ctx->k1_tiles_done, ntiles));
+            CKR(launch_threshold_tiles<float>(ctx, ctx->trace, thr_f, 0, upto, ctx->k1_tiles_done, ntiles));
         }
         ctx->k1_tiles_done += ntiles;
     }
     k1_finalize_runs<<<ctx->sm_count, 256, 0, ctx->stream>>>(
         upto, ctx->ctr, (const int64_t *)ctx->run_start.p, (const unsigned long long *)ctx->run_minkey.p,
         (const unsigned long long *)ctx->run_maxkey.p, ctx->cap_runs, (int64_t *)ctx->run_len.p,
-        (double *)ctx->run_min.p, (double *)ctx->run_max.p, (unsigned char *)ctx->run_below.p);
+        (double *)ctx->run_min.p, (double *)ctx->run_max.p, (unsigned char *)ctx->run_below.p,
+        ctx->trace16 != nullptr, ctx->adc);
     LAUNCHED(ctx);
     return PP_OK;
 }
 
 int enqueue_threshold(pp_ctx *ctx, double threshold, int64_t scan_len)
 {
-    if ((!ctx->trace && !ctx->trace64) || ctx->n <= 0) return fail(ctx, PP_ERR_STATE, "no trace resident");
+    if (!has_trace(ctx) || ctx->n <= 0) return fail(ctx, PP_ERR_STATE, "no trace resident");
     if (scan_len < 0 || scan_len > ctx->n) scan_len = ctx->n;
     CKR(begin_threshold(ctx, scan_len));
     return enqueue_threshold_tiles(ctx, threshold, scan_len, (scan_len + K1_TILE - 1) / K1_TILE);
@@ -340,7 +366,7 @@ int enqueue_select(pp_ctx *ctx, int rule_mask, int64_t duration_gt, int64_t dura
                    const long long *dev_plan = nullptr)
 {
     StageRange nvtx_range("pypore:select");
-    ctx->src_kind = ctx->trace64 ? PP_SRC_TRACE64 : PP_SRC_TRACE32;
+    ctx->src_kind = trace_kind(ctx);
     ctx->flat_cap = ctx->n;
     k1_select_events<<<1, SEL_THREADS, 0, ctx->stream>>>(
         ctx->ctr, (const int64_t *)ctx->run_start.p, (const int64_t *)ctx->run_len.p,
@@ -458,6 +484,33 @@ int prepare_split(pp_ctx *ctx, int mw, int MW, int W)
     return PP_OK;
 }
 
+// K2's tiled scan with the exactness proof over the samples `samples` of the event source `src`
+template <typename T>
+int enqueue_prefix_tiled(pp_ctx *ctx, const PPSource &src, const T *samples, int prefix_mode)
+{
+    // short events: one pass, one warp per event
+    k2_event_scan<T><<<ctx->sm_count * K2F_CFG_CTAS * 2, K2F_WARPS * 32, 0, ctx->stream>>>(
+        src, samples, (const int64_t *)ctx->ev_len.p, ctx->ctr, (unsigned *)ctx->inexact.p, (double2 *)ctx->cc.p,
+        prefix_mode != PP_PREFIX_PARALLEL);
+    LAUNCHED(ctx);
+    // long events: multi-CTA reduce / carries / scan over their tiles
+    const int grid = ctx->sm_count * 8;
+    k2_tile_reduce<T><<<grid, K2_THREADS, 0, ctx->stream>>>(
+        src, samples, (const int64_t *)ctx->ev_len.p, (const int64_t *)ctx->ev_tile_off.p, ctx->ctr,
+        (K2TileState *)ctx->k2_tiles.p, (K2EventBits *)ctx->k2_bits.p);
+    LAUNCHED(ctx);
+    k2_event_carries<<<ctx->sm_count * 2, 256, 0, ctx->stream>>>(
+        ctx->ctr, (const int64_t *)ctx->ev_len.p, (const int64_t *)ctx->ev_tile_off.p,
+        (K2TileState *)ctx->k2_tiles.p, (const K2EventBits *)ctx->k2_bits.p, (unsigned *)ctx->inexact.p,
+        prefix_mode != PP_PREFIX_PARALLEL);
+    LAUNCHED(ctx);
+    k2_tile_scan<T><<<grid, K2_THREADS, 0, ctx->stream>>>(
+        src, samples, (const int64_t *)ctx->ev_len.p, (const int64_t *)ctx->ev_tile_off.p, ctx->ctr,
+        (const K2TileState *)ctx->k2_tiles.p, (double2 *)ctx->cc.p);
+    LAUNCHED(ctx);
+    return PP_OK;
+}
+
 // K2 over the events [ev_begin, n_events) (device-side range)
 int enqueue_prefix(pp_ctx *ctx, int prefix_mode)
 {
@@ -478,43 +531,9 @@ int enqueue_prefix(pp_ctx *ctx, int prefix_mode)
                                                      (int64_t *)ctx->ev_tile_off.p, (K2EventBits *)ctx->k2_bits.p,
                                                      (unsigned *)ctx->inexact.p);
         LAUNCHED(ctx);
-        // short events: one pass, one warp per event
-        if (ctx->src_kind == PP_SRC_TRACE32)
-            k2_event_scan<float><<<ctx->sm_count * K2F_CFG_CTAS * 2, K2F_WARPS * 32, 0, ctx->stream>>>(
-                src, ctx->trace, (const int64_t *)ctx->ev_len.p, ctx->ctr, (unsigned *)ctx->inexact.p,
-                (double2 *)ctx->cc.p, prefix_mode != PP_PREFIX_PARALLEL);
-        else
-            k2_event_scan<double><<<ctx->sm_count * K2F_CFG_CTAS * 2, K2F_WARPS * 32, 0, ctx->stream>>>(
-                src, f64_samples(ctx), (const int64_t *)ctx->ev_len.p, ctx->ctr,
-                (unsigned *)ctx->inexact.p, (double2 *)ctx->cc.p, prefix_mode != PP_PREFIX_PARALLEL);
-        LAUNCHED(ctx);
-        // long events: multi-CTA reduce / carries / scan over their tiles
-        const int grid = ctx->sm_count * 8;
-        if (ctx->src_kind == PP_SRC_TRACE32)
-            k2_tile_reduce<float><<<grid, K2_THREADS, 0, ctx->stream>>>(
-                src, ctx->trace, (const int64_t *)ctx->ev_len.p, (const int64_t *)ctx->ev_tile_off.p, ctx->ctr,
-                (K2TileState *)ctx->k2_tiles.p, (K2EventBits *)ctx->k2_bits.p);
-        else
-            k2_tile_reduce<double><<<grid, K2_THREADS, 0, ctx->stream>>>(
-                src, f64_samples(ctx), (const int64_t *)ctx->ev_len.p,
-                (const int64_t *)ctx->ev_tile_off.p, ctx->ctr, (K2TileState *)ctx->k2_tiles.p,
-                (K2EventBits *)ctx->k2_bits.p);
-        LAUNCHED(ctx);
-        k2_event_carries<<<ctx->sm_count * 2, 256, 0, ctx->stream>>>(
-            ctx->ctr, (const int64_t *)ctx->ev_len.p, (const int64_t *)ctx->ev_tile_off.p,
-            (K2TileState *)ctx->k2_tiles.p, (const K2EventBits *)ctx->k2_bits.p, (unsigned *)ctx->inexact.p,
-            prefix_mode != PP_PREFIX_PARALLEL);
-        LAUNCHED(ctx);
-        if (ctx->src_kind == PP_SRC_TRACE32)
-            k2_tile_scan<float><<<grid, K2_THREADS, 0, ctx->stream>>>(
-                src, ctx->trace, (const int64_t *)ctx->ev_len.p, (const int64_t *)ctx->ev_tile_off.p, ctx->ctr,
-                (const K2TileState *)ctx->k2_tiles.p, (double2 *)ctx->cc.p);
-        else
-            k2_tile_scan<double><<<grid, K2_THREADS, 0, ctx->stream>>>(
-                src, f64_samples(ctx), (const int64_t *)ctx->ev_len.p,
-                (const int64_t *)ctx->ev_tile_off.p, ctx->ctr, (const K2TileState *)ctx->k2_tiles.p,
-                (double2 *)ctx->cc.p);
-        LAUNCHED(ctx);
+        if (ctx->src_kind == PP_SRC_TRACE32) CKR(enqueue_prefix_tiled<float>(ctx, src, ctx->trace, prefix_mode));
+        else if (ctx->src_kind == PP_SRC_ADC16) CKR(enqueue_prefix_tiled<int16_t>(ctx, src, ctx->trace16, prefix_mode));
+        else CKR(enqueue_prefix_tiled<double>(ctx, src, f64_samples(ctx), prefix_mode));
         if (prefix_mode != PP_PREFIX_PARALLEL) {
             k2_prefix_sequential<<<ctx->sm_count * 3, K2S_WARPS * 32, 0, ctx->stream>>>(
                 src, (const int64_t *)ctx->ev_len.p, ctx->ctr, (const unsigned *)ctx->inexact.p,
@@ -630,22 +649,35 @@ int enqueue_split(pp_ctx *ctx, int mw, int MW, int W, double min_gain, int prefi
     return PP_OK;
 }
 
+// K4 over the rows of the current event source: segments (flat_start = seg_flat, row_event = seg_event) or whole
+// events (rows_are_events, flat_start = ev_off, row_event = nullptr)
+int launch_stats(pp_ctx *ctx, int rows_are_events, const int64_t *flat_start, const int *row_event, int64_t cap_rows,
+                 double *mean, double *sd, double *mn, double *mx)
+{
+    const unsigned grid = ctx->sm_count * 8;
+    const int64_t *ev_off = (const int64_t *)ctx->ev_off.p;
+    if (ctx->src_kind == PP_SRC_TRACE32)
+        k4_segment_stats<float><<<grid, 256, 0, ctx->stream>>>(
+            ctx->trace, (const int64_t *)ctx->ev_start.p, ev_off, ctx->ctr, rows_are_events, flat_start, row_event,
+            cap_rows, mean, sd, mn, mx, ctx->adc);
+    else if (ctx->src_kind == PP_SRC_ADC16)
+        k4_segment_stats<int16_t><<<grid, 256, 0, ctx->stream>>>(
+            ctx->trace16, (const int64_t *)ctx->ev_start.p, ev_off, ctx->ctr, rows_are_events, flat_start, row_event,
+            cap_rows, mean, sd, mn, mx, ctx->adc);
+    else
+        k4_segment_stats<double><<<grid, 256, 0, ctx->stream>>>(
+            f64_samples(ctx), f64_bases(ctx), ev_off, ctx->ctr, rows_are_events, flat_start, row_event, cap_rows,
+            mean, sd, mn, mx, ctx->adc);
+    LAUNCHED(ctx);
+    return PP_OK;
+}
+
 int enqueue_stats(pp_ctx *ctx)
 {
     StageRange nvtx_range("pypore:stats");
-    if (ctx->src_kind == PP_SRC_TRACE32)
-        k4_segment_stats<float><<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(
-            ctx->trace, (const int64_t *)ctx->ev_start.p, (const int64_t *)ctx->ev_off.p, ctx->ctr, 0,
-            (const int64_t *)ctx->seg_flat.p, (const int *)ctx->seg_event.p, ctx->cap_segs,
-            (double *)ctx->seg_mean.p, (double *)ctx->seg_std.p, (double *)ctx->seg_min.p,
-            (double *)ctx->seg_max.p);
-    else
-        k4_segment_stats<double><<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(
-            f64_samples(ctx), f64_bases(ctx), (const int64_t *)ctx->ev_off.p,
-            ctx->ctr, 0, (const int64_t *)ctx->seg_flat.p, (const int *)ctx->seg_event.p, ctx->cap_segs,
-            (double *)ctx->seg_mean.p, (double *)ctx->seg_std.p, (double *)ctx->seg_min.p,
-            (double *)ctx->seg_max.p);
-    LAUNCHED(ctx);
+    CKR(launch_stats(ctx, 0, (const int64_t *)ctx->seg_flat.p, (const int *)ctx->seg_event.p, ctx->cap_segs,
+                     (double *)ctx->seg_mean.p, (double *)ctx->seg_std.p, (double *)ctx->seg_min.p,
+                     (double *)ctx->seg_max.p));
     CKR(record_boundary(ctx, ST_STATS + 1));
     ctx->stage_ran[ST_STATS] = true;
     ctx->stats_valid = true;
@@ -824,8 +856,7 @@ static int trace_upload_impl(pp_ctx *ctx, const void *host, int64_t n, int64_t e
     CKR(set_device(ctx));
     CKR(ensure(ctx, ctx->trace_buf, elem * (size_t)(n + extra_capacity)));
     CK(cudaMemcpyAsync(ctx->trace_buf.p, host, elem * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-    ctx->trace = elem == sizeof(float) ? (const float *)ctx->trace_buf.p : nullptr;
-    ctx->trace64 = elem == sizeof(double) ? (const double *)ctx->trace_buf.p : nullptr;
+    point_trace(ctx, ctx->trace_buf.p, elem);
     ctx->n = n;
     ctx->trace_cap = (int64_t)(ctx->trace_buf.cap / elem);
     ctx->adopted = false;
@@ -844,6 +875,48 @@ int pp_trace_upload_f64(pp_ctx *ctx, const double *host, int64_t n)
     return trace_upload_impl(ctx, host, n, 0, sizeof(double));
 }
 
+// decode(c) on the host: the product is rounded on its own (no contraction into an FMA), like the device's
+static double adc_decode_host(int c, double scale, double offset)
+{
+    volatile double prod = (double)c * scale;
+    return prod + offset;
+}
+
+int pp_adc16_check(double scale, double offset)
+{
+    if (!isfinite(scale) || scale == 0.0 || !isfinite(offset)) return PP_ERR_ARG;
+    // decode is monotone in c: every count decodes to a finite value iff both ends do
+    if (!isfinite(adc_decode_host(-32768, scale, offset)) || !isfinite(adc_decode_host(32767, scale, offset)))
+        return PP_ERR_ARG;
+    return PP_OK;
+}
+
+int pp_adc16_key_threshold(double scale, double offset, double threshold, int32_t *key, int32_t *kxor)
+{
+    if (!key || !kxor || pp_adc16_check(scale, offset) != PP_OK) return PP_ERR_ARG;
+    // decode(k ^ kx) is non-decreasing in the key k, so `!(decode < threshold)` is false, then true over the 65,536
+    // keys (true throughout for a NaN threshold): find the first key where it holds, 32768 if none does
+    const int kx = scale < 0.0 ? -1 : 0;
+    int lo = -32768, hi = 32768;
+    while (lo < hi) {
+        const int mid = lo + ((hi - lo) >> 1);
+        if (!(adc_decode_host(mid ^ kx, scale, offset) < threshold)) hi = mid;
+        else lo = mid + 1;
+    }
+    *key = lo;
+    *kxor = kx;
+    return PP_OK;
+}
+
+int pp_trace_upload_adc16(pp_ctx *ctx, const int16_t *host, int64_t n, double scale, double offset)
+{
+    if (pp_adc16_check(scale, offset) != PP_OK)
+        return fail(ctx, PP_ERR_ARG, "ADC scale must be finite and non-zero, offset finite, every count decoding finite");
+    CKR(trace_upload_impl(ctx, host, n, 0, sizeof(int16_t)));
+    ctx->adc = PPAdc{scale, offset};
+    return PP_OK;
+}
+
 // ---- double-buffered upload (back-to-back traces: the copy of trace i+1 runs under the kernels of trace i) ----
 static int ensure_copy_stream(pp_ctx *ctx)
 {
@@ -858,6 +931,7 @@ static int ensure_copy_stream(pp_ctx *ctx)
 int pp_trace_prefetch(pp_ctx *ctx, const float *host, int64_t n, int64_t extra_capacity)
 {
     if (!ctx || !host || n <= 0 || extra_capacity < 0) return fail(ctx, PP_ERR_ARG, "bad trace");
+    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "prefetch takes float32 traces; an ADC trace is resident");
     if (ctx->n_pend >= 2) return fail(ctx, PP_ERR_STATE, "two prefetched traces are already waiting for pp_trace_swap");
     CKR(set_device(ctx));
     CKR(ensure_copy_stream(ctx));
@@ -911,8 +985,7 @@ int pp_trace_swap(pp_ctx *ctx)
     ctx->pf_t0 = q.t0; ctx->pf_t1 = q.t1;
     q.t0 = a; q.t1 = b;
     if (!q.t0) { CK(cudaEventCreate(&q.t0)); CK(cudaEventCreate(&q.t1)); }
-    ctx->trace = (const float *)ctx->trace_buf.p;
-    ctx->trace64 = nullptr;
+    point_trace(ctx, ctx->trace_buf.p, sizeof(float));
     ctx->n = q.n;
     q.n = -1;
     if (ctx->n_pend == 2) {       // the younger one moves up
@@ -932,8 +1005,8 @@ int pp_trace_adopt(pp_ctx *ctx, const float *dev, int64_t n, int64_t capacity)
 {
     if (!ctx || !dev || n <= 0 || capacity < n) return fail(ctx, PP_ERR_ARG, "bad trace");
     if (((uintptr_t)dev) & 15) return fail(ctx, PP_ERR_ARG, "device trace must be 16-byte aligned");
-    ctx->trace = dev;
-    ctx->trace64 = nullptr;
+    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "adopt takes float32 traces; an ADC trace is resident");
+    point_trace(ctx, (void *)dev, sizeof(float));
     ctx->n = n;
     ctx->trace_cap = capacity;
     ctx->adopted = true;
@@ -1053,7 +1126,7 @@ int pp_set_events(pp_ctx *ctx, const int64_t *start, const int64_t *length, int6
 {
     if (!ctx || n_events < 0 || (n_events > 0 && (!start || !length)))
         return fail(ctx, PP_ERR_ARG, "bad events");
-    if (!ctx->trace && !ctx->trace64) return fail(ctx, PP_ERR_STATE, "no trace resident");
+    if (!has_trace(ctx)) return fail(ctx, PP_ERR_STATE, "no trace resident");
     CKR(set_device(ctx));
     for (int64_t i = 0; i < n_events; ++i)
         if (start[i] < 0 || length[i] <= 0 || start[i] + length[i] > ctx->n)
@@ -1066,7 +1139,7 @@ int pp_set_events(pp_ctx *ctx, const int64_t *start, const int64_t *length, int6
     k1_event_offsets<<<1, SEL_THREADS, 0, ctx->stream>>>(ctx->ctr, (const int64_t *)ctx->ev_len.p, n_events,
                                                          (int64_t *)ctx->ev_off.p);
     LAUNCHED(ctx);
-    ctx->src_kind = ctx->trace64 ? PP_SRC_TRACE64 : PP_SRC_TRACE32;
+    ctx->src_kind = trace_kind(ctx);
     int64_t tot = 0;
     for (int64_t i = 0; i < n_events; ++i) tot += length[i];
     ctx->flat_cap = tot > 0 ? tot : 1;
@@ -1305,17 +1378,8 @@ int pp_event_stats_download(pp_ctx *ctx, int64_t cap, double *mean, double *std,
     CKR(ensure(ctx, ctx->evs_std, 8 * e));
     CKR(ensure(ctx, ctx->evs_min, 8 * e));
     CKR(ensure(ctx, ctx->evs_max, 8 * e));
-    if (ctx->src_kind == PP_SRC_TRACE32)
-        k4_segment_stats<float><<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(
-            ctx->trace, (const int64_t *)ctx->ev_start.p, (const int64_t *)ctx->ev_off.p, ctx->ctr, 1,
-            (const int64_t *)ctx->ev_off.p, nullptr, (int64_t)e, (double *)ctx->evs_mean.p,
-            (double *)ctx->evs_std.p, (double *)ctx->evs_min.p, (double *)ctx->evs_max.p);
-    else
-        k4_segment_stats<double><<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(
-            f64_samples(ctx), f64_bases(ctx), (const int64_t *)ctx->ev_off.p,
-            ctx->ctr, 1, (const int64_t *)ctx->ev_off.p, nullptr, (int64_t)e, (double *)ctx->evs_mean.p,
-            (double *)ctx->evs_std.p, (double *)ctx->evs_min.p, (double *)ctx->evs_max.p);
-    LAUNCHED(ctx);
+    CKR(launch_stats(ctx, 1, (const int64_t *)ctx->ev_off.p, nullptr, (int64_t)e, (double *)ctx->evs_mean.p,
+                     (double *)ctx->evs_std.p, (double *)ctx->evs_min.p, (double *)ctx->evs_max.p));
     if (mean) CK(cudaMemcpyAsync(mean, ctx->evs_mean.p, 8 * e, cudaMemcpyDeviceToHost, ctx->stream));
     if (std) CK(cudaMemcpyAsync(std, ctx->evs_std.p, 8 * e, cudaMemcpyDeviceToHost, ctx->stream));
     if (mn) CK(cudaMemcpyAsync(mn, ctx->evs_min.p, 8 * e, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1436,6 +1500,7 @@ int pp_pipeline(pp_ctx *ctx, const pp_pipeline_params *p, int64_t out[4])
 int pp_shard_scan(pp_ctx *ctx, double threshold, int64_t scan_len, double *dev_record)
 {
     if (!ctx || !dev_record) return PP_ERR_ARG;
+    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "the sharded path takes float32 traces");
     CKR(set_device(ctx));
     reset_stages(ctx);
     CKR(record_boundary(ctx, 0));
@@ -1454,6 +1519,7 @@ int pp_shard_finish(pp_ctx *ctx, const pp_pipeline_params *p, int skip_first, in
                     int64_t ev_start, int64_t ev_len, int64_t *dev_record)
 {
     if (!ctx || !p || !dev_record) return PP_ERR_ARG;
+    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "the sharded path takes float32 traces");
     if (p->filter_ncoef > 0) return fail(ctx, PP_ERR_ARG, "the sharded path does not filter");
     CKR(set_device(ctx));
     CKR(enqueue_select(ctx, p->rule_mask, p->duration_gt, p->duration_lt, p->min_gt, p->max_lt, skip_first,
@@ -1479,6 +1545,7 @@ int pp_shard_plan(pp_ctx *ctx, const double *dev_infos, int rank, int world, con
 {
     if (!ctx || !p || !dev_infos || !dev_plan || world < 1 || rank < 0 || rank >= world || halo_avail < 0)
         return fail(ctx, PP_ERR_ARG, "bad shard plan arguments");
+    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "the sharded path takes float32 traces");
     CKR(set_device(ctx));
     k_shard_plan<<<1, 32, 0, ctx->stream>>>(dev_infos, rank, world, p->rule_mask, p->duration_gt, p->duration_lt,
                                             p->min_gt, p->max_lt, halo_avail, (long long *)dev_plan);
@@ -1489,6 +1556,7 @@ int pp_shard_plan(pp_ctx *ctx, const double *dev_infos, int rank, int world, con
 int pp_shard_finish_planned(pp_ctx *ctx, const pp_pipeline_params *p, const int64_t *dev_plan, int64_t *dev_record)
 {
     if (!ctx || !p || !dev_plan || !dev_record) return PP_ERR_ARG;
+    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "the sharded path takes float32 traces");
     if (p->filter_ncoef > 0) return fail(ctx, PP_ERR_ARG, "the sharded path does not filter");
     CKR(set_device(ctx));
     CKR(enqueue_select(ctx, p->rule_mask, p->duration_gt, p->duration_lt, p->min_gt, p->max_lt, 0, 0, 0,
@@ -1509,6 +1577,7 @@ int pp_shard_finish_planned(pp_ctx *ctx, const pp_pipeline_params *p, const int6
 int pp_shard_commit(pp_ctx *ctx, const int64_t rec[8])
 {
     if (!ctx || !rec) return PP_ERR_ARG;
+    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "the sharded path takes float32 traces");
     ctx->n_runs = rec[0];
     ctx->n_events = rec[1];
     ctx->n_event_samples = rec[2];
@@ -1644,10 +1713,12 @@ int pp_unpack_tables_range(pp_ctx *ctx, const int64_t *dev_gathered, int world, 
 // stage up to the split search runs on the events completed so far while the next chunk is in flight.
 // With host tables (pp_pipeline_host_tables) compaction, statistics and the copy-out of the finished rows also
 // run per chunk, so that only the last chunk's rows are left when the last copy has landed.
-static int pipeline_host_impl(pp_ctx *ctx, const float *host, int64_t n, int64_t chunk_samples,
+// `kind`: PP_SRC_TRACE32 (float32 samples) or PP_SRC_ADC16 (int16 counts decoded with `adc`).
+static int pipeline_host_impl(pp_ctx *ctx, const void *host, int kind, PPAdc adc, int64_t n, int64_t chunk_samples,
                               const pp_pipeline_params *p, const pp_host_tables *tables, int64_t out[4])
 {
     if (!ctx || !p || !host || n <= 0) return fail(ctx, PP_ERR_ARG, "bad trace");
+    const size_t elem = kind == PP_SRC_ADC16 ? sizeof(int16_t) : sizeof(float);
     CKR(set_device(ctx));
     PPHostTables H;
     memset(&H, 0, sizeof H);
@@ -1678,7 +1749,8 @@ static int pipeline_host_impl(pp_ctx *ctx, const float *host, int64_t n, int64_t
     chunk_samples = (chunk_samples + K1_TILE - 1) / K1_TILE * K1_TILE;
     if (p->filter_ncoef > 0 || n <= chunk_samples) {
         // filtering needs every event before the split; a short trace gains nothing from chunking
-        CKR(pp_trace_upload(ctx, host, n, 0));
+        if (kind == PP_SRC_ADC16) CKR(pp_trace_upload_adc16(ctx, (const int16_t *)host, n, adc.scale, adc.offset));
+        else CKR(pp_trace_upload(ctx, (const float *)host, n, 0));
         CKR(pp_pipeline(ctx, p, out));
         if (tables) {
             CKR(enqueue_export(ctx, H, p->with_stats));
@@ -1688,13 +1760,13 @@ static int pipeline_host_impl(pp_ctx *ctx, const float *host, int64_t n, int64_t
         return PP_OK;
     }
     CKR(ensure_copy_stream(ctx));
-    CKR(ensure(ctx, ctx->trace_buf, sizeof(float) * (size_t)n));
-    ctx->trace = (const float *)ctx->trace_buf.p;
-    ctx->trace64 = nullptr;
+    CKR(ensure(ctx, ctx->trace_buf, elem * (size_t)n));
+    point_trace(ctx, ctx->trace_buf.p, elem);
+    ctx->adc = adc;
     ctx->n = n;
-    ctx->trace_cap = (int64_t)(ctx->trace_buf.cap / sizeof(float));
+    ctx->trace_cap = (int64_t)(ctx->trace_buf.cap / elem);
     ctx->adopted = false;
-    ctx->src_kind = PP_SRC_TRACE32;
+    ctx->src_kind = kind;
     ctx->flat_cap = n;
     reset_stages(ctx);
     CKR(begin_threshold(ctx, n));
@@ -1704,7 +1776,7 @@ static int pipeline_host_impl(pp_ctx *ctx, const float *host, int64_t n, int64_t
     CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->compute_ev, 0));
     for (int64_t a = 0; a < n; a += chunk_samples) {
         const int64_t b = a + chunk_samples < n ? a + chunk_samples : n;
-        CK(cudaMemcpyAsync((void *)(ctx->trace + a), host + a, sizeof(float) * (size_t)(b - a),
+        CK(cudaMemcpyAsync((char *)ctx->trace_buf.p + elem * a, (const char *)host + elem * a, elem * (size_t)(b - a),
                            cudaMemcpyHostToDevice, ctx->copy_stream));
         CK(cudaEventRecord(ctx->copy_ev, ctx->copy_stream));
         CK(cudaStreamWaitEvent(ctx->stream, ctx->copy_ev, 0));
@@ -1751,17 +1823,28 @@ static int pipeline_host_impl(pp_ctx *ctx, const float *host, int64_t n, int64_t
     return PP_OK;
 }
 
+static const PPAdc PP_NO_ADC = {1.0, 0.0};
+
 int pp_pipeline_host(pp_ctx *ctx, const float *host, int64_t n, int64_t chunk_samples,
                      const pp_pipeline_params *p, int64_t out[4])
 {
-    return pipeline_host_impl(ctx, host, n, chunk_samples, p, nullptr, out);
+    return pipeline_host_impl(ctx, host, PP_SRC_TRACE32, PP_NO_ADC, n, chunk_samples, p, nullptr, out);
 }
 
 int pp_pipeline_host_tables(pp_ctx *ctx, const float *host, int64_t n, int64_t chunk_samples,
                             const pp_pipeline_params *p, const pp_host_tables *tables, int64_t out[4])
 {
     if (!tables) return fail(ctx, PP_ERR_ARG, "no host tables");
-    return pipeline_host_impl(ctx, host, n, chunk_samples, p, tables, out);
+    return pipeline_host_impl(ctx, host, PP_SRC_TRACE32, PP_NO_ADC, n, chunk_samples, p, tables, out);
+}
+
+int pp_pipeline_host_adc16(pp_ctx *ctx, const int16_t *host, int64_t n, double scale, double offset,
+                           int64_t chunk_samples, const pp_pipeline_params *p, const pp_host_tables *tables,
+                           int64_t out[4])
+{
+    if (pp_adc16_check(scale, offset) != PP_OK)
+        return fail(ctx, PP_ERR_ARG, "ADC scale must be finite and non-zero, offset finite, every count decoding finite");
+    return pipeline_host_impl(ctx, host, PP_SRC_ADC16, PPAdc{scale, offset}, n, chunk_samples, p, tables, out);
 }
 
 }  // extern "C"

@@ -48,24 +48,42 @@ enum { PP_OVF_RUNS = 1, PP_OVF_QUEUE = 2, PP_OVF_SEGS = 4, PP_OVF_FILTER_SHORT =
        PP_OVF_EXPORT = 32 /* host tables of pp_pipeline_host_tables too small */,
        PP_OVF_CTL = 64 /* multi-GPU: a peer's record did not arrive (pp_ctl_exchange timed out) */ };
 
+// int16 ADC counts and what they stand for: current = fl(fl(c * scale) + offset), two IEEE roundings and no FMA --
+// exactly what NumPy computes for counts.astype(np.float64) * scale + offset.
+struct PPAdc {
+    double scale, offset;
+};
+__device__ __forceinline__ double pp_adc_decode(int c, const PPAdc &a)
+{
+    return __dadd_rn(__dmul_rn((double)c, a.scale), a.offset);
+}
+// A sample as the float64 value every stage computes with (float32 / float64 samples as they are)
+__device__ __forceinline__ double pp_val(float x, const PPAdc &) { return (double)x; }
+__device__ __forceinline__ double pp_val(double x, const PPAdc &) { return x; }
+__device__ __forceinline__ double pp_val(int16_t c, const PPAdc &a) { return pp_adc_decode(c, a); }
+
 // Where an event's samples live.
 //   kind 0: float32 trace, sample j of event e = trace[ev_start[e] + j]
 //   kind 1: float64 packed array, sample j of event e = flat[ev_off[e] + j]   (uploaded events, filtered current)
 //   kind 2: float64 trace, sample j of event e = trace64[ev_start[e] + j]
+//   kind 3: int16 ADC trace, sample j of event e = decode(trace16[ev_start[e] + j]) with `adc`
 struct PPSource {
     const float *trace;
     const double *trace64;
+    const int16_t *trace16;
     const double *flat;
     const int64_t *ev_start;
     const int64_t *ev_off;
+    PPAdc adc;
     int kind;
 };
-enum { PP_SRC_TRACE32 = 0, PP_SRC_FLAT64 = 1, PP_SRC_TRACE64 = 2 };
+enum { PP_SRC_TRACE32 = 0, PP_SRC_FLAT64 = 1, PP_SRC_TRACE64 = 2, PP_SRC_ADC16 = 3 };
 
 __device__ __forceinline__ double pp_sample(const PPSource &s, int64_t ev, int64_t j)
 {
     if (s.kind == PP_SRC_TRACE32) return (double)__ldg(s.trace + s.ev_start[ev] + j);
     if (s.kind == PP_SRC_TRACE64) return __ldg(s.trace64 + s.ev_start[ev] + j);
+    if (s.kind == PP_SRC_ADC16) return pp_adc_decode(__ldg(s.trace16 + s.ev_start[ev] + j), s.adc);
     return __ldg(s.flat + s.ev_off[ev] + j);
 }
 

@@ -44,7 +44,7 @@ __device__ __forceinline__ void k2s_load(const T *__restrict__ p, int64_t base, 
 
 template <typename T>
 __device__ __forceinline__ void k2s_event(const T *__restrict__ p, int64_t len, double2 *__restrict__ out,
-                                          double (*v)[K2S_TILE], int lane)
+                                          double (*v)[K2S_TILE], int lane, const PPAdc &adc)
 {
     double acc = 0.0;  // lane 0: c, lane 1: c2
     T xv[K2S_TILE / 32], xn[K2S_TILE / 32];
@@ -53,7 +53,7 @@ __device__ __forceinline__ void k2s_event(const T *__restrict__ p, int64_t len, 
         const int cnt = (int)((len - base) < K2S_TILE ? (len - base) : K2S_TILE);
 #pragma unroll
         for (int k = 0; k < K2S_TILE / 32; ++k) {
-            const double x = (double)xv[k];
+            const double x = pp_val(xv[k], adc);
             v[0][k * 32 + lane] = x;
             v[1][k * 32 + lane] = __dmul_rn(x, x);
         }
@@ -104,9 +104,10 @@ k2_prefix_sequential(PPSource src, const int64_t *__restrict__ ev_len, PPCounter
         }
         const int64_t len = ev_len[e];
         const int64_t off = src.ev_off[e];
-        if (src.kind == PP_SRC_TRACE32) k2s_event(src.trace + src.ev_start[e], len, cc + off, sv[warp], lane);
-        else if (src.kind == PP_SRC_TRACE64) k2s_event(src.trace64 + src.ev_start[e], len, cc + off, sv[warp], lane);
-        else k2s_event(src.flat + off, len, cc + off, sv[warp], lane);
+        if (src.kind == PP_SRC_TRACE32) k2s_event(src.trace + src.ev_start[e], len, cc + off, sv[warp], lane, src.adc);
+        else if (src.kind == PP_SRC_TRACE64) k2s_event(src.trace64 + src.ev_start[e], len, cc + off, sv[warp], lane, src.adc);
+        else if (src.kind == PP_SRC_ADC16) k2s_event(src.trace16 + src.ev_start[e], len, cc + off, sv[warp], lane, src.adc);
+        else k2s_event(src.flat + off, len, cc + off, sv[warp], lane, src.adc);
     }
 }
 
@@ -275,7 +276,7 @@ k2_event_scan(PPSource src, const T *__restrict__ samples, const int64_t *__rest
         double carry_c = 0.0, carry_c2 = 0.0;
         K2FBits fb;
         fb.init();
-        K2Exp ex;   // float64 source: both x and x*x are analysed
+        K2Exp ex;   // float64 / ADC source: both x and x*x are analysed
         ex.init();
         T xv[K2F_ITEMS], xn[K2F_ITEMS];
 #pragma unroll
@@ -303,8 +304,8 @@ k2_event_scan(PPSource src, const T *__restrict__ samples, const int64_t *__rest
 #pragma unroll
             for (int k = 0; k < K2F_ITEMS; ++k) {
                 const T xs = sin[lane * K2F_PAD + k];
-                if (sizeof(T) == 4) fb.add(xs); else ex.add(xs);
-                const double x = (double)xs;
+                const double x = pp_val(xs, src.adc);
+                if constexpr (sizeof(T) == 4) fb.add(xs); else ex.add(x);
                 c = __dadd_rn(c, x);
                 c2 = __dadd_rn(c2, __dmul_rn(x, x));
                 pc[k] = c; pc2[k] = c2;
@@ -436,7 +437,7 @@ __device__ __forceinline__ K2Tile k2_locate(const PPSource &src, const int64_t *
 // Pass 1: per-tile sums and exponent statistics.  Any summation order will do (see above).
 template <typename T>
 __global__ void __launch_bounds__(K2_THREADS)
-k2_tile_reduce(PPSource src, const T *__restrict__ samples /* trace (kind 0) or flat (kind 1) */,
+k2_tile_reduce(PPSource src, const T *__restrict__ samples /* the trace, or flat for kind 1 */,
                const int64_t *__restrict__ ev_len, const int64_t *__restrict__ ev_tile_off, const PPCounters *ctr,
                K2TileState *__restrict__ tiles, K2EventBits *__restrict__ bits)
 {
@@ -459,8 +460,8 @@ k2_tile_reduce(PPSource src, const T *__restrict__ samples /* trace (kind 0) or 
         ex.init();
 #pragma unroll
         for (int i = 0; i < K2_ITEMS; ++i) {
-            const double x = (double)xv[i];
-            ex.add(xv[i]);
+            const double x = pp_val(xv[i], src.adc);
+            if constexpr (sizeof(T) == 4) ex.add(xv[i]); else ex.add(x);
             c = __dadd_rn(c, x);
             c2 = __dadd_rn(c2, __dmul_rn(x, x));
         }
@@ -571,7 +572,7 @@ k2_tile_scan(PPSource src, const T *__restrict__ samples, const int64_t *__restr
         double c = 0.0, c2 = 0.0;
 #pragma unroll
         for (int k = 0; k < K2_ITEMS; ++k) {
-            const double x = (double)sin[tid * K2_PAD + k];
+            const double x = pp_val(sin[tid * K2_PAD + k], src.adc);
             c = __dadd_rn(c, x);
             c2 = __dadd_rn(c2, __dmul_rn(x, x));
             pc[k] = c; pc2[k] = c2;

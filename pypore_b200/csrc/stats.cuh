@@ -13,7 +13,8 @@
 //     8-lane group instead of 17 (the first cut issued 32 thread instructions per sample, most of them
 //     per-row set-up and scalar loads: 31 % of the HBM peak);
 //   * longer rows: two passes (mean first, then deviations from it), like np.std.
-// min / max run on the samples' own type; a NaN anywhere makes both NaN like np.min / np.max.
+// min / max run on the samples' own type (int16 ADC counts: on the counts, decoded at the end); a NaN anywhere
+// makes both NaN like np.min / np.max.
 #pragma once
 #include "common.cuh"
 
@@ -55,10 +56,26 @@ __device__ __forceinline__ double k4_group_max(double v)
     for (int d = G / 2; d > 0; d >>= 1) v = fmax(v, __shfl_xor_sync(PP_FULL, v, d));
     return v;
 }
+template <int G>
+__device__ __forceinline__ int16_t k4_group_min(int16_t v)
+{
+#pragma unroll
+    for (int d = G / 2; d > 0; d >>= 1) v = min(v, (int16_t)__shfl_xor_sync(PP_FULL, (int)v, d));
+    return v;
+}
+template <int G>
+__device__ __forceinline__ int16_t k4_group_max(int16_t v)
+{
+#pragma unroll
+    for (int d = G / 2; d > 0; d >>= 1) v = max(v, (int16_t)__shfl_xor_sync(PP_FULL, (int)v, d));
+    return v;
+}
 __device__ __forceinline__ float k4_min(float a, float b) { return fminf(a, b); }
 __device__ __forceinline__ float k4_max(float a, float b) { return fmaxf(a, b); }
 __device__ __forceinline__ double k4_min(double a, double b) { return fmin(a, b); }
 __device__ __forceinline__ double k4_max(double a, double b) { return fmax(a, b); }
+__device__ __forceinline__ int16_t k4_min(int16_t a, int16_t b) { return a < b ? a : b; }
+__device__ __forceinline__ int16_t k4_max(int16_t a, int16_t b) { return a > b ? a : b; }
 
 template <typename T> struct K4Vec;
 template <> struct K4Vec<float> {
@@ -71,6 +88,21 @@ template <> struct K4Vec<double> {
     typedef double2 V;
     static __device__ __forceinline__ void get(const V &q, double *o) { o[0] = q.x; o[1] = q.y; }
 };
+template <> struct K4Vec<int16_t> {   // ADC counts: min / max on the counts, decoded once at the end
+    static constexpr int N = 8;
+    typedef int4 V;
+    static __device__ __forceinline__ void get(const V &q, int16_t *o)
+    {
+        const int w[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+        for (int i = 0; i < 4; ++i) { o[2 * i] = (int16_t)(w[i] & 0xffff); o[2 * i + 1] = (int16_t)(w[i] >> 16); }
+    }
+};
+// start values of the min / max tracking: +-inf, or the ends of the int16 range
+template <typename T> __device__ __forceinline__ T k4_top() { return (T)__longlong_as_double(0x7ff0000000000000LL); }
+template <> __device__ __forceinline__ int16_t k4_top<int16_t>() { return 32767; }
+template <typename T> __device__ __forceinline__ T k4_bottom() { return -k4_top<T>(); }
+template <> __device__ __forceinline__ int16_t k4_bottom<int16_t>() { return -32768; }
 
 // Rows k = group, group + ngroups, ...; every lane of a warp runs the same number of rows
 // so that the full-mask shuffles stay convergent (inactive groups work on an empty row).
@@ -79,7 +111,7 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
                                         const int64_t *__restrict__ ev_off, int64_t row0, int64_t rows, int64_t total,
                                         const int64_t *__restrict__ flat_start, const int *__restrict__ row_event,
                                         double *__restrict__ o_mean, double *__restrict__ o_std,
-                                        double *__restrict__ o_min, double *__restrict__ o_max)
+                                        double *__restrict__ o_min, double *__restrict__ o_max, const PPAdc &adc)
 {
     typedef K4Vec<T> VT;
     constexpr int N = VT::N;
@@ -87,7 +119,6 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
     const int64_t group0 = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) / G;
     const int64_t ngroups = ((int64_t)gridDim.x * blockDim.x) / G;
     const int64_t warp_first = group0 - ((threadIdx.x & 31) / G);  // row of the warp's first group
-    const T inf = (T)__longlong_as_double(0x7ff0000000000000LL);
     for (int64_t kw = row0 + warp_first; kw < rows; kw += ngroups) {  // rows [row0, rows)
         const int64_t k = kw + ((threadIdx.x & 31) / G);
         const bool live = k < rows;
@@ -101,7 +132,7 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
             p = samples + ev_base[ev] + (f0 - ev_off[ev]);
         }
         double s1 = 0.0, s2 = 0.0;
-        T mn = inf, mx = -inf;
+        T mn = k4_top<T>(), mx = k4_bottom<T>();
         int nan = 0;
         double mean, var;
         if (__all_sync(PP_FULL, len <= K4_ONE_PASS)) {
@@ -110,7 +141,7 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
             const typename VT::V *pv = reinterpret_cast<const typename VT::V *>(p - mis);
             const int64_t last = mis + len;                  // elements [mis, last) of the vector stream are the row
             const int64_t nvec = (last + N - 1) / N;
-            double K = len > 0 ? (double)__ldg(p) : 0.0;     // the shift: the row's first sample
+            double K = len > 0 ? pp_val(__ldg(p), adc) : 0.0;  // the shift: the row's first sample
             if (!(fabs(K) <= 1.7e308)) K = 0.0;              // inf / NaN: plain sums
             for (int64_t v0 = gl; v0 < nvec; v0 += K4_U * G) {
                 typename VT::V q[K4_U];
@@ -126,7 +157,7 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
                     if (e0 >= mis && e0 + N <= last) {
 #pragma unroll
                         for (int c = 0; c < N; ++c) {
-                            const double d = (double)x[c] - K;
+                            const double d = pp_val(x[c], adc) - K;
                             s1 += d;
                             s2 = fma(d, d, s2);
                             mn = k4_min(mn, x[c]);
@@ -137,7 +168,7 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
 #pragma unroll
                         for (int c = 0; c < N; ++c) {
                             if (e0 + c >= mis && e0 + c < last) {
-                                const double d = (double)x[c] - K;
+                                const double d = pp_val(x[c], adc) - K;
                                 s1 += d;
                                 s2 = fma(d, d, s2);
                                 mn = k4_min(mn, x[c]);
@@ -158,14 +189,14 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
         } else {
             for (int64_t j = gl; j < len; j += G) {
                 const T x = p[j];
-                s1 += (double)x;
+                s1 += pp_val(x, adc);
                 mn = k4_min(mn, x);
                 mx = k4_max(mx, x);
                 nan |= (x != x);
             }
             mean = k4_group_sum<G>(s1) / (double)len;
             for (int64_t j = gl; j < len; j += G) {
-                const double d = (double)p[j] - mean;
+                const double d = pp_val(p[j], adc) - mean;
                 s2 = fma(d, d, s2);
             }
             var = k4_group_sum<G>(s2) / (double)len;
@@ -176,23 +207,25 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
         for (int d = G / 2; d > 0; d >>= 1) nan |= __shfl_xor_sync(PP_FULL, nan, d);
         if (live && gl == 0) {
             const double qnan = __longlong_as_double(0x7ff8000000000000LL);
+            double dmn = pp_val(mn, adc), dmx = pp_val(mx, adc);
+            if (sizeof(T) == 2 && adc.scale < 0.0) { const double t = dmn; dmn = dmx; dmx = t; }  // decreasing decode
             o_mean[k] = mean;
             o_std[k] = sqrt(var < 0.0 ? 0.0 : var);
-            o_min[k] = nan ? qnan : (double)mn;
-            o_max[k] = nan ? qnan : (double)mx;
+            o_min[k] = nan ? qnan : dmn;
+            o_max[k] = nan ? qnan : dmx;
         }
     }
 }
 
 // flat_start[k] .. flat_start[k+1] (or `total` for the last) bounds row k;
-// row_event == nullptr means row k is event k (statistics of whole events).
+// row_event == nullptr means row k is event k (statistics of whole events).  `adc` decodes int16 samples.
 template <typename T>
 __global__ void __launch_bounds__(256)
 k4_segment_stats(const T *__restrict__ samples, const int64_t *__restrict__ ev_base,
                  const int64_t *__restrict__ ev_off, const PPCounters *ctr, int rows_are_events,
                  const int64_t *__restrict__ flat_start, const int *__restrict__ row_event,
                  int64_t cap_rows, double *__restrict__ o_mean, double *__restrict__ o_std,
-                 double *__restrict__ o_min, double *__restrict__ o_max)
+                 double *__restrict__ o_min, double *__restrict__ o_max, PPAdc adc)
 {
     int64_t rows = rows_are_events ? (int64_t)ctr->n_events : (int64_t)ctr->n_segments;
     if (rows > cap_rows) rows = cap_rows;
@@ -201,7 +234,7 @@ k4_segment_stats(const T *__restrict__ samples, const int64_t *__restrict__ ev_b
     const int64_t row0 = rows_are_events ? 0 : (int64_t)ctr->seg_done;
     if (rows <= row0) return;
     if (total / rows < 512)
-        k4_rows<T, 8>(samples, ev_base, ev_off, row0, rows, total, flat_start, row_event, o_mean, o_std, o_min, o_max);
+        k4_rows<T, 8>(samples, ev_base, ev_off, row0, rows, total, flat_start, row_event, o_mean, o_std, o_min, o_max, adc);
     else
-        k4_rows<T, 32>(samples, ev_base, ev_off, row0, rows, total, flat_start, row_event, o_mean, o_std, o_min, o_max);
+        k4_rows<T, 32>(samples, ev_base, ev_off, row0, rows, total, flat_start, row_event, o_mean, o_std, o_min, o_max, adc);
 }

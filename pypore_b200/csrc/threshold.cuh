@@ -2,7 +2,8 @@
 //
 // Replaces PyPore/parsers.py:148-155 (mask / diff / where / split) and the
 // np.min / np.max second pass of _lambda_select (parsers.py:136-140 through
-// core.py:215-220).  One read of the trace (4 B/sample for float32 input, 8 B/sample for float64 input):
+// core.py:215-220).  One read of the trace (4 B/sample for float32 input, 8 B/sample for float64 input, 2 B/sample
+// for int16 ADC counts):
 //
 //   k1_scan_tiles   persistent CTAs stream 4096-sample tiles through a ring of shared-memory stages filled by
 //                   1-D TMA bulk copies (cp.async.bulk + mbarrier, three tiles in flight per CTA).  Each WARP owns a
@@ -18,6 +19,11 @@
 //                   A span with more than K1_STAGE crossings (noise riding on the threshold) is walked again here,
 //                   sample by sample.
 //   k1_finalize_runs decodes the run table (length, side, min / max as float64).
+//
+// ADC counts are scanned as integer keys k = c ^ kxor (kxor = -1 for a negative scale: ~c = -c - 1 reverses the
+// order), in which the decoded current fl(fl(c * scale) + offset) is non-decreasing.  So `current < threshold` is
+// `k < key threshold` (pp_adc16_key_threshold), the no-crossing path is a warp integer min / max and a vote, there
+// is no NaN, and the run extrema are the keys' extrema, decoded once by k1_finalize_runs.
 //
 // The first round's kernel did all of this in one pass with the look-back inside the streaming kernel: 28 % of the
 // HBM peak, 11 barrier-stall cycles per issue (profiles/r01o_ncu_summary.csv).
@@ -109,6 +115,26 @@ template <> __device__ __forceinline__ double k1_min<double>(double a, double b)
 template <typename T> __device__ __forceinline__ T k1_max(T a, T b);
 template <> __device__ __forceinline__ float k1_max<float>(float a, float b) { return fmaxf(a, b); }
 template <> __device__ __forceinline__ double k1_max<double>(double a, double b) { return fmax(a, b); }
+template <> __device__ __forceinline__ int k1_min<int>(int a, int b) { return min(a, b); }
+template <> __device__ __forceinline__ int k1_max<int>(int a, int b) { return max(a, b); }
+
+// What the scan compares: float32 / float64 samples as they are, int16 ADC counts as their keys c ^ kxor.
+template <typename T> struct K1Key {
+    typedef T V;
+    static __device__ __forceinline__ V of(T x, int) { return x; }
+};
+template <> struct K1Key<int16_t> {
+    typedef int V;
+    static __device__ __forceinline__ V of(int16_t c, int kxor) { return (int)c ^ kxor; }
+};
+
+// run-key extrema of a warp (keys as in the run table: pp_dkey of the value)
+__device__ __forceinline__ unsigned long long k1_warp_min_key(float m) { return k1_warp_min_u64(pp_dkey((double)m)); }
+__device__ __forceinline__ unsigned long long k1_warp_max_key(float m) { return k1_warp_max_u64(pp_dkey((double)m)); }
+__device__ __forceinline__ unsigned long long k1_warp_min_key(double m) { return k1_warp_min_u64(pp_dkey(m)); }
+__device__ __forceinline__ unsigned long long k1_warp_max_key(double m) { return k1_warp_max_u64(pp_dkey(m)); }
+__device__ __forceinline__ unsigned long long k1_warp_min_key(int m) { return pp_dkey((double)__reduce_min_sync(PP_FULL, m)); }
+__device__ __forceinline__ unsigned long long k1_warp_max_key(int m) { return pp_dkey((double)__reduce_max_sync(PP_FULL, m)); }
 
 __device__ __forceinline__ void k1_mbar_arrive(void *bar)
 {
@@ -125,6 +151,7 @@ __device__ __forceinline__ float k1_max_nan(float a, float b)
     return d;
 }
 __device__ __forceinline__ double k1_max_nan(double a, double b) { return (a != a || b != b) ? a + b : fmax(a, b); }
+__device__ __forceinline__ int k1_max_nan(int a, int b) { return max(a, b); }
 
 // Shared memory of k1_scan_tiles: the stages (one tile each, source and destination of the bulk copy 128-byte
 // aligned -- a copy that started 16 bytes before the tile to bring the previous sample along ran at a third of
@@ -140,12 +167,14 @@ constexpr int K1_CTA_THREADS = K1_THREADS + 32;   // eight consumer warps + the 
 
 // Tiles [tile_begin, tile_begin + n_tiles) of the trace prefix x[0, n).  thr: `sample < thr` <=> below
 // (float32 input: the smallest float32 >= the threshold, so that the comparison equals the reference's
-// double(x) < threshold for every float32 x; float64 input: the threshold itself).
+// double(x) < threshold for every float32 x; float64 input: the threshold itself; int16 input: the key threshold,
+// compared with the keys c ^ kxor).
 template <typename T>
 __global__ void __launch_bounds__(K1_CTA_THREADS)
-k1_scan_tiles(const T *__restrict__ x, int64_t n, T thr, int64_t tile_begin, int64_t n_tiles,
-              K1Record *__restrict__ rec, K1Staged *__restrict__ staged)
+k1_scan_tiles(const T *__restrict__ x, int64_t n, typename K1Key<T>::V thr, int kxor, int64_t tile_begin,
+              int64_t n_tiles, K1Record *__restrict__ rec, K1Staged *__restrict__ staged)
 {
+    typedef typename K1Key<T>::V V;
     extern __shared__ __align__(128) unsigned char k1_raw[];
     K1Smem<T> &S = *reinterpret_cast<K1Smem<T> *>(k1_raw);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -183,45 +212,49 @@ k1_scan_tiles(const T *__restrict__ x, int64_t n, T thr, int64_t tile_begin, int
         const int s = (int)(it % K1_STAGES);
         // the sample in front of the tile comes straight from global memory (warp 0 alone needs it; the load is
         // in flight while the warp waits for the tile)
-        T before = (T)0;
-        if (warp == 0 && base > 0) before = __ldg(x + base - 1);
+        V before = (V)0;
+        if (warp == 0 && base > 0) before = K1Key<T>::of(__ldg(x + base - 1), kxor);
         k1_mbar_wait(&S.full[s], (unsigned)((it / K1_STAGES) & 1));
         // ---- this warp's span: 4 rows of 128 samples, lane l holds samples 4l .. 4l+3 of each row ----
         T *sp = &S.stage[s][0] + warp * K1_SPAN;
         const bool ragged = base + K1_TILE > n;
-        T ahead = (T)0;                                     // ragged tile: the sample in front of this warp's span
+        V ahead = (V)0;                                     // ragged tile: the sample in front of this warp's span
         if (ragged) {
             // last tile of the trace: nothing was staged; every warp brings its own span in (past n the last sample
             // repeats, which adds no crossing and no new extreme) and reads back only what it wrote itself
             const int64_t g0 = base + warp * K1_SPAN;
             const T fill = __ldg(x + (n - 1));
             for (int k = lane; k < K1_SPAN; k += 32) sp[k] = g0 + k < n ? __ldg(x + g0 + k) : fill;
-            if (warp > 0) ahead = g0 - 1 < n ? __ldg(x + g0 - 1) : fill;
+            if (warp > 0) ahead = K1Key<T>::of(g0 - 1 < n ? __ldg(x + g0 - 1) : fill, kxor);
             __syncwarp();
         }
-        T v[4][4];
+        V v[4][4];
 #pragma unroll
         for (int r = 0; r < 4; ++r) {
-            if (sizeof(T) == 4) {
+            if constexpr (sizeof(T) == 4) {
                 const float4 q = *reinterpret_cast<const float4 *>(sp + r * 128 + lane * 4);
                 v[r][0] = (T)q.x; v[r][1] = (T)q.y; v[r][2] = (T)q.z; v[r][3] = (T)q.w;
-            } else {
+            } else if constexpr (sizeof(T) == 8) {
                 const double2 q0 = *reinterpret_cast<const double2 *>(sp + r * 128 + lane * 4);
                 const double2 q1 = *reinterpret_cast<const double2 *>(sp + r * 128 + lane * 4 + 2);
                 v[r][0] = (T)q0.x; v[r][1] = (T)q0.y; v[r][2] = (T)q1.x; v[r][3] = (T)q1.y;
+            } else {
+                const uint2 q = *reinterpret_cast<const uint2 *>(sp + r * 128 + lane * 4);
+                v[r][0] = K1Key<T>::of((T)(q.x & 0xffffu), kxor); v[r][1] = K1Key<T>::of((T)(q.x >> 16), kxor);
+                v[r][2] = K1Key<T>::of((T)(q.y & 0xffffu), kxor); v[r][3] = K1Key<T>::of((T)(q.y >> 16), kxor);
             }
         }
         // side of the sample in front of the span
-        const bool carry_below = (warp == 0 ? before : (ragged ? ahead : sp[-1])) < thr;
+        const bool carry_below = (warp == 0 ? before : (ragged ? ahead : K1Key<T>::of(sp[-1], kxor))) < thr;
         __syncwarp();
         if (lane == 0) k1_mbar_arrive(&S.empty[s]);   // this warp has its samples in registers
 
-        T m = v[0][0], M = v[0][0];
+        V m = v[0][0], M = v[0][0];
 #pragma unroll
         for (int r = 0; r < 4; ++r)
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
-                m = k1_min<T>(m, v[r][k]);
+                m = k1_min<V>(m, v[r][k]);
                 M = k1_max_nan(M, v[r][k]);
             }
         const bool w_below = __any_sync(PP_FULL, m < thr), w_above = __any_sync(PP_FULL, !(M < thr));
@@ -232,8 +265,8 @@ k1_scan_tiles(const T *__restrict__ x, int64_t n, T thr, int64_t tile_begin, int
         const bool carry = (base == 0 && warp == 0) ? first_below : carry_below;
         if (!(w_below && w_above) && carry == w_below) {
             // ---- no crossing: the whole span continues the open run ----
-            unsigned long long kmin = k1_warp_min_u64(pp_dkey((double)m));
-            unsigned long long kmax = k1_warp_max_u64(pp_dkey((double)M));
+            unsigned long long kmin = k1_warp_min_key(m);
+            unsigned long long kmax = k1_warp_max_key(M);
             if (w_nan) { kmin = 0ull; kmax = ~0ull; }
             if (lane == 0) {
                 K1Record R;
@@ -285,16 +318,16 @@ k1_scan_tiles(const T *__restrict__ x, int64_t n, T thr, int64_t tile_begin, int
         }
         const unsigned q_last = count < (unsigned)K1_STAGE ? count : (unsigned)K1_STAGE;
         for (unsigned q = 0; q <= q_last; ++q) {
-            T pm = v[0][0], pM = v[0][0];
+            V pm = v[0][0], pM = v[0][0];
             bool have = false, pnan = false;
 #pragma unroll
             for (int r = 0; r < 4; ++r)
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {
                     const bool mine = rid[r][k] == q;
-                    const T val = v[r][k];
-                    pm = mine ? (have ? k1_min<T>(pm, val) : val) : pm;
-                    pM = mine ? (have ? k1_max<T>(pM, val) : val) : pM;
+                    const V val = v[r][k];
+                    pm = mine ? (have ? k1_min<V>(pm, val) : val) : pm;
+                    pM = mine ? (have ? k1_max<V>(pM, val) : val) : pM;
                     pnan |= mine && (val != val);
                     have |= mine;
                 }
@@ -342,7 +375,7 @@ constexpr int K1B_THREADS = 256;
 
 template <typename T>
 __global__ void __launch_bounds__(K1B_THREADS)
-k1_stitch(const T *__restrict__ x, int64_t n, T thr, int64_t rec_begin, int64_t rec_end,
+k1_stitch(const T *__restrict__ x, int64_t n, typename K1Key<T>::V thr, int kxor, int64_t rec_begin, int64_t rec_end,
           const K1Record *__restrict__ rec, const K1Staged *__restrict__ staged,
           unsigned long long *__restrict__ blk_state, PPCounters *ctr, int flip, int64_t *__restrict__ run_start,
           unsigned long long *__restrict__ run_minkey, unsigned long long *__restrict__ run_maxkey, int64_t cap_runs)
@@ -430,11 +463,11 @@ k1_stitch(const T *__restrict__ x, int64_t n, T thr, int64_t rec_begin, int64_t 
     }
     // ---- more crossings than were staged (noise riding on the threshold): walk the span again ----
     unsigned long long rid = first_run;
-    bool below = span0 > 0 ? (__ldg(x + span0 - 1) < thr) : (__ldg(x) < thr);
+    bool below = K1Key<T>::of(__ldg(x + (span0 > 0 ? span0 - 1 : 0)), kxor) < thr;
     unsigned long long kmin = PP_MINKEY64_EMPTY, kmax = PP_MAXKEY64_EMPTY;
     const int64_t end = span0 + K1_SPAN < n ? span0 + K1_SPAN : n;
     for (int64_t p = span0; p < end; ++p) {
-        const T val = __ldg(x + p);
+        const typename K1Key<T>::V val = K1Key<T>::of(__ldg(x + p), kxor);
         const bool b = val < thr;
         if (b != below) {
             if ((int64_t)rid < cap_runs && kmin != PP_MINKEY64_EMPTY) {
@@ -469,14 +502,16 @@ __device__ __forceinline__ double pp_decode_max64(unsigned long long k)
     return pp_dkey_inv(k);
 }
 
-// Decode the run table: length, side, min/max as float64 (what the rules see).
+// Decode the run table: length, side, min/max as float64 (what the rules see).  adc != 0: the keys are ADC keys
+// c ^ kxor, decoded with `a` (the current is non-decreasing in the key, so the extreme keys give the extremes).
 __global__ void __launch_bounds__(256)
 k1_finalize_runs(int64_t n, const PPCounters *ctr, const int64_t *__restrict__ run_start,
                  const unsigned long long *__restrict__ run_minkey,
                  const unsigned long long *__restrict__ run_maxkey,
                  int64_t cap_runs, int64_t *__restrict__ run_len, double *__restrict__ run_min,
-                 double *__restrict__ run_max, unsigned char *__restrict__ run_below)
+                 double *__restrict__ run_max, unsigned char *__restrict__ run_below, int adc, PPAdc a)
 {
+    const int kxor = a.scale < 0.0 ? -1 : 0;
     int64_t n_runs = (int64_t)ctr->n_runs;
     if (n_runs > cap_runs) n_runs = cap_runs;
     const unsigned first_below = ctr->first_below;
@@ -485,8 +520,13 @@ k1_finalize_runs(int64_t n, const PPCounters *ctr, const int64_t *__restrict__ r
         const int64_t s = run_start[r];
         const int64_t e = (r + 1 < (int64_t)ctr->n_runs && r + 1 < cap_runs) ? run_start[r + 1] : n;
         run_len[r] = e - s;
-        run_min[r] = pp_decode_min64(run_minkey[r]);
-        run_max[r] = pp_decode_max64(run_maxkey[r]);
+        double mn = pp_decode_min64(run_minkey[r]), mx = pp_decode_max64(run_maxkey[r]);
+        if (adc) {   // (an empty run stays NaN)
+            if (mn == mn) mn = pp_adc_decode((int)mn ^ kxor, a);
+            if (mx == mx) mx = pp_adc_decode((int)mx ^ kxor, a);
+        }
+        run_min[r] = mn;
+        run_max[r] = mx;
         run_below[r] = (unsigned char)((first_below ^ (unsigned)(r & 1)) & 1u);
     }
 }

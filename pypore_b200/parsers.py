@@ -11,6 +11,7 @@ import math
 import numpy as np
 
 from . import _lib
+from .adc import AdcTrace
 from .core import Segment
 
 
@@ -116,7 +117,8 @@ class RuleSet(list):
 
 class _RunProxy(object):
     """What a rule sees of one piece (SURVEY App. A.1 item 6): ``duration``, ``start``,
-    ``min``, ``max``, ``n`` from the device run table; ``current``/``mean``/``std`` lazily."""
+    ``min``, ``max``, ``n`` from the device run table; ``current``/``mean``/``std`` lazily (``current`` of an
+    AdcTrace: the decoded slice)."""
 
     def __init__(self, host_current, start, n, mn, mx):
         self.start, self.duration, self.n, self.min, self.max = start, n, n, mn, mx
@@ -186,9 +188,9 @@ class lambda_event_parser(parser):
         return r_start[keep], r_len[keep], r_min[keep], r_max[keep]
 
     def parse(self, current):
-        """One Segment per surviving run: ``current`` (a copy), ``start`` (np.int64
-        sample index) and ``duration`` (samples) -- no ``end``, like the reference."""
-        host = np.asarray(current)
+        """One Segment per surviving run: ``current`` (a copy; decoded float64 for an AdcTrace), ``start``
+        (np.int64 sample index) and ``duration`` (samples) -- no ``end``, like the reference."""
+        host = current if isinstance(current, AdcTrace) else np.asarray(current)
         if host.shape[0] == 0:
             return []
         ctx = _lib.default_context()
@@ -220,7 +222,10 @@ def _device_trace(x):
 
 
 def _upload_trace(ctx, x):
-    """`x` (any accepted dtype) resident on `ctx`; returns the array that went up."""
+    """`x` (any accepted dtype, or an AdcTrace) resident on `ctx`; returns what went up."""
+    if isinstance(x, AdcTrace):
+        ctx.upload_trace_adc16(x)
+        return x
     dev = _device_trace(x)
     if dev.dtype == np.float32:
         ctx.upload_trace(dev)
@@ -230,8 +235,10 @@ def _upload_trace(ctx, x):
 
 
 def _run_pipeline(ctx, x, threshold, **kw):
-    """pp_pipeline for a host trace of any accepted dtype: float32 traces stream through the chunked host call,
-    float64 ones are uploaded whole (8 B per sample) and run resident."""
+    """pp_pipeline for a host trace of any accepted dtype: float32 traces and AdcTraces stream through the chunked
+    host call, float64 ones are uploaded whole (8 B per sample) and run resident."""
+    if isinstance(x, AdcTrace):
+        return ctx.pipeline(threshold, host_trace=x, **kw)
     dev = _device_trace(x)
     if dev.dtype == np.float32:
         return ctx.pipeline(threshold, host_trace=dev, **kw)
