@@ -222,6 +222,12 @@ int pp_split_counters(pp_ctx *ctx, int64_t out[8]);
  * pe-ps-2*min_width+1 entries.  eps receives the bound the kernel applies to this window. */
 int pp_debug_screen(pp_ctx *ctx, int64_t ev, int ps, int pe, int min_width, double *h_screen,
                     double *h_exact, uint8_t *ok, double *eps);
+/* Validation: the resident prefix sums (K2) of all events, de-interleaved into c (cumsum of x) and c2 (cumsum of
+ * x*x), n_event_samples entries each in flat event space, and per event whether the strict-order kernel computed
+ * them: the exactness verdict under PP_PREFIX_AUTO, all 0 under PP_PREFIX_PARALLEL, all 1 under
+ * PP_PREFIX_SEQUENTIAL.  cap bounds both lengths.  PP_ERR_STATE unless pp_prefix / pp_statsplit ran on the current
+ * events. */
+int pp_debug_prefix(pp_ctx *ctx, int64_t cap, double *c, double *c2, uint8_t *redone);
 
 /* Validation hook for the hardware term of the screening bound: the largest absolute error,
  * over all 2^23 float32 mantissas in [1, 2), of the 23-bit fixed-point log2 the screening

@@ -101,6 +101,7 @@ SIGNATURES = {
     "pp_table_device_ptr": (_c.c_void_p, [_c.c_void_p, _c.c_int]),
     "pp_split_counters": (_c.c_int, [_c.c_void_p, _i64p]),
     "pp_debug_screen": (_c.c_int, [_c.c_void_p, _i64, _c.c_int, _c.c_int, _c.c_int, _f64p, _f64p, _u8p, _f64p]),
+    "pp_debug_prefix": (_c.c_int, [_c.c_void_p, _i64, _f64p, _f64p, _u8p]),
     "pp_debug_lg2_error": (_c.c_int, [_c.c_void_p, _f64p]),
     "pp_stream": (_c.c_void_p, [_c.c_void_p]),
     "pp_trace_prefetch_ms": (_c.c_int, [_c.c_void_p, _c.POINTER(_c.c_float)]),
@@ -505,6 +506,14 @@ class Context(object):
         self._ck(self._L.pp_debug_screen(self._h, int(ev), int(ps), int(pe), int(min_width), _ptr(hs, _f64p),
                                          _ptr(he, _f64p), _ptr(ok, _u8p), _c.byref(eps)))
         return hs, he, ok.astype(bool), float(eps.value)
+
+    def debug_prefix(self, n_events, n_samples):
+        """The resident prefix sums (c = cumsum(x), c2 = cumsum(x*x), flat event space) and, per event, whether
+        the strict-order kernel computed them."""
+        cap = max(int(n_events), int(n_samples))
+        c, c2, redone = np.empty(cap), np.empty(cap), np.empty(cap, np.uint8)
+        self._ck(self._L.pp_debug_prefix(self._h, cap, _ptr(c, _f64p), _ptr(c2, _f64p), _ptr(redone, _u8p)))
+        return c[:n_samples], c2[:n_samples], redone[:n_events].astype(bool)
 
     def debug_lg2_error(self):
         v = _c.c_double()

@@ -102,6 +102,7 @@ struct pp_ctx {
     bool stats_valid = false;
     int64_t split_counters[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     bool prefix_valid = false;  // cc holds the prefix sums of the current events
+    int prefix_mode = PP_PREFIX_AUTO;  // mode of the last K2 run (what `inexact` means for pp_debug_prefix)
 
     // event stats
     DevBuf evs_mean, evs_std, evs_min, evs_max;
@@ -420,7 +421,7 @@ int enqueue_filter(pp_ctx *ctx, const double *b, const double *a, const double *
         switch (nc - 1) {
         case 1: launch_filter_pass<1>(ctx, src, backward); break;
         case 2: launch_filter_pass<2>(ctx, src, backward); break;
-        case 3: launch_filter_pass<3>(ctx, src, backward); break;
+        case 3: launch_filter_sequential<3>(ctx, src, backward); break;
         case 4: launch_filter_sequential<4>(ctx, src, backward); break;
         case 5: launch_filter_sequential<5>(ctx, src, backward); break;
         case 6: launch_filter_sequential<6>(ctx, src, backward); break;
@@ -517,6 +518,7 @@ int enqueue_prefix(pp_ctx *ctx, int prefix_mode)
     StageRange nvtx_range("pypore:prefix");
     const int64_t ncap = ctx->flat_cap;
     PPSource src = make_source(ctx);
+    ctx->prefix_mode = prefix_mode;
     if (prefix_mode == PP_PREFIX_SEQUENTIAL) {
         k2_prefix_sequential<<<ctx->sm_count * 3, K2S_WARPS * 32, 0, ctx->stream>>>(
             src, (const int64_t *)ctx->ev_len.p, ctx->ctr, nullptr, (double2 *)ctx->cc.p);
@@ -1440,6 +1442,34 @@ int pp_debug_screen(pp_ctx *ctx, int64_t ev, int ps, int pe, int min_width, doub
     release(a); release(b); release(c);
     if (eps) *eps = (double)(pe - ps) * K3_EPS_PER_SAMPLE + K3_EPS_CONST;
     return PP_OK;
+}
+
+int pp_debug_prefix(pp_ctx *ctx, int64_t cap, double *c, double *c2, uint8_t *redone)
+{
+    if (!ctx || !c || !c2 || !redone) return PP_ERR_ARG;
+    if (!ctx->prefix_valid) return fail(ctx, PP_ERR_STATE, "prefix sums are not resident (pp_prefix / pp_statsplit)");
+    if (cap < ctx->n_event_samples || cap < ctx->n_events) return fail(ctx, PP_ERR_CAPACITY, "buffers too small");
+    CKR(set_device(ctx));
+    const size_t n = (size_t)ctx->n_event_samples, e = (size_t)ctx->n_events;
+    double2 *cc = (double2 *)malloc(sizeof(double2) * (n ? n : 1));
+    unsigned *fl = (unsigned *)malloc(sizeof(unsigned) * (e ? e : 1));
+    if (!cc || !fl) { free(cc); free(fl); return fail(ctx, PP_ERR_ARG, "out of host memory"); }
+    auto run = [&]() -> int {
+        if (n) CK(cudaMemcpyAsync(cc, ctx->cc.p, sizeof(double2) * n, cudaMemcpyDeviceToHost, ctx->stream));
+        if (e && ctx->prefix_mode == PP_PREFIX_AUTO)
+            CK(cudaMemcpyAsync(fl, ctx->inexact.p, sizeof(unsigned) * e, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        return PP_OK;
+    };
+    const int rc = run();
+    if (rc == PP_OK) {
+        for (size_t i = 0; i < n; ++i) { c[i] = cc[i].x; c2[i] = cc[i].y; }
+        // PARALLEL redoes nothing, SEQUENTIAL runs every event in the strict order
+        for (size_t i = 0; i < e; ++i)
+            redone[i] = ctx->prefix_mode == PP_PREFIX_AUTO ? (fl[i] != 0u) : ctx->prefix_mode == PP_PREFIX_SEQUENTIAL;
+    }
+    free(cc); free(fl);
+    return rc;
 }
 
 int pp_debug_lg2_error(pp_ctx *ctx, double *max_err)

@@ -305,7 +305,8 @@ k2_event_scan(PPSource src, const T *__restrict__ samples, const int64_t *__rest
             for (int k = 0; k < K2F_ITEMS; ++k) {
                 const T xs = sin[lane * K2F_PAD + k];
                 const double x = pp_val(xs, src.adc);
-                if constexpr (sizeof(T) == 4) fb.add(xs); else ex.add(x);
+                // padding decodes to the ADC offset, which is no sample of the event: kept out of the proof
+                if constexpr (sizeof(T) == 4) fb.add(xs); else if (lane * K2F_ITEMS + k < cnt) ex.add(x);
                 c = __dadd_rn(c, x);
                 c2 = __dadd_rn(c2, __dmul_rn(x, x));
                 pc[k] = c; pc2[k] = c2;
@@ -461,7 +462,7 @@ k2_tile_reduce(PPSource src, const T *__restrict__ samples /* the trace, or flat
 #pragma unroll
         for (int i = 0; i < K2_ITEMS; ++i) {
             const double x = pp_val(xv[i], src.adc);
-            if constexpr (sizeof(T) == 4) ex.add(xv[i]); else ex.add(x);
+            if constexpr (sizeof(T) == 4) ex.add(xv[i]); else if (i * K2_THREADS + tid < t.cnt) ex.add(x);
             c = __dadd_rn(c, x);
             c2 = __dadd_rn(c2, __dmul_rn(x, x));
         }

@@ -4,15 +4,23 @@
 // A group of G lanes (8 for short rows, 32 for long ones) owns one row (segment or event).
 // std is computed from deviations, never from prefix-sum differences (SURVEY App. D.3):
 //   * rows of at most K4_ONE_PASS samples: ONE pass with the shift K = the row's first sample:
-//     d = x - K,  mean = K + sum(d)/n,  var = sum(d*d)/n - (sum(d)/n)^2.  The cancellation in the
-//     last line is bounded by 1 + (K - mean)^2 / var <= 1 + n (K is one of the samples, so
-//     (K - mean)^2 <= n var), i.e. a relative error of var below ~4 (1 + n) 2^-53 < 3e-11 for
-//     n <= 65536: std stays within 1e-9 even when the first sample is the worst outlier of the row;
+//     d = x - K,  m1 = sum(d)/n,  mean = K + m1,  var = sum(d*d)/n - m1^2.  Each lane adds k = n/G terms
+//     and the group adds its G lane sums, so with u = 2^-53 the sums carry errors up to
+//     (k + log2 G) u sum|d| and (k + log2 G) u sum(d*d) (sum(d*d) = n (var + m1^2)).  Hence
+//       |error of mean| <~ (k + log2 G + 2) u (|m1| + sqrt(var))   (mean|d| <= |m1| + sqrt(var)),
+//       relative error of var <~ (k + log2 G + 3) u (1 + m1^2 / var).
+//     Both grow with m1^2 / var = (K - mean)^2 / var, which reaches n when K is the row's worst outlier:
+//     at n = 65536 the first-order bounds are ~1e-6 and the errors were measured at several 1e-9 (one
+//     float32 sample of 1000.123 followed by 65,535 samples of 1e-3).  So a row with m1^2 > 2^10 var is
+//     summed again in two passes (next point); below that the var bound is 1025 (k + 8) u < 1e-9 and the
+//     mean error < 33 (k + 7) u sqrt(var), no more than the two-pass sum's own (k + 5) u mean|x| allows
+//     for a row whose spread is not tiny against its mean.  Constant rows come out exact (d = 0);
 //   * samples travel as 16-byte vectors (float4 / double2) from the row's 16-byte-aligned start, the
 //     elements in front of and behind the row are masked: a row of ~130 float32 samples is 5 trips of an
 //     8-lane group instead of 17 (the first cut issued 32 thread instructions per sample, most of them
 //     per-row set-up and scalar loads: 31 % of the HBM peak);
-//   * longer rows: two passes (mean first, then deviations from it), like np.std.
+//   * longer rows (every row of a warp that holds one) and the rows above: two passes (mean = sum(x)/n, then
+//     the deviations from it), like np.std, from scalar loads; a finite constant row gets its value and 0.
 // min / max run on the samples' own type (int16 ADC counts: on the counts, decoded at the end); a NaN anywhere
 // makes both NaN like np.min / np.max.
 #pragma once
@@ -135,7 +143,9 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
         T mn = k4_top<T>(), mx = k4_bottom<T>();
         int nan = 0;
         double mean, var;
-        if (__all_sync(PP_FULL, len <= K4_ONE_PASS)) {
+        const bool one_pass = __all_sync(PP_FULL, len <= K4_ONE_PASS);
+        bool redo = !one_pass;  // this group's row takes the two passes
+        if (one_pass) {
             // 16-byte vectors from the aligned start: `mis` elements of the first vector lie in front of the row
             const int mis = (int)((reinterpret_cast<uintptr_t>(p) & 15) / sizeof(T));
             const typename VT::V *pv = reinterpret_cast<const typename VT::V *>(p - mis);
@@ -186,25 +196,37 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
             mean = K + m1;
             var = s2 * rl - m1 * m1;
             if (len == 0) { mean = __longlong_as_double(0x7ff8000000000000LL); var = mean; }
-        } else {
-            for (int64_t j = gl; j < len; j += G) {
+            redo = m1 * m1 > 1024.0 * var;  // heavy cancellation: the shift sits far from the mean (false for NaN)
+        }
+        if (__any_sync(PP_FULL, redo)) {
+            // rows of the other groups run with length 0: the group sums below are warp-wide
+            const int64_t n2 = redo ? len : 0;
+            double t1 = 0.0, t2 = 0.0;
+            for (int64_t j = gl; j < n2; j += G) {
                 const T x = p[j];
-                s1 += pp_val(x, adc);
-                mn = k4_min(mn, x);
-                mx = k4_max(mx, x);
-                nan |= (x != x);
+                t1 += pp_val(x, adc);
+                if (!one_pass) {
+                    mn = k4_min(mn, x);
+                    mx = k4_max(mx, x);
+                    nan |= (x != x);
+                }
             }
-            mean = k4_group_sum<G>(s1) / (double)len;
-            for (int64_t j = gl; j < len; j += G) {
-                const double d = pp_val(p[j], adc) - mean;
-                s2 = fma(d, d, s2);
+            const double m2 = k4_group_sum<G>(t1) / (double)len;
+            for (int64_t j = gl; j < n2; j += G) {
+                const double d = pp_val(p[j], adc) - m2;
+                t2 = fma(d, d, t2);
             }
-            var = k4_group_sum<G>(s2) / (double)len;
+            t2 = k4_group_sum<G>(t2);
+            if (redo) { mean = m2; var = t2 / (double)len; }
         }
         mn = k4_group_min<G>(mn);
         mx = k4_group_max<G>(mx);
 #pragma unroll
         for (int d = G / 2; d > 0; d >>= 1) nan |= __shfl_xor_sync(PP_FULL, nan, d);
+        if (!one_pass && !nan && mn == mx) {  // a finite constant row: its value and exactly 0, as in one pass
+            const double v = pp_val(mn, adc);
+            if (fabs(v) <= 1.7e308) { mean = v; var = 0.0; }
+        }
         if (live && gl == 0) {
             const double qnan = __longlong_as_double(0x7ff8000000000000LL);
             double dmn = pp_val(mn, adc), dmx = pp_val(mx, adc);

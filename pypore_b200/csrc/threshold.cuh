@@ -680,6 +680,7 @@ k1_event_offsets(PPCounters *ctr, const int64_t *__restrict__ ev_len, int64_t n_
         ctr->n_events = (unsigned long long)n_events;
         ctr->n_event_samples = (unsigned long long)s_carry;
         ctr->ev_begin = 0;
+        ctr->overflow &= ~(unsigned)PP_OVF_FILTER_SHORT;  // a refused filter spoke of the previous events
     }
 }
 

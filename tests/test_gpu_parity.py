@@ -491,8 +491,8 @@ def test_filter_edge_lengths_and_orders(ctx):
             got = y[k:k + len(e)]
             err = np.max(np.abs(got - ref) / np.abs(ref))
             assert err < FILTER_RTOL, (order, len(e), err)
-            # orders 1-3: parallel scan (rounding differs from the sequential order, measured <= 2e-9);
-            # orders 4-8: scipy's own operation order, bit-identical to the oracle
+            # orders 1-2: parallel scan (rounding differs from the sequential order, measured <= 2e-9);
+            # orders 3-8: scipy's own operation order, bit-identical to the oracle
             assert err < (1e-8 if order <= 3 else 1e-15), (order, len(e), err)
             k += len(e)
         # not longer than padlen: scipy raises ValueError
