@@ -92,6 +92,8 @@ enum pp_option {
     PP_OPT_SPLIT_KERNEL = 3
 };
 int pp_set_option(pp_ctx *ctx, int option, int64_t value);
+/* The current value of an option (so that a caller can restore it). */
+int pp_get_option(pp_ctx *ctx, int option, int64_t *value);
 /* Number of kernel launches this context has issued since creation. */
 int64_t pp_launch_count(pp_ctx *ctx);
 /* Milliseconds between two internal CUDA events bracketing the named stage of
@@ -213,7 +215,14 @@ const void *pp_table_device_ptr(pp_ctx *ctx, int which);
 /* Work counters of the last pp_statsplit: [0] candidate evaluations (same count
  * as the reference's inner loop), [1] window scans, [2] events whose prefix sums
  * were redone sequentially, [3] queue tasks processed, [4] candidates evaluated
- * with the exact reference arithmetic after screening, [5..7] reserved. */
+ * with the exact reference arithmetic after screening.  How the screened search
+ * decided its windows (all 0 with PP_OPT_SCREEN = 0): [5] on the screened gain
+ * alone (one contender, clear of min_gain by more than the error bound), [6] by
+ * the argmax over the exact gains of several contenders (re-screened pieces
+ * included), [7] by an exact scan of every candidate (a candidate failed the
+ * validity test, the window cannot be screened, or its exact-evaluation requests
+ * overflowed).  Windows with one contender evaluated exactly count in none of
+ * [5..7].  The sharded multi-GPU path reports [0], [1] and [4] only. */
 int pp_split_counters(pp_ctx *ctx, int64_t out[8]);
 
 /* Validation hook for the screening bound: for window [ps,pe) of event `ev` (prefix sums

@@ -283,6 +283,75 @@ def score_samples(event, no_split=False, min_width=100, max_width=1000000, windo
     return rec(0, L, no_split)
 
 
+EPS_PER_SAMPLE, EPS_CONST = 3.6e-7, 1e-6   # the device's screening error bound (split.cuh K3_EPS_*), nats
+
+
+def scan_log(event, min_width=100, max_width=1000000, window_width=10000, gain=None, **gain_kwargs):
+    """One record per window scan of FastStatSplit.parse (cparsers.pyx:157-203), in the C oracle's arithmetic.
+
+    Walks the recursion like score_samples (explicit stack: any order gives the same scans).  Each record is a dict:
+    ps, pe, x (the split, -1 for none: first occurrence of the largest gain above min_gain, NaN never wins), best /
+    best_i (largest non-NaN gain, first occurrence; -inf / -1 if every gain is NaN), second / second_i (largest
+    non-NaN gain at another candidate), n_nan, n_posinf, n_near (candidates within 2 eps(n) of best, eps(n) =
+    n * EPS_PER_SAMPLE + EPS_CONST) and gains (every candidate ps+mw .. pe-mw).  Also returns the breakpoints,
+    sorted, and the work counters (ncand, nscan) of statsplit(return_info=True)."""
+    x = _f64(event)
+    if gain is None:
+        gain = min_gain(min_width, max_width, window_width, **gain_kwargs)
+    mw, MW, W = int(min_width), int(max_width), int(window_width)
+    c, c2 = cumsum(x)
+    log, bps = [], []
+    stack = [(0, x.shape[0])]
+    while stack:
+        start, end = stack.pop()
+        split_at, forced_right = -1, False
+        for ps in range(start, end - 2 * mw, W // 2):
+            if ps > start + MW:
+                split_at, forced_right = min(start + MW, end - mw), True
+                break
+            pe = min(end, ps + W)
+            if pe - ps <= 2 * mw:
+                continue
+            g = _window_gains(c, c2, ps, pe, ps + mw, pe - mw)
+            r = dict(ps=ps, pe=pe, x=_sequential_best(g, gain, ps + mw)[1], gains=g)
+            ok = ~np.isnan(g)
+            r["n_nan"] = int((~ok).sum())
+            r["n_posinf"] = int(np.isposinf(g).sum())
+            r["best"], r["best_i"], r["second"], r["second_i"], r["n_near"] = -np.inf, -1, -np.inf, -1, 0
+            if ok.any():
+                j = int(np.argmax(np.where(ok, g, -np.inf)))
+                if not ok[j]:
+                    j = int(np.flatnonzero(ok)[0])
+                r["best"], r["best_i"] = float(g[j]), ps + mw + j
+                rest = ok.copy()
+                rest[j] = False
+                if rest.any():
+                    k = int(np.argmax(np.where(rest, g, -np.inf)))
+                    if not rest[k]:
+                        k = int(np.flatnonzero(rest)[0])
+                    r["second"], r["second_i"] = float(g[k]), ps + mw + k
+                n = pe - ps
+                with np.errstate(invalid="ignore"):
+                    r["n_near"] = int((g[ok] >= r["best"] - 2 * (n * EPS_PER_SAMPLE + EPS_CONST)).sum())
+            log.append(r)
+            split_at = r["x"]
+            if split_at >= 0:
+                break
+        if forced_right:
+            bps.append(split_at)
+            stack.append((split_at, end))
+            continue
+        if split_at == -1:
+            if end - start <= MW:
+                continue
+            split_at = min(start + MW, end - mw)
+        bps.append(split_at)
+        stack.append((split_at, end))
+        stack.append((start, split_at))
+    ncand = int(sum(len(r["gains"]) for r in log))
+    return log, np.sort(np.asarray(bps, np.int64)), dict(ncand=ncand, nscan=len(log))
+
+
 def statsplit_events(trace, ev_start, ev_len, min_width=100, max_width=1000000, window_width=10000,
                      gain=None, threads=1, **gain_kwargs):
     """FastStatSplit over many events of one float64 trace.

@@ -69,6 +69,7 @@ SIGNATURES = {
     "pp_last_error": (_c.c_char_p, [_c.c_void_p]),
     "pp_sync": (_c.c_int, [_c.c_void_p]),
     "pp_set_option": (_c.c_int, [_c.c_void_p, _c.c_int, _i64]),
+    "pp_get_option": (_c.c_int, [_c.c_void_p, _c.c_int, _i64p]),
     "pp_launch_count": (_i64, [_c.c_void_p]),
     "pp_stage_ms": (_c.c_int, [_c.c_void_p, _c.c_int, _c.POINTER(_c.c_float)]),
     "pp_trace_upload": (_c.c_int, [_c.c_void_p, _c.c_void_p, _i64, _i64]),
@@ -340,6 +341,11 @@ class Context(object):
     def set_option(self, option, value):
         self._ck(self._L.pp_set_option(self._h, int(option), int(value)))
 
+    def get_option(self, option):
+        v = _i64()
+        self._ck(self._L.pp_get_option(self._h, int(option), _c.byref(v)))
+        return int(v.value)
+
     def set_screening(self, on):
         """Two-stage split search (default on); off = exact arithmetic for every candidate."""
         self.set_option(0, 1 if on else 0)
@@ -497,7 +503,7 @@ class Context(object):
         out = np.zeros(8, np.int64)
         self._ck(self._L.pp_split_counters(self._h, _ptr(out, _i64p)))
         return dict(candidates=int(out[0]), scans=int(out[1]), seq_redo=int(out[2]), tasks=int(out[3]),
-                    exact=int(out[4]))
+                    exact=int(out[4]), sure=int(out[5]), multi=int(out[6]), full=int(out[7]))
 
     def debug_screen(self, ev, ps, pe, min_width):
         n = pe - ps - 2 * min_width + 1

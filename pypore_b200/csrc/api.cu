@@ -707,6 +707,9 @@ void absorb_counters(pp_ctx *ctx)
     ctx->split_counters[2] = (int64_t)h->n_seq_redo;
     ctx->split_counters[3] = (int64_t)h->n_tasks;
     ctx->split_counters[4] = (int64_t)h->n_exact;
+    ctx->split_counters[5] = (int64_t)h->n_sure;
+    ctx->split_counters[6] = (int64_t)h->n_multi;
+    ctx->split_counters[7] = (int64_t)h->n_full;
 }
 
 }  // namespace
@@ -833,6 +836,18 @@ int pp_set_option(pp_ctx *ctx, int option, int64_t value)
         if (value < 0 || value > (1 << 20)) return fail(ctx, PP_ERR_ARG, "bad CTA count %lld", (long long)value);
         ctx->opt_split_ctas = (int)value;
         return PP_OK;
+    default: return fail(ctx, PP_ERR_ARG, "unknown option %d", option);
+    }
+}
+
+int pp_get_option(pp_ctx *ctx, int option, int64_t *value)
+{
+    if (!ctx || !value) return PP_ERR_ARG;
+    switch (option) {
+    case PP_OPT_SCREEN: *value = ctx->opt_screen; return PP_OK;
+    case PP_OPT_SPINE: *value = ctx->opt_spine; return PP_OK;
+    case PP_OPT_SPLIT_KERNEL: *value = ctx->opt_split_kernel; return PP_OK;
+    case PP_OPT_SPLIT_CTAS: *value = ctx->opt_split_ctas; return PP_OK;
     default: return fail(ctx, PP_ERR_ARG, "unknown option %d", option);
     }
 }

@@ -26,6 +26,9 @@ struct PPCounters {
     unsigned long long n_scan;        // window scans
     unsigned long long n_tasks;       // tasks processed
     unsigned long long n_exact;       // exact (reference-arithmetic) candidate evaluations
+    unsigned long long n_sure;        // screened windows decided on the screened gain alone
+    unsigned long long n_multi;       // screened windows decided by the argmax over several contenders' exact gains
+    unsigned long long n_full;        // windows scanned exactly in full although screening was on
     unsigned long long n_seq_redo;    // events whose prefix sums were redone sequentially
     unsigned long long n_scan_tiles;  // prefix-scan tiles over all events
     // incremental (streamed) pipeline: the stages after the threshold scan work on the events

@@ -111,6 +111,9 @@ struct K3Item { int s, e, ps, pad; };  // interval and the start of the window t
 struct K3Params { int mw, MW, W; double min_gain; };
 struct K3Best { double g; int x; };
 struct K3Scr { unsigned long long k1, k2; int i1, bad; };  // per-lane screening state: two smallest keys
+// How screened windows were decided (PPCounters::n_sure / n_multi / n_full): on the screened gain alone, by the
+// argmax over several contenders' exact gains, or by an exact scan of every candidate.
+struct K3Branches { unsigned sure, multi, full; };
 
 struct K3Global {
     const double2 *cc;
@@ -171,6 +174,8 @@ struct K3Shared {
     int ebase;                             // biased exponent of the task's variance - 127, or K3_NO_EBASE
     PPTask task;
     unsigned long long cand, scans, exact;
+    unsigned n_sure, n_multi, n_full;      // decision branches over all tasks of the CTA (PPCounters::n_sure ..)
+    unsigned n_cont;                       // contenders of the window k3_cta_scan is deciding
     K3Global G;                            // copies of the kernel parameters for the out-of-line bookkeeping
     K3Params P;
 };
@@ -607,6 +612,7 @@ __device__ __forceinline__ K3Best k3_cta_scan(const CC &cc, int ps, int pe, cons
         if (__syncthreads_or(a.bad)) screen = false;
     }
     if (!screen) {
+        if (tid == 0 && G.screen && P.mw >= 1 && P.W <= K3_MAX_SCREEN_W) S.n_full += 1;
         b = k3_scan_range(cc, ps, pe, P.mw, P.min_gain, tid, K3_THREADS);
         return k3_cta_reduce(b, S);
     }
@@ -617,6 +623,9 @@ __device__ __forceinline__ K3Best k3_cta_scan(const CC &cc, int ps, int pe, cons
 #pragma unroll
     for (int w = 1; w < K3_WARPS; ++w) m = S.red_k[w] < m ? S.red_k[w] : m;
     const unsigned long long thr = m + k3_eps2_key(pe - ps);
+    // contenders of the window, summed in shared memory behind the barriers of k3_cta_reduce (no barrier of its own)
+    const unsigned ncont = (a.k1 <= thr ? 1u : 0u) + (a.k2 <= thr ? 1u : 0u);
+    if (ncont) atomicAdd(&S.n_cont, ncont);
     unsigned nexact = 0;
     if (a.k2 <= thr) {
         // rare: several of this thread's candidates qualify -> rescan its subset
@@ -636,7 +645,12 @@ __device__ __forceinline__ K3Best k3_cta_scan(const CC &cc, int ps, int pe, cons
         if (g > b.g) { b.g = g; b.x = a.i1; }
     }
     if (nexact) atomicAdd(&S.exact, (unsigned long long)nexact);
-    return k3_cta_reduce(b, S);
+    b = k3_cta_reduce(b, S);
+    if (tid == 0) {  // every thread's contribution is in (barriers of k3_cta_reduce); reset before the next window's
+        if (S.n_cont > 1) S.n_multi += 1;  // several contenders: the lowest index among equal exact gains wins
+        S.n_cont = 0;
+    }
+    return b;
 }
 
 // ---------------------------------------------------------------------------
@@ -654,7 +668,9 @@ __device__ __forceinline__ bool k3_worth(const K3Params &P, int s, int e)
     return ((long long)e - s > 2LL * P.mw) || (e - s > P.MW);
 }
 
-__device__ void k3_push_global(const K3Global &G, int ev, int s, int e)
+// Interval [s,e) of event ev for any CTA; its window loop resumes at ps (the windows before ps were scanned
+// without a split).
+__device__ void k3_push_global(const K3Global &G, int ev, int s, int e, int ps)
 {
     atomicAdd((unsigned long long *)&G.ctr->q_pending, 1ull);
     const unsigned long long slot = atomicAdd(&G.ctr->q_tail, 1ull);
@@ -664,7 +680,7 @@ __device__ void k3_push_global(const K3Global &G, int ev, int s, int e)
         return;
     }
     PPTask t;
-    t.ev = ev; t.s = s; t.e = e; t.flags = 0;
+    t.ev = ev; t.s = s; t.e = e; t.flags = ps - s;
     *reinterpret_cast<int4 *>(&G.tasks[slot]) = *reinterpret_cast<int4 *>(&t);
     __threadfence();
     atomicExch(&G.ready[slot], 1);
@@ -723,7 +739,7 @@ __device__ __noinline__ void k3_place(K3Shared *Sp, K3Level *nxp, K3Count *ncp, 
                     r.s = x; r.e = it.e; r.ps = x; r.pad = 0;
                     const bool wl = k3_worth(P, l.s, l.e), wr = k3_worth(P, r.s, r.e);
                     if (wl && wr) {
-                        if (sp < 4) st[sp++] = r; else k3_push_global(G, S.ev, r.s, r.e);
+                        if (sp < 4) st[sp++] = r; else k3_push_global(G, S.ev, r.s, r.e, r.ps);
                         it = l;
                         continue;
                     }
@@ -750,7 +766,9 @@ __device__ __noinline__ void k3_place(K3Shared *Sp, K3Level *nxp, K3Count *ncp, 
             const unsigned old = atomicAdd(&nc.alloc, K3_ALLOC_SLOT | nch);
             const unsigned slot = old >> 20;
             if (slot >= (unsigned)K3_LIST) {
-                k3_push_global(G, S.ev, it.s, it.e);  // restart at ps = s elsewhere: redundant scans, same result
+                // the level is full: another CTA continues the interval at the same window, so no window is
+                // scanned twice and the work counters stay the reference's
+                k3_push_global(G, S.ev, it.s, it.e, it.ps);
                 break;
             }
             nx.item[slot] = it;
@@ -797,7 +815,7 @@ void k3_resolve(const K3Global &G, K3Shared &S, K3Level &nx, K3Count &nc,
             bool away = K3_SHARE > 0 && x - it.s >= K3_SHARE && it.e - x >= K3_SHARE;
             if (!away && K3_IDLE_SHARE > 0 && S.share > 0 && x - it.s >= K3_IDLE_SHARE && it.e - x >= K3_IDLE_SHARE)
                 away = atomicSub(&S.share, 1) > 0;
-            if (away) k3_push_global(G, S.ev, x, it.e);
+            if (away) k3_push_global(G, S.ev, x, it.e, x);
             else { c.s = x; c.e = it.e; c.ps = x; k3_place(&S, &nx, &nc, screen, c); }
         }
     } else {
@@ -913,6 +931,7 @@ __global__ void __launch_bounds__(K3_THREADS, K3_CTAS_PER_SM) k3_split(K3Global 
         S.G = G;
         S.P = P;
         S.few = ((long long)G.ctr->n_events - (long long)G.ctr->ev_begin) < 2LL * gridDim.x ? 1 : 0;
+        S.n_sure = 0; S.n_multi = 0; S.n_full = 0; S.n_cont = 0;
     }
     if (tid == 0 && blockIdx.x == 0) G.ctr->n_long = 0ull;  // k3_spine is done with it; ready for the next search
     for (;;) {
@@ -971,7 +990,7 @@ __global__ void __launch_bounds__(K3_THREADS, K3_CTAS_PER_SM) k3_split(K3Global 
                     const int x = k3_forced(P, s, e);
                     if (tid == 0) {
                         k3_emit(G, off, x);
-                        if (k3_worth(P, s, x)) k3_push_global(G, ev, s, x);
+                        if (k3_worth(P, s, x)) k3_push_global(G, ev, s, x, s);
                     }
                     s = x; ps = s;
                     continue;
@@ -993,7 +1012,7 @@ __global__ void __launch_bounds__(K3_THREADS, K3_CTAS_PER_SM) k3_split(K3Global 
                 if (b.x >= 0) {
                     if (tid == 0) {
                         k3_emit(G, off, b.x);
-                        if (k3_worth(P, s, b.x)) k3_push_global(G, ev, s, b.x);
+                        if (k3_worth(P, s, b.x)) k3_push_global(G, ev, s, b.x, s);
                     }
                     s = b.x; ps = s;
                 } else {
@@ -1079,8 +1098,11 @@ __global__ void __launch_bounds__(K3_THREADS, K3_CTAS_PER_SM) k3_split(K3Global 
                         const double d = (double)(long long)(kt - gmin);
                         const double want = P.min_gain * K3_KEY_PER_NAT;
                         const double margin = (double)eps2 + 64.0;
-                        if (d > want + margin) { k3_resolve(G, S, NX, NC, P, screen, it, i_one, 1); continue; }
-                        if (d < want - margin) { k3_resolve(G, S, NX, NC, P, screen, it, -1, 1); continue; }
+                        if (d > want + margin || d < want - margin) {
+                            atomicAdd(&S.n_sure, 1u);
+                            k3_resolve(G, S, NX, NC, P, screen, it, d > want ? i_one : -1, 1);
+                            continue;
+                        }
                     }
                 }
 #endif
@@ -1166,8 +1188,10 @@ __global__ void __launch_bounds__(K3_THREADS, K3_CTAS_PER_SM) k3_split(K3Global 
                     __syncthreads();
                     for (int k = tid; k < nwin; k += K3_THREADS) {
                         const int fl = L.flag[k];
-                        if ((fl & K3_MULTI_FLAG) && !(fl & K3_FULL_FLAG))
+                        if ((fl & K3_MULTI_FLAG) && !(fl & K3_FULL_FLAG)) {
+                            atomicAdd(&S.n_multi, 1u);
                             k3_resolve(G, S, NX, NC, P, screen, L.item[k], S.best_key[k] ? S.best_idx[k] : -1, 1);
+                        }
                     }
                 }
             }
@@ -1182,7 +1206,10 @@ __global__ void __launch_bounds__(K3_THREADS, K3_CTAS_PER_SM) k3_split(K3Global 
                     K3Best b = k3_scan_range(acc, it.ps, pe, mw, P.min_gain, tid, K3_THREADS);
                     b = k3_cta_reduce(b, S);
                     if (tid == 0) {
-                        if (screen) atomicAdd(&S.exact, (unsigned long long)(pe - it.ps - 2 * mw + 1));
+                        if (screen) {
+                            atomicAdd(&S.exact, (unsigned long long)(pe - it.ps - 2 * mw + 1));
+                            S.n_full += 1;
+                        }
                         k3_resolve(G, S, NX, NC, P, screen, it, b.x);
                     }
                 }
@@ -1200,6 +1227,11 @@ __global__ void __launch_bounds__(K3_THREADS, K3_CTAS_PER_SM) k3_split(K3Global 
             __threadfence();
             atomicAdd((unsigned long long *)&G.ctr->q_pending, (unsigned long long)(-1LL));
         }
+    }
+    if (tid == 0) {
+        if (S.n_sure) atomicAdd(&G.ctr->n_sure, (unsigned long long)S.n_sure);
+        if (S.n_multi) atomicAdd(&G.ctr->n_multi, (unsigned long long)S.n_multi);
+        if (S.n_full) atomicAdd(&G.ctr->n_full, (unsigned long long)S.n_full);
     }
 }
 
@@ -1285,7 +1317,8 @@ __device__ __forceinline__ K3Best k3_spine_reduce(K3Best b, K3SpineShared &S, in
 
 // One window [ps,pe) scanned by the whole cluster; every thread returns the same split position (or -1).
 __device__ __forceinline__ int k3_spine_scan(const K3GlobalCC &acc, int ps, int pe, const K3Params &P, const K3Global &G,
-                                             K3SpineShared &S, int ebase, bool screen, int par, unsigned &nexact)
+                                             K3SpineShared &S, int ebase, bool screen, int par, unsigned &nexact,
+                                             K3Branches &br)
 {
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
@@ -1351,9 +1384,10 @@ __device__ __forceinline__ int k3_spine_scan(const K3GlobalCC &acc, int ps, int 
                 const double d = (double)(long long)(kt - gmin);
                 const double want = P.min_gain * K3_KEY_PER_NAT;
                 const double margin = (double)eps2 + 64.0;
-                if (d > want + margin) return i_one;
-                if (d < want - margin) return -1;
+                if (d > want + margin) { ++br.sure; return i_one; }
+                if (d < want - margin) { ++br.sure; return -1; }
             }
+            if (rescan || nr > 1) ++br.multi;
             // contenders in the reference's exact arithmetic
             K3Best b;
             b.g = P.min_gain;
@@ -1379,6 +1413,7 @@ __device__ __forceinline__ int k3_spine_scan(const K3GlobalCC &acc, int ps, int 
         }
     }
     // exact scan of every candidate (validation mode, or a candidate failed the validity test)
+    if (screen) ++br.full;
     K3Best b = k3_scan_range(acc, ps, pe, P.mw, P.min_gain, gtid, K3S_TOTAL);
     if (ps + P.mw + gtid <= pe - P.mw) nexact += (unsigned)((pe - P.mw - (ps + P.mw + gtid)) / K3S_TOTAL + 1);
     return k3_spine_reduce(b, S, par).x;
@@ -1462,6 +1497,8 @@ __global__ void __cluster_dims__(K3S_CLUSTER, 1, 1) __launch_bounds__(K3S_THREAD
             int s = 0, ps = 0;
             unsigned long long cand = 0, scans = 0;
             unsigned nexact = 0;
+            K3Branches br;
+            br.sure = br.multi = br.full = 0u;
             while ((long long)e - s > K3_CAP) {
                 const long long lim = (long long)e - 2LL * mw;
                 if (ps >= lim) {
@@ -1483,7 +1520,8 @@ __global__ void __cluster_dims__(K3S_CLUSTER, 1, 1) __launch_bounds__(K3S_THREAD
                 const long long pe_l = (long long)ps + W;
                 const int pe = (int)(pe_l < e ? pe_l : e);
                 if (pe - ps <= 2 * mw) { ps = k3_next_ps(P, ps, e); continue; }
-                const int x = k3_spine_scan(acc, ps, pe, P, G, S, ebase, screen, par, nexact);
+                const int x = k3_spine_scan(acc, ps, pe, P, G, S, ebase, screen, par, nexact, br);
+                if (screen_ok && !screen) ++br.full;  // the event's variance rules screening out
                 par ^= 1;
                 cand += (unsigned long long)(pe - ps - 2 * mw + 1);
                 scans += 1;
@@ -1507,6 +1545,9 @@ __global__ void __cluster_dims__(K3S_CLUSTER, 1, 1) __launch_bounds__(K3S_THREAD
             if (leader) {
                 atomicAdd(&G.ctr->n_cand, cand);
                 atomicAdd(&G.ctr->n_scan, scans);
+                if (br.sure) atomicAdd(&G.ctr->n_sure, (unsigned long long)br.sure);
+                if (br.multi) atomicAdd(&G.ctr->n_multi, (unsigned long long)br.multi);
+                if (br.full) atomicAdd(&G.ctr->n_full, (unsigned long long)br.full);
             }
         }
     }
@@ -1624,6 +1665,9 @@ k3_init_queue(K3Global G, int use_spine)
             G.ctr->n_scan = 0;
             G.ctr->n_tasks = 0;
             G.ctr->n_exact = 0;
+            G.ctr->n_sure = 0;
+            G.ctr->n_multi = 0;
+            G.ctr->n_full = 0;
         }
     }
 }

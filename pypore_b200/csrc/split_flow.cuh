@@ -104,6 +104,7 @@ struct K3FShared {
     K3Item lst[K3F_WARPS][K3F_LSTACK];   // private stacks of the warps
     int n_free, top, lock, fetching, drained, few, failed, pad;
     unsigned long long cand, scans, exact, tasks;
+    unsigned long long sure, multi, full;   // decision branches (PPCounters::n_sure ..)
     K3Global G;
     K3Params P;
 };
@@ -308,7 +309,8 @@ __device__ __noinline__ int f_contend(const double *RN, const double2 *ccg, int 
 // the summary of piece p (other lanes: K3_NOKEY / -1); pc = chunks per piece.
 __device__ __forceinline__ int f_decide(const K3Global &G, const K3Params &P, const double2 *ccg, const double2 lo,
                                         const double2 hi, int ps, int pe, int ebase, int np, int pc,
-                                        unsigned long long K1, unsigned long long K2, int I1, unsigned &nexact)
+                                        unsigned long long K1, unsigned long long K2, int I1, unsigned &nexact,
+                                        K3Branches &br)
 {
     const int lane = threadIdx.x & 31;
     const int mw = P.mw;
@@ -317,14 +319,17 @@ __device__ __forceinline__ int f_decide(const K3Global &G, const K3Params &P, co
     if (anybad || gmin == K3_NOKEY) {
         // a candidate failed the validity test: the whole window in the reference's arithmetic
         nexact += (unsigned)(pe - ps - 2 * mw + 1);
+        ++br.full;
         return f_exact_range(ccg, ps, pe, ps + mw + lane, pe - mw, P.min_gain).x;
     }
     const unsigned long long eps2 = k3_eps2_key(pe - ps);
     const unsigned long long thr = gmin + eps2;
     const unsigned rescan = __ballot_sync(PP_FULL, lane < np && K2 <= thr);
     const unsigned single = __ballot_sync(PP_FULL, lane < np && K2 > thr && K1 <= thr);
-    if (rescan || __popc(single) != 1)
+    if (rescan || __popc(single) != 1) {
+        ++br.multi;
         return f_contend(G.RN, ccg, ps, pe, mw, ebase, pc, P.min_gain, thr, single, rescan, I1, nexact);
+    }
     const int i_one = ps + (__shfl_sync(PP_FULL, I1, __ffs(single) - 1) & 0x1fffffff);
     unsigned long long kt = 0ull;
     const unsigned nw = (unsigned)(pe - ps);
@@ -334,14 +339,14 @@ __device__ __forceinline__ int f_decide(const K3Global &G, const K3Params &P, co
         const double d = (double)(long long)(kt - gmin);
         const double want = P.min_gain * K3_KEY_PER_NAT;
         const double margin = (double)eps2 + 64.0;
-        if (d > want + margin) return i_one;
-        if (d < want - margin) return -1;
+        if (d > want + margin) { ++br.sure; return i_one; }
+        if (d < want - margin) { ++br.sure; return -1; }
     }
     nexact += 1;
     return f_exact_one(ccg, ps, pe, i_one, P.min_gain) ? i_one : -1;
 }
 
-struct K3FTally { unsigned long long cand, scans, exact; };   // per warp, in registers; lane 0's copy counts
+struct K3FTally { unsigned long long cand, scans, exact; K3Branches br; };   // per warp, in registers; lane 0's copy counts
 
 // Take the next task of the global queue.  Lane 0 acts, no lock held; returns (event slot << 8 | 1) when the task's
 // interval went onto the calling warp's private stack, -1 otherwise (placed on the shared stack, empty, or none left).
@@ -429,6 +434,7 @@ __global__ void __launch_bounds__(K3F_THREADS, K3F_CTAS_PER_SM) k3_flow(K3Global
         S.n_free = K3F_WINS;
         S.top = 0; S.lock = 0; S.fetching = 0; S.drained = 0; S.failed = 0;
         S.cand = S.scans = S.exact = S.tasks = 0ull;
+        S.sure = S.multi = S.full = 0ull;
         for (int e = 0; e < K3F_EVS; ++e) { S.evs[e].ev = -1; S.evs[e].live = 0; }
     }
     for (int k = tid; k < K3F_WINS; k += K3F_THREADS) S.free_list[k] = K3F_WINS - 1 - k;
@@ -437,6 +443,7 @@ __global__ void __launch_bounds__(K3F_THREADS, K3F_CTAS_PER_SM) k3_flow(K3Global
 
     K3FTally T;
     T.cand = T.scans = T.exact = 0ull;
+    T.br.sure = T.br.multi = T.br.full = 0u;
     long long idle = 0;
     int ln = 0;     // entries on the private stack (all of event slot `les`)
     int les = -1;   // event slot this warp holds one `live` count of (while it has, or just had, private work)
@@ -603,7 +610,7 @@ __global__ void __launch_bounds__(K3F_THREADS, K3F_CTAS_PER_SM) k3_flow(K3Global
         int x;
         unsigned nexact = 0;
         if (!exact) {
-            x = f_decide(G, P, ccg, lo, hi, it.ps, pe, ebase, np, pc, K1, K2, I1, nexact);
+            x = f_decide(G, P, ccg, lo, hi, it.ps, pe, ebase, np, pc, K1, K2, I1, nexact, T.br);
         } else {
             K3Best b;
             b.g = __longlong_as_double((long long)K1);
@@ -613,7 +620,10 @@ __global__ void __launch_bounds__(K3F_THREADS, K3F_CTAS_PER_SM) k3_flow(K3Global
                 b = k3_warp_reduce(b);
             }
             x = __shfl_sync(PP_FULL, b.x, 0);
-            if (screen) nexact = (unsigned)ncand;
+            if (screen) {
+                nexact = (unsigned)ncand;
+                ++T.br.full;
+            }
         }
         T.cand += (unsigned long long)ncand;
         T.scans += 1;
@@ -668,6 +678,9 @@ __global__ void __launch_bounds__(K3F_THREADS, K3F_CTAS_PER_SM) k3_flow(K3Global
         atomicAdd(&S.cand, T.cand);
         atomicAdd(&S.scans, T.scans);
         atomicAdd(&S.exact, T.exact);
+        if (T.br.sure) atomicAdd(&S.sure, (unsigned long long)T.br.sure);
+        if (T.br.multi) atomicAdd(&S.multi, (unsigned long long)T.br.multi);
+        if (T.br.full) atomicAdd(&S.full, (unsigned long long)T.br.full);
     }
     __syncthreads();
     if (tid == 0) {
@@ -675,5 +688,8 @@ __global__ void __launch_bounds__(K3F_THREADS, K3F_CTAS_PER_SM) k3_flow(K3Global
         atomicAdd(&G.ctr->n_scan, S.scans);
         atomicAdd(&G.ctr->n_exact, S.exact);
         atomicAdd(&G.ctr->n_tasks, S.tasks);
+        if (S.sure) atomicAdd(&G.ctr->n_sure, S.sure);
+        if (S.multi) atomicAdd(&G.ctr->n_multi, S.multi);
+        if (S.full) atomicAdd(&G.ctr->n_full, S.full);
     }
 }
