@@ -292,6 +292,29 @@ int pp_pipeline_host_adc16(pp_ctx *ctx, const int16_t *host, int64_t n, double s
                            int64_t chunk_samples, const pp_pipeline_params *p,
                            const pp_host_tables *tables /* NULL: device tables only */, int64_t out[4]);
 
+/* ---- hidden Markov models over segment means (Event.apply_hmm / Event.parse(hmm=), DataTypes.py:292-355) ----
+ * S = n_states emitting states (1..128) with normal emissions, every log taken by the host: inv_std[j] = 1/sigma_j,
+ * log_norm[j] = -log(sigma_j) - log(2 pi)/2, log_start[j], log_trans[i*S + j] (row-normalised), log_end[j] (NULL:
+ * no end term).  Emission e_j(x) = log_norm[j] - 0.5 * z*z, z = (x - mean[j]) * inv_std[j], one rounding per
+ * operation and no FMA (bit-equal to NumPy).  algorithm 0: Viterbi -- log-probability of the best path and the path,
+ * bit-exact (ties go to the lowest state index); 1: forward log-likelihood (CUDA exp / log, not bit-exact).  A NaN
+ * value gives log-probability NaN, an impossible sequence -inf; the states of both are all -1. */
+typedef struct pp_hmm {
+    int n_states;
+    const double *mean, *inv_std, *log_norm, *log_start, *log_trans /* [i*S+j] */, *log_end /* NULL: none */;
+} pp_hmm;
+/* Decode the resident segment table, one sequence of segment means per event.  merge = 1 (Viterbi only): every run
+ * of consecutive segments of one event that share a state >= 0 becomes one segment whose statistics are computed
+ * again from the samples (K4, same sample source); *n_segments receives the new row count.  PP_ERR_STATE without
+ * resident segment statistics, PP_ERR_ARG for n_states outside 1..128 or merge with forward. */
+int pp_hmm_decode(pp_ctx *ctx, const pp_hmm *model, int algorithm, int merge, int64_t *n_segments);
+/* Decode n host sequences packed back to back in x (len[k] >= 1 values each). */
+int pp_hmm_decode_sequences(pp_ctx *ctx, const pp_hmm *model, int algorithm, const double *x, const int64_t *len,
+                            int64_t n);
+/* Results of the last decode: one log-probability per sequence, one state per value (per segment row of the
+ * merged table after a merge).  state may be NULL; it must be after a forward decode (PP_ERR_STATE otherwise). */
+int pp_hmm_download(pp_ctx *ctx, int64_t cap_seq, double *log_prob, int64_t cap_states, int32_t *state);
+
 /* ---- multi-GPU: one context per rank, contiguous trace chunks (SURVEY 8e) -------------
  * The exchange itself (NCCL all-gathers of the records / tables, point-to-point halos) is
  * driven by pypore_b200/dist.py; these calls keep every stage on the device between them.

@@ -10,7 +10,9 @@ signatures and side effects (DataTypes.py:258-289, 589-602).  The design is tabl
 * ``File.to_json`` / ``File.to_meta`` / the verbose lines of ``Experiment.parse`` work on the tables directly while
   no object has been handed out (``wire.file_tree``); after that they walk the objects, like the reference.
 
-HMM-guided parsing, plotting, MySQL and .abf reading are out of scope (SURVEY.md section 2).
+``File.parse(..., hmm=)`` and ``Event.parse(parser, hmm=)`` decode every event's segment means with a
+``pypore_b200.hmm.HMM`` (Viterbi, on the device) and merge consecutive segments that share a state.  Plotting, MySQL
+and .abf reading are out of scope (SURVEY.md section 2).
 """
 import json
 from functools import lru_cache
@@ -108,16 +110,53 @@ class Event(Segment):
         self.filtered, self.filter_order, self.filter_cutoff = True, order, cutoff
 
     def parse(self, parser=SpeedyStatSplit(prior_segments_per_second=10), hmm=None):
-        """Segment the event with a plug-in state parser (DataTypes.py:276-289,333); returns the segment count."""
-        if hmm is not None and hmm:
-            raise NotImplementedError("HMM-guided segmentation needs yahmm and is out of scope")
+        """Segment the event with a plug-in state parser (DataTypes.py:276-289,333); returns the segment count.
+
+        With ``hmm`` (a ``pypore_b200.hmm.HMM``; the parser must be a ``SpeedyStatSplit``) the segment means are
+        decoded with Viterbi and every run of consecutive segments in one state becomes one segment, whose
+        statistics are computed again from the samples; each segment carries its ``state`` (-1 for every segment of
+        an event whose sequence is impossible or holds a NaN)."""
         second = float(self.file.second)
-        pieces = parser.parse(self.current)
+        pieces = self._parse_hmm(parser, hmm) if hmm else parser.parse(self.current)
         for piece in pieces:
             piece.event = self
             piece.scale(second)
         self.segments, self.state_parser = pieces, parser
         return len(pieces)
+
+    def _parse_hmm(self, parser, hmm):
+        if not isinstance(parser, SpeedyStatSplit):
+            raise TypeError("HMM-guided segmentation runs on the device with a SpeedyStatSplit parser")
+        mw, MW, W, gain = parser._params()
+        cur = SpeedyStatSplit._as_event(self.current)
+        if cur.shape[0] == 0:
+            return parser.parse(cur)
+        ctx = _lib.default_context()
+        ctx.upload_events_f64([cur])
+        ctx.statsplit(mw, MW, W, gain)
+        ctx.segment_stats()
+        n = ctx.hmm_decode(hmm, "viterbi", merge=True)
+        tab = ctx.segments(n)
+        logp, states = ctx.hmm_download(1, n)
+        self.log_probability = float(logp[0])
+        pieces = []
+        for k in range(n):
+            a, b = int(tab["start"][k]), int(tab["end"][k])
+            seg = Segment(current=cur[a:b], start=a, duration=b - a, end=b)
+            seg._set_stats(tab["mean"][k], tab["std"][k], tab["min"][k], tab["max"][k])
+            seg.state = int(states[k])
+            pieces.append(seg)
+        return pieces
+
+    def apply_hmm(self, hmm, algorithm="viterbi"):
+        """Decode the segment means with ``hmm`` (DataTypes.py:349-355): "viterbi" gives (log-probability, states),
+        "forward" the log-likelihood."""
+        means = np.array([seg.mean for seg in self.segments], dtype=np.float64)
+        if algorithm == "viterbi":
+            return hmm.viterbi(means)
+        if algorithm == "forward":
+            return hmm.log_probability(means)
+        raise ValueError("algorithm must be 'viterbi' or 'forward', got %r" % (algorithm,))
 
     def delete(self):
         for name in ("current", "state_parser"):
@@ -216,15 +255,20 @@ class File(Segment):
     n = property(lambda self: len(self.events))
 
     def parse(self, parser=lambda_event_parser(threshold=90), segmenter=None, filter_params=None,
-              context=None):
+              context=None, hmm=None):
         """Detect events with a plug-in event parser (DataTypes.py:589-602).
 
         With ``segmenter=`` (a ``SpeedyStatSplit``) the whole pipeline runs on the
         resident trace -- threshold scan, optional ``Event.filter(*filter_params)``,
         split search, statistics -- and every event comes back with its
         ``segments`` already parsed, as after ``event.parse(parser=segmenter)``.
+        With ``hmm=`` (a ``pypore_b200.hmm.HMM``) one more device call decodes every event's segment means and
+        merges runs of segments in one state, as after ``event.parse(parser=segmenter, hmm=hmm)``:
+        ``segment_table`` gains a ``state`` column and ``event_table`` a ``log_probability`` column.
         """
         self.__dict__.pop("_tables", None)
+        if hmm is not None and segmenter is None:
+            raise ValueError("hmm= decodes segment means: it needs a segmenter")
         if segmenter is None and filter_params is None and not isinstance(parser, lambda_event_parser):
             # any duck-typed parser, exactly like the reference: seg.current / seg.start / seg.duration in samples
             rate, self.event_parser = self.second, parser
@@ -234,10 +278,10 @@ class File(Segment):
             return
         if not isinstance(parser, lambda_event_parser):
             raise TypeError("the device-resident pipeline needs a pypore_b200 lambda_event_parser")
-        self._parse_resident(context or _lib.default_context(), self._samples(), parser, segmenter, filter_params)
+        self._parse_resident(context or _lib.default_context(), self._samples(), parser, segmenter, filter_params, hmm)
 
     # ------------------------------------------------------------------
-    def _parse_resident(self, ctx, host, parser, segmenter, filter_params):
+    def _parse_resident(self, ctx, host, parser, segmenter, filter_params, hmm=None):
         filt = bessel_coefficients(filter_params[0], filter_params[1], self.second) if filter_params is not None else None
         rules = parser._device_rules()
         seg_table = None
@@ -251,7 +295,7 @@ class File(Segment):
             counts = _run_pipeline(ctx, host, parser.threshold, min_width=mw, max_width=MW, window_width=W,
                                    min_gain=gain, filter_ba=filt, with_stats=True, **rules.device_args())
             ev_start, ev_len = ctx.events(counts["events"])
-            seg_table = ctx.segments(counts["segments"])
+            seg_table = ctx.segments(counts["segments"]) if hmm is None else None
         else:
             _upload_trace(ctx, host)
             ev_start, ev_len = parser._detect(ctx, host)[:2]
@@ -260,14 +304,24 @@ class File(Segment):
             if segmenter is not None and len(ev_start):
                 n_seg = ctx.statsplit(mw, MW, W, gain)
                 ctx.segment_stats()
-                seg_table = ctx.segments(n_seg)
+                seg_table = ctx.segments(n_seg) if hmm is None else None
         n_ev = len(ev_start)
+        log_prob = None
+        if hmm is not None:
+            log_prob, state = np.zeros(0), np.zeros(0, np.int32)
+            if n_ev:
+                n_seg = ctx.hmm_decode(hmm, "viterbi", merge=True)
+                seg_table = ctx.segments(n_seg)
+                log_prob, state = ctx.hmm_download(n_ev, n_seg)
         ev_stats = ctx.event_stats(n_ev) if n_ev else {k: np.zeros(0) for k in ("mean", "std", "min", "max")}
         filtered = ctx.event_samples(int(ev_len.sum())) if filt is not None and n_ev else None
         if segmenter is not None and seg_table is None:
             seg_table = {"event": np.zeros(0, np.int32), "start": np.zeros(0, np.int64), "end": np.zeros(0, np.int64),
                          **{k: np.zeros(0) for k in ("mean", "std", "min", "max")}}
         self.event_table = dict(start=ev_start, length=ev_len, **ev_stats)
+        if hmm is not None:
+            seg_table["state"] = state
+            self.event_table["log_probability"] = log_prob
         self.segment_table = seg_table
         self.event_parser = parser
         self._attach(wire.FileTables(self.second, self.event_table, seg_table, filter_params, segmenter),
@@ -302,8 +356,11 @@ class File(Segment):
                 def meta_segment(j):
                     k = lo + j
                     a = int(sg["start"][k])
-                    return MetaSegment(**dict(zip(("mean", "std", "min", "max"), stats(sg, k))),
-                                       **span(a, int(sg["end"][k]) - a))
+                    seg = MetaSegment(**dict(zip(("mean", "std", "min", "max"), stats(sg, k))),
+                                      **span(a, int(sg["end"][k]) - a))
+                    if "state" in sg:
+                        seg.state = int(sg["state"][k])
+                    return seg
                 kw["segments"] = _LazyList(int(bounds[i + 1]) - lo, meta_segment)
                 kw["state_parser"] = tables.state_parser
             return MetaEvent(**kw)
@@ -313,6 +370,8 @@ class File(Segment):
             samples = filtered[ev_off[i]:ev_off[i + 1]] if filtered is not None else np.array(host[a:a + n])
             event = Event(current=samples, second=second, file=self, **span(a, n))
             event._set_stats(*stats(ev, i))
+            if "log_probability" in ev:
+                event.log_probability = float(ev["log_probability"][i])
             if fp is not None:
                 event.filtered, (event.filter_order, event.filter_cutoff) = True, fp
             if sg is not None:
@@ -323,6 +382,8 @@ class File(Segment):
                     s, e = int(sg["start"][k]), int(sg["end"][k])
                     seg = Segment(current=samples[s:e], start=s, duration=e - s, end=e)._set_stats(*stats(sg, k))
                     seg.event = event
+                    if "state" in sg:
+                        seg.state = int(sg["state"][k])
                     seg.scale(float(second))
                     return seg
                 event.segments = _LazyList(int(bounds[i + 1]) - lo, segment)

@@ -60,6 +60,14 @@ class UnpackedTables(_c.Structure):
                 ("mean", _c.c_void_p), ("std", _c.c_void_p), ("min", _c.c_void_p), ("max", _c.c_void_p)]
 
 
+class Hmm(_c.Structure):
+    """pp_hmm: a model in log space (pypore_b200.hmm.HMM builds it)."""
+    _fields_ = [("n_states", _c.c_int), ("mean", _f64p), ("inv_std", _f64p), ("log_norm", _f64p),
+                ("log_start", _f64p), ("log_trans", _f64p), ("log_end", _f64p)]
+
+
+HMM_ALGORITHMS = {"viterbi": 0, "forward": 1}
+
 # name -> (restype, argtypes); every symbol include/pypore_b200.h declares
 SIGNATURES = {
     "pp_version": (_c.c_int, []),
@@ -132,6 +140,9 @@ SIGNATURES = {
     "pp_pipeline_host_adc16": (_c.c_int, [_c.c_void_p, _c.c_void_p, _i64, _c.c_double, _c.c_double, _i64,
                                           _c.POINTER(PipelineParams), _c.POINTER(HostTables), _i64p]),
     "pp_pipeline": (_c.c_int, [_c.c_void_p, _c.POINTER(PipelineParams), _i64p]),
+    "pp_hmm_decode": (_c.c_int, [_c.c_void_p, _c.POINTER(Hmm), _c.c_int, _c.c_int, _i64p]),
+    "pp_hmm_decode_sequences": (_c.c_int, [_c.c_void_p, _c.POINTER(Hmm), _c.c_int, _f64p, _i64p, _i64]),
+    "pp_hmm_download": (_c.c_int, [_c.c_void_p, _i64, _f64p, _i64, _i32p]),
 }
 
 _lib = None
@@ -607,6 +618,40 @@ class Context(object):
         p.prefix_mode = int(prefix_mode)
         p.with_stats = int(bool(with_stats))
         return p, keep
+
+    # -- HMM decoding (csrc/hmm.cuh) -----------------------------------------------
+    @staticmethod
+    def _hmm(model):
+        """pp_hmm over the log-space arrays of `model` (a pypore_b200.hmm.HMM); the arrays outlive the call."""
+        m = Hmm()
+        m.n_states = int(model.n_states)
+        for name in ("mean", "inv_std", "log_norm", "log_start", "log_trans"):
+            setattr(m, name, _ptr(getattr(model, name), _f64p))
+        m.log_end = _ptr(model.log_end, _f64p)
+        return m
+
+    def hmm_decode(self, model, algorithm="viterbi", merge=False):
+        """Decode the resident segment table, one sequence of segment means per event (pp_hmm_decode); with
+        merge=True (Viterbi) runs of segments sharing a state become one segment.  Returns the segment count."""
+        n = _i64()
+        self._ck(self._L.pp_hmm_decode(self._h, _c.byref(self._hmm(model)), HMM_ALGORITHMS[algorithm],
+                                       int(bool(merge)), _c.byref(n)))
+        return int(n.value)
+
+    def hmm_decode_sequences(self, model, algorithm, seqs):
+        """Decode host sequences (float64 arrays, none empty) in one device call."""
+        lens = np.asarray([len(q) for q in seqs], np.int64)
+        x = np.ascontiguousarray(np.concatenate(seqs) if len(seqs) else np.zeros(0), np.float64)
+        self._ck(self._L.pp_hmm_decode_sequences(self._h, _c.byref(self._hmm(model)), HMM_ALGORITHMS[algorithm],
+                                                 _ptr(x, _f64p), _ptr(lens, _i64p), lens.shape[0]))
+        return lens
+
+    def hmm_download(self, n_seq, n_states=None):
+        """(log-probabilities [n_seq], states [n_states] int32 or None) of the last decode."""
+        logp = np.empty(n_seq, np.float64)
+        state = np.empty(n_states, np.int32) if n_states is not None else None
+        self._ck(self._L.pp_hmm_download(self._h, n_seq, _ptr(logp, _f64p), n_states or 0, _ptr(state, _i32p)))
+        return logp, state
 
     # -- multi-GPU (driven by pypore_b200.dist) ----------------------------------
     def shard_scan(self, threshold, scan_len, dev_record_ptr):

@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libpypore_b200.so")
 SOURCES = ["api.cu"]
-HEADERS = ["common.cuh", "threshold.cuh", "prefix.cuh", "split.cuh", "split_flow.cuh", "stats.cuh", "filter.cuh",
+HEADERS = ["common.cuh", "threshold.cuh", "prefix.cuh", "split.cuh", "split_flow.cuh", "stats.cuh", "filter.cuh", "hmm.cuh",
            os.path.join("..", "..", "include", "pypore_b200.h")]
 
 NVCC_FLAGS = [

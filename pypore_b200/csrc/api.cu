@@ -9,6 +9,7 @@
 #include "split_flow.cuh"
 #include "stats.cuh"
 #include "filter.cuh"
+#include "hmm.cuh"
 
 #include <new>
 #include <stdarg.h>
@@ -109,6 +110,11 @@ struct pp_ctx {
 
     // filter scratch
     DevBuf filt_tmp, filt_carry, filt_coef;
+
+    // HMM decoding (pp_hmm_*): model block, host sequences and their offsets, results of the last decode
+    DevBuf hmm_model, hmm_x, hmm_off, hmm_logp, hmm_state, hmm_bp, hmm_next, hmm_old_flat, hmm_old_state;
+    int64_t hmm_n_seq = -1, hmm_n_rows = -1;
+    bool hmm_states = false;   // the last decode was a Viterbi decode
 
     // streamed pipeline (pp_pipeline_host): copies run on their own stream
     cudaStream_t copy_stream = nullptr;
@@ -779,7 +785,9 @@ void pp_destroy(pp_ctx *ctx)
                       &ctx->tasks, &ctx->ready, &ctx->block_count, &ctx->block_off, &ctx->inexact, &ctx->Ttab, &ctx->ev_tile_off, &ctx->k2_bits, &ctx->k2_tiles,
                       &ctx->seg_flat, &ctx->seg_event, &ctx->seg_start, &ctx->seg_end, &ctx->seg_mean,
                       &ctx->seg_std, &ctx->seg_min, &ctx->seg_max, &ctx->evs_mean, &ctx->evs_std,
-                      &ctx->evs_min, &ctx->evs_max, &ctx->filt_tmp, &ctx->filt_carry, &ctx->filt_coef, &ctx->hk, &ctx->unpack_flag, &ctx->ctl_buf, &ctx->ctl_peers_dev};
+                      &ctx->evs_min, &ctx->evs_max, &ctx->filt_tmp, &ctx->filt_carry, &ctx->filt_coef, &ctx->hk, &ctx->unpack_flag, &ctx->ctl_buf, &ctx->ctl_peers_dev,
+                      &ctx->hmm_model, &ctx->hmm_x, &ctx->hmm_off, &ctx->hmm_logp, &ctx->hmm_state, &ctx->hmm_bp,
+                      &ctx->hmm_next, &ctx->hmm_old_flat, &ctx->hmm_old_state};
     for (DevBuf *b : bufs) release(*b);
     if (ctx->ctr) cudaFree(ctx->ctr);
     if (ctx->h_ctr) cudaFreeHost(ctx->h_ctr);
@@ -1890,6 +1898,206 @@ int pp_pipeline_host_adc16(pp_ctx *ctx, const int16_t *host, int64_t n, double s
     if (pp_adc16_check(scale, offset) != PP_OK)
         return fail(ctx, PP_ERR_ARG, "ADC scale must be finite and non-zero, offset finite, every count decoding finite");
     return pipeline_host_impl(ctx, host, PP_SRC_ADC16, PPAdc{scale, offset}, n, chunk_samples, p, tables, out);
+}
+
+// ---- HMM decoding (csrc/hmm.cuh) -----------------------------------------------
+// The model as the block of doubles the kernels stage in shared memory; PP_ERR_ARG for S outside 1..128
+static int hmm_upload_model(pp_ctx *ctx, const pp_hmm *m)
+{
+    if (!m) return fail(ctx, PP_ERR_ARG, "no model");
+    const int S = m->n_states;
+    if (S < 1 || S > HMM_MAX_STATES) return fail(ctx, PP_ERR_ARG, "n_states must be 1..%d, got %d", HMM_MAX_STATES, S);
+    if (!m->mean || !m->inv_std || !m->log_norm || !m->log_start || !m->log_trans)
+        return fail(ctx, PP_ERR_ARG, "incomplete model");
+    const size_t W = hmm_model_words(S);
+    double *blk = (double *)malloc(sizeof(double) * W);
+    if (!blk) return fail(ctx, PP_ERR_ARG, "out of host memory");
+    for (int j = 0; j < S; ++j) {
+        blk[j] = m->mean[j];
+        blk[S + j] = m->inv_std[j];
+        blk[2 * S + j] = m->log_norm[j];
+        blk[3 * S + j] = m->log_start[j];
+        blk[4 * S + j] = m->log_end ? m->log_end[j] : 0.0;
+    }
+    memcpy(blk + 5 * S, m->log_trans, sizeof(double) * (size_t)S * S);
+    int rc = ensure(ctx, ctx->hmm_model, sizeof(double) * W);
+    if (rc == PP_OK) {
+        cudaError_t e = cudaMemcpyAsync(ctx->hmm_model.p, blk, sizeof(double) * W, cudaMemcpyHostToDevice, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);   // pageable block: consumed before it is freed
+        if (e != cudaSuccess) rc = fail(ctx, PP_ERR_CUDA, "model upload failed: %s", cudaGetErrorString(e));
+    }
+    free(blk);
+    return rc;
+}
+
+static int hmm_grid(pp_ctx *ctx, const void *kernel, int threads, size_t smem, int64_t want, int *grid)
+{
+    CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 0;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
+    int64_t g = (int64_t)ctx->sm_count * (per_sm > 0 ? per_sm : 1);
+    *grid = (int)(g < want ? g : want);
+    return PP_OK;
+}
+
+// Decode the sequences x[off[k] .. off[k+1]) (device memory, n_seq of them over n_rows samples) with the staged model
+static int hmm_enqueue_decode(pp_ctx *ctx, int S, int algorithm, const double *x, const int64_t *off, int64_t n_seq,
+                              int64_t n_rows)
+{
+    const bool vit = algorithm == 0;
+    CKR(ensure(ctx, ctx->hmm_logp, sizeof(double) * (size_t)(n_seq > 0 ? n_seq : 1)));
+    CKR(ensure(ctx, ctx->hmm_next, sizeof(unsigned long long)));
+    if (vit) {
+        CKR(ensure(ctx, ctx->hmm_state, sizeof(int) * (size_t)(n_rows > 0 ? n_rows : 1)));
+        CKR(ensure(ctx, ctx->hmm_bp, (size_t)(n_rows > 0 ? n_rows : 1) * S));
+    }
+    ctx->hmm_n_seq = n_seq;
+    ctx->hmm_n_rows = n_rows;
+    ctx->hmm_states = vit;
+    if (n_seq == 0) return PP_OK;
+    HMMSeqs Q;
+    Q.x = x;
+    Q.off = off;
+    Q.n = n_seq;
+    Q.logp = (double *)ctx->hmm_logp.p;
+    Q.state = vit ? (int *)ctx->hmm_state.p : nullptr;
+    Q.bp = vit ? (unsigned char *)ctx->hmm_bp.p : nullptr;
+    Q.next = (unsigned long long *)ctx->hmm_next.p;
+    CK(cudaMemsetAsync(Q.next, 0, sizeof(unsigned long long), ctx->stream));
+    const size_t model_bytes = sizeof(double) * hmm_model_words(S);
+    const double *model = (const double *)ctx->hmm_model.p;
+    int grid = 0;
+    if (S <= 32) {
+        const int64_t want = (n_seq + HMM_WARP_THREADS / 32 - 1) / (HMM_WARP_THREADS / 32);
+        if (vit) {
+            CKR(hmm_grid(ctx, (const void *)k_hmm_warp<true>, HMM_WARP_THREADS, model_bytes, want, &grid));
+            k_hmm_warp<true><<<grid, HMM_WARP_THREADS, model_bytes, ctx->stream>>>(model, S, Q);
+        } else {
+            CKR(hmm_grid(ctx, (const void *)k_hmm_warp<false>, HMM_WARP_THREADS, model_bytes, want, &grid));
+            k_hmm_warp<false><<<grid, HMM_WARP_THREADS, model_bytes, ctx->stream>>>(model, S, Q);
+        }
+    } else {
+        const size_t smem = model_bytes + sizeof(double) * 2 * HMM_MAX_STATES;
+        if (vit) {
+            CKR(hmm_grid(ctx, (const void *)k_hmm_cta<true>, HMM_CTA_THREADS, smem, n_seq, &grid));
+            k_hmm_cta<true><<<grid, HMM_CTA_THREADS, smem, ctx->stream>>>(model, S, Q);
+        } else {
+            CKR(hmm_grid(ctx, (const void *)k_hmm_cta<false>, HMM_CTA_THREADS, smem, n_seq, &grid));
+            k_hmm_cta<false><<<grid, HMM_CTA_THREADS, smem, ctx->stream>>>(model, S, Q);
+        }
+    }
+    LAUNCHED(ctx);
+    if (vit) {
+        const int64_t tb = (n_seq + 127) / 128;
+        k_hmm_traceback<<<(unsigned)(tb < ctx->sm_count * 8 ? tb : ctx->sm_count * 8), 128, 0, ctx->stream>>>(Q, S);
+        LAUNCHED(ctx);
+    }
+    return PP_OK;
+}
+
+// Merge runs of segments that share a Viterbi state: new breakpoints, the existing compaction and K4 statistics
+static int hmm_enqueue_merge(pp_ctx *ctx)
+{
+    const int64_t n_old = ctx->n_segments;
+    const unsigned grid = (unsigned)ctx->sm_count * 4;
+    CKR(ensure(ctx, ctx->hmm_old_flat, sizeof(int64_t) * (size_t)(n_old > 0 ? n_old : 1)));
+    CKR(ensure(ctx, ctx->hmm_old_state, sizeof(int) * (size_t)(n_old > 0 ? n_old : 1)));
+    if (n_old > 0) {
+        CK(cudaMemcpyAsync(ctx->hmm_old_flat.p, ctx->seg_flat.p, sizeof(int64_t) * n_old, cudaMemcpyDeviceToDevice,
+                           ctx->stream));
+        CK(cudaMemcpyAsync(ctx->hmm_old_state.p, ctx->hmm_state.p, sizeof(int) * n_old, cudaMemcpyDeviceToDevice,
+                           ctx->stream));
+    }
+    CK(cudaMemsetAsync(ctx->bits.p, 0, sizeof(unsigned) * ctx->n_words, ctx->stream));
+    k_hmm_merge_bits<<<grid, 256, 0, ctx->stream>>>((const int *)ctx->seg_event.p, (const int64_t *)ctx->seg_flat.p,
+                                                    (const int *)ctx->hmm_state.p, n_old, (unsigned *)ctx->bits.p);
+    LAUNCHED(ctx);
+    // the whole table is rebuilt: no range was finalised (the streamed export leaves these at the totals)
+    CK(cudaMemsetAsync(&ctx->ctr->seg_done, 0, 3 * sizeof(unsigned long long), ctx->stream));
+    CKR(enqueue_compact(ctx));
+    k_hmm_merged_states<<<grid, 256, 0, ctx->stream>>>(ctx->ctr, (const int64_t *)ctx->seg_flat.p,
+                                                       (const int64_t *)ctx->hmm_old_flat.p,
+                                                       (const int *)ctx->hmm_old_state.p, n_old, (int *)ctx->hmm_state.p);
+    LAUNCHED(ctx);
+    CKR(launch_stats(ctx, 0, (const int64_t *)ctx->seg_flat.p, (const int *)ctx->seg_event.p, ctx->cap_segs,
+                     (double *)ctx->seg_mean.p, (double *)ctx->seg_std.p, (double *)ctx->seg_min.p,
+                     (double *)ctx->seg_max.p));
+    CKR(fetch_counters(ctx));
+    CKR(check_overflow(ctx));
+    ctx->n_segments = (int64_t)ctx->h_ctr->n_segments;
+    ctx->hmm_n_rows = ctx->n_segments;
+    return PP_OK;
+}
+
+int pp_hmm_decode(pp_ctx *ctx, const pp_hmm *model, int algorithm, int merge, int64_t *n_segments)
+{
+    if (!ctx) return PP_ERR_ARG;
+    if (algorithm != 0 && algorithm != 1) return fail(ctx, PP_ERR_ARG, "algorithm must be 0 (Viterbi) or 1 (forward)");
+    if (merge && algorithm != 0) return fail(ctx, PP_ERR_ARG, "merging needs Viterbi states");
+    if (!model || model->n_states < 1 || model->n_states > HMM_MAX_STATES)
+        return fail(ctx, PP_ERR_ARG, "n_states must be 1..%d", HMM_MAX_STATES);
+    if (ctx->n_segments < 0 || !ctx->stats_valid || ctx->n_events < 0)
+        return fail(ctx, PP_ERR_STATE, "no resident segment statistics (pp_statsplit + pp_segment_stats / pp_pipeline)");
+    CKR(set_device(ctx));
+    CKR(hmm_upload_model(ctx, model));
+    const int64_t E = ctx->n_events, R = ctx->n_segments;
+    CKR(ensure(ctx, ctx->hmm_off, sizeof(int64_t) * (size_t)(E + 1)));
+    k_hmm_event_offsets<<<(unsigned)(E / 256 + 1 < ctx->sm_count * 4 ? E / 256 + 1 : ctx->sm_count * 4), 256, 0,
+                          ctx->stream>>>((const int *)ctx->seg_event.p, R, E, (int64_t *)ctx->hmm_off.p);
+    LAUNCHED(ctx);
+    CKR(hmm_enqueue_decode(ctx, model->n_states, algorithm, (const double *)ctx->seg_mean.p,
+                           (const int64_t *)ctx->hmm_off.p, E, R));
+    if (merge) CKR(hmm_enqueue_merge(ctx));
+    if (n_segments) *n_segments = ctx->n_segments;
+    return PP_OK;
+}
+
+int pp_hmm_decode_sequences(pp_ctx *ctx, const pp_hmm *model, int algorithm, const double *x, const int64_t *len,
+                            int64_t n)
+{
+    if (!ctx) return PP_ERR_ARG;
+    if (algorithm != 0 && algorithm != 1) return fail(ctx, PP_ERR_ARG, "algorithm must be 0 (Viterbi) or 1 (forward)");
+    if (n < 0 || (n > 0 && (!x || !len))) return fail(ctx, PP_ERR_ARG, "bad sequences");
+    int64_t *off = (int64_t *)malloc(sizeof(int64_t) * (size_t)(n + 1));
+    if (!off) return fail(ctx, PP_ERR_ARG, "out of host memory");
+    off[0] = 0;
+    for (int64_t k = 0; k < n; ++k) {
+        if (len[k] <= 0) { free(off); return fail(ctx, PP_ERR_ARG, "sequence %lld is empty", (long long)k); }
+        off[k + 1] = off[k] + len[k];
+    }
+    const int64_t total = off[n];
+    auto run = [&]() -> int {
+        CKR(set_device(ctx));
+        CKR(hmm_upload_model(ctx, model));
+        CKR(ensure(ctx, ctx->hmm_off, sizeof(int64_t) * (size_t)(n + 1)));
+        CKR(ensure(ctx, ctx->hmm_x, sizeof(double) * (size_t)(total > 0 ? total : 1)));
+        CK(cudaMemcpyAsync(ctx->hmm_off.p, off, sizeof(int64_t) * (size_t)(n + 1), cudaMemcpyHostToDevice, ctx->stream));
+        if (total) CK(cudaMemcpyAsync(ctx->hmm_x.p, x, sizeof(double) * (size_t)total, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));   // pageable host memory: consumed before the call returns
+        return hmm_enqueue_decode(ctx, model->n_states, algorithm, (const double *)ctx->hmm_x.p,
+                                  (const int64_t *)ctx->hmm_off.p, n, total);
+    };
+    const int rc = run();
+    free(off);
+    return rc;
+}
+
+int pp_hmm_download(pp_ctx *ctx, int64_t cap_seq, double *log_prob, int64_t cap_states, int32_t *state)
+{
+    if (!ctx) return PP_ERR_ARG;
+    if (ctx->hmm_n_seq < 0) return fail(ctx, PP_ERR_STATE, "no HMM decode has run");
+    if (state && !ctx->hmm_states) return fail(ctx, PP_ERR_STATE, "the last decode computed no states (forward)");
+    if ((log_prob && cap_seq < ctx->hmm_n_seq) || (state && cap_states < ctx->hmm_n_rows))
+        return fail(ctx, PP_ERR_CAPACITY, "HMM result buffers too small");
+    CKR(set_device(ctx));
+    if (log_prob && ctx->hmm_n_seq)
+        CK(cudaMemcpyAsync(log_prob, ctx->hmm_logp.p, sizeof(double) * (size_t)ctx->hmm_n_seq, cudaMemcpyDeviceToHost,
+                           ctx->stream));
+    if (state && ctx->hmm_n_rows)
+        CK(cudaMemcpyAsync(state, ctx->hmm_state.p, sizeof(int) * (size_t)ctx->hmm_n_rows, cudaMemcpyDeviceToHost,
+                           ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return PP_OK;
 }
 
 }  // extern "C"
