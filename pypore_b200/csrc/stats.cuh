@@ -19,7 +19,7 @@
 //     elements in front of and behind the row are masked: a row of ~130 float32 samples is 5 trips of an
 //     8-lane group instead of 17 (the first cut issued 32 thread instructions per sample, most of them
 //     per-row set-up and scalar loads: 31 % of the HBM peak);
-//   * longer rows (every row of a warp that holds one) and the rows above: two passes (mean = sum(x)/n, then
+//   * longer rows and the rows above: two passes (mean = sum(x)/n, then
 //     the deviations from it), like np.std, from scalar loads; a finite constant row gets its value and 0.
 // min / max run on the samples' own type (int16 ADC counts: on the counts, decoded at the end); a NaN anywhere
 // makes both NaN like np.min / np.max.
@@ -143,15 +143,20 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
         T mn = k4_top<T>(), mx = k4_bottom<T>();
         int nan = 0;
         double mean, var;
-        const bool one_pass = __all_sync(PP_FULL, len <= K4_ONE_PASS);
-        bool redo = !one_pass;  // this group's row takes the two passes
-        if (one_pass) {
+        // Which passes a row takes depends on the row alone, never on the rows that share its warp: the streamed
+        // pipeline's per-chunk launches start at another row (seg_done) than one launch over the whole table, and
+        // both must give the same bits.  A long row's group runs the one-pass loop over nothing, the two-pass
+        // block below over its row (shuffles stay warp-wide in both).
+        const bool long_row = len > K4_ONE_PASS;
+        const int64_t n1 = long_row ? 0 : len;
+        bool redo = long_row;  // this group's row takes the two passes
+        if (__any_sync(PP_FULL, !long_row)) {
             // 16-byte vectors from the aligned start: `mis` elements of the first vector lie in front of the row
             const int mis = (int)((reinterpret_cast<uintptr_t>(p) & 15) / sizeof(T));
             const typename VT::V *pv = reinterpret_cast<const typename VT::V *>(p - mis);
-            const int64_t last = mis + len;                  // elements [mis, last) of the vector stream are the row
+            const int64_t last = mis + n1;                   // elements [mis, last) of the vector stream are the row
             const int64_t nvec = (last + N - 1) / N;
-            double K = len > 0 ? pp_val(__ldg(p), adc) : 0.0;  // the shift: the row's first sample
+            double K = n1 > 0 ? pp_val(__ldg(p), adc) : 0.0;  // the shift: the row's first sample
             if (!(fabs(K) <= 1.7e308)) K = 0.0;              // inf / NaN: plain sums
             for (int64_t v0 = gl; v0 < nvec; v0 += K4_U * G) {
                 typename VT::V q[K4_U];
@@ -191,12 +196,13 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
             }
             s1 = k4_group_sum<G>(s1);
             s2 = k4_group_sum<G>(s2);
-            const double rl = 1.0 / (double)(len > 0 ? len : 1);
+            const double rl = 1.0 / (double)(n1 > 0 ? n1 : 1);
             const double m1 = s1 * rl;
             mean = K + m1;
             var = s2 * rl - m1 * m1;
-            if (len == 0) { mean = __longlong_as_double(0x7ff8000000000000LL); var = mean; }
-            redo = m1 * m1 > 1024.0 * var;  // heavy cancellation: the shift sits far from the mean (false for NaN)
+            if (n1 == 0) { mean = __longlong_as_double(0x7ff8000000000000LL); var = mean; }
+            // heavy cancellation: the shift sits far from the mean (false for NaN)
+            redo = long_row || m1 * m1 > 1024.0 * var;
         }
         if (__any_sync(PP_FULL, redo)) {
             // rows of the other groups run with length 0: the group sums below are warp-wide
@@ -205,7 +211,7 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
             for (int64_t j = gl; j < n2; j += G) {
                 const T x = p[j];
                 t1 += pp_val(x, adc);
-                if (!one_pass) {
+                if (long_row) {
                     mn = k4_min(mn, x);
                     mx = k4_max(mx, x);
                     nan |= (x != x);
@@ -223,7 +229,7 @@ __device__ __forceinline__ void k4_rows(const T *__restrict__ samples, const int
         mx = k4_group_max<G>(mx);
 #pragma unroll
         for (int d = G / 2; d > 0; d >>= 1) nan |= __shfl_xor_sync(PP_FULL, nan, d);
-        if (!one_pass && !nan && mn == mx) {  // a finite constant row: its value and exactly 0, as in one pass
+        if (long_row && !nan && mn == mx) {  // a finite constant row: its value and exactly 0, as in one pass
             const double v = pp_val(mn, adc);
             if (fabs(v) <= 1.7e308) { mean = v; var = 0.0; }
         }
