@@ -281,21 +281,6 @@ class Context(object):
         self._keep = []
         return len(trace)
 
-    def upload_trace_any(self, x):
-        """float32 arrays go up as they are, float64 ones as float32 when that loses nothing (half the bytes,
-        same results: double(x32) == x), as float64 otherwise; integer arrays are exact in float64."""
-        x = np.asarray(x)
-        if x.dtype == np.float32:
-            return self.upload_trace(x)
-        if x.dtype.kind in "iub":
-            x = x.astype(np.float64)
-        if x.dtype != np.float64:
-            raise TypeError("trace must be float32, float64 or an integer type, got %s" % x.dtype)
-        x32 = x.astype(np.float32)
-        if np.array_equal(x32.astype(np.float64), x, equal_nan=True):
-            return self.upload_trace(x32)
-        return self.upload_trace_f64(x)
-
     def upload_trace_async(self, x32, extra_capacity=0):
         """For pinned host arrays; caller keeps `x32` alive until sync()."""
         assert x32.dtype == np.float32 and x32.flags.c_contiguous

@@ -14,14 +14,32 @@
 #include <new>
 #include <stdarg.h>
 #include <stdlib.h>
+#include <utility>
+#include <vector>
 
 #include <nvtx3/nvToolsExt.h>   // header-only (no link dependency); ranges cost nothing without a profiler attached
 
 namespace {
 
+// Device memory that belongs to one owner (a pp_ctx member or a scratch local) and is freed with it
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
+
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    DevBuf(DevBuf &&o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+    DevBuf &operator=(DevBuf &&o) noexcept
+    {
+        if (this != &o) {
+            if (p) cudaFree(p);
+            p = std::exchange(o.p, nullptr);
+            cap = std::exchange(o.cap, 0);
+        }
+        return *this;
+    }
+    ~DevBuf() { if (p) cudaFree(p); }
 };
 
 enum { ST_THRESHOLD = 0, ST_SELECT, ST_FILTER, ST_PREFIX, ST_SPLIT, ST_COMPACT, ST_STATS, ST_COUNT };
@@ -43,8 +61,11 @@ struct pp_ctx {
     char err[512] = {0};
     int64_t launches = 0;
 
-    // trace: float32 (trace), float64 (trace64) or int16 ADC (trace16, decoded with adc) samples, one of the three
+    // trace: the resident samples (in trace_buf, or adopted), float32, float64 or int16 ADC counts (decoded with adc)
+    // as trace_kind (PP_SRC_*) says
     DevBuf trace_buf;
+    const void *trace = nullptr;
+    int trace_kind = PP_SRC_TRACE32;
     // pp_trace_prefetch: up to two float32 traces on their way up while the resident one is processed (oldest first);
     // trace_spare is the buffer the last swap retired
     struct Pending {
@@ -54,12 +75,8 @@ struct pp_ctx {
     } pend[2];
     int n_pend = 0;
     DevBuf trace_spare;
-    const float *trace = nullptr;
-    const double *trace64 = nullptr;
-    const int16_t *trace16 = nullptr;
     PPAdc adc = {1.0, 0.0};
     int64_t n = 0, trace_cap = 0;
-    bool adopted = false;
 
     // counters
     PPCounters *ctr = nullptr;
@@ -176,11 +193,16 @@ int ensure(pp_ctx *ctx, DevBuf &b, size_t bytes)
     return PP_OK;
 }
 
-void release(DevBuf &b)
+// Host scratch freed with its scope; a failed allocation is reported, not thrown across the C ABI
+template <typename T>
+int host_scratch(pp_ctx *ctx, std::vector<T> &v, size_t n)
 {
-    if (b.p) cudaFree(b.p);
-    b.p = nullptr;
-    b.cap = 0;
+    try {
+        v.resize(n);
+    } catch (const std::exception &) {
+        return fail(ctx, PP_ERR_ARG, "out of host memory");
+    }
+    return PP_OK;
 }
 
 int set_device(pp_ctx *ctx)
@@ -202,12 +224,77 @@ void reset_stages(pp_ctx *ctx)
     for (int i = 0; i <= ST_COUNT; ++i) ctx->rec[i] = false;
 }
 
+// A call whose stages pp_stage_ms times: earlier boundaries are forgotten, the first one is recorded now
+int begin_call(pp_ctx *ctx, int first_boundary)
+{
+    CKR(set_device(ctx));
+    reset_stages(ctx);
+    return record_boundary(ctx, first_boundary);
+}
+
+// stage `st` is enqueued: the boundary that ends it
+int end_stage(pp_ctx *ctx, int st)
+{
+    CKR(record_boundary(ctx, st + 1));
+    ctx->stage_ran[st] = true;
+    return PP_OK;
+}
+
+// State derived from the trace, each level from the one before it: dropping a level drops the levels after it too
+enum { LV_RUNS, LV_EVENTS, LV_PREFIX, LV_SEGMENTS, LV_STATS };
+
+void drop_from(pp_ctx *ctx, int level)
+{
+    if (level <= LV_RUNS) ctx->n_runs = -1;
+    if (level <= LV_EVENTS) ctx->n_events = ctx->n_event_samples = -1;
+    if (level <= LV_PREFIX) ctx->prefix_valid = false;
+    if (level <= LV_SEGMENTS) ctx->n_segments = -1;
+    ctx->stats_valid = false;
+}
+
+size_t sample_bytes(int kind)
+{
+    return kind == PP_SRC_TRACE64 ? sizeof(double) : kind == PP_SRC_ADC16 ? sizeof(int16_t) : sizeof(float);
+}
+
+// `n` samples of `kind` at `p` (room for `cap`) become the resident trace
+void set_trace(pp_ctx *ctx, const void *p, int kind, int64_t n, int64_t cap)
+{
+    ctx->trace = p;
+    ctx->trace_kind = kind;
+    ctx->n = n;
+    ctx->trace_cap = cap;
+    drop_from(ctx, LV_RUNS);
+}
+
+// the resident samples as T if they are of `kind`, else null
+template <typename T>
+const T *trace_as(const pp_ctx *ctx, int kind)
+{
+    return ctx->trace_kind == kind ? (const T *)ctx->trace : nullptr;
+}
+
+// Which resident traces a call takes: bits 1 << PP_SRC_* of the trace kinds, TAKES_NONE for no trace at all
+enum : unsigned {
+    TAKES_F32 = 1u << PP_SRC_TRACE32,
+    TAKES_NONE = 1u << 8,
+    NOT_ADC = TAKES_F32 | 1u << PP_SRC_TRACE64 | TAKES_NONE,
+};
+
+int require_trace(pp_ctx *ctx, unsigned takes, const char *what)
+{
+    if (takes & (ctx->trace ? 1u << ctx->trace_kind : TAKES_NONE)) return PP_OK;
+    const char *have = !ctx->trace ? "no trace" : ctx->trace_kind == PP_SRC_ADC16 ? "an ADC trace"
+                       : ctx->trace_kind == PP_SRC_TRACE64 ? "a float64 trace" : "a float32 trace";
+    return fail(ctx, PP_ERR_STATE, "%s; %s is resident", what, have);
+}
+
 PPSource make_source(pp_ctx *ctx)
 {
     PPSource s;
-    s.trace = ctx->trace;
-    s.trace64 = ctx->trace64;
-    s.trace16 = ctx->trace16;
+    s.trace = trace_as<float>(ctx, PP_SRC_TRACE32);
+    s.trace64 = trace_as<double>(ctx, PP_SRC_TRACE64);
+    s.trace16 = trace_as<int16_t>(ctx, PP_SRC_ADC16);
     s.adc = ctx->adc;
     s.flat = (const double *)ctx->flat64.p;
     s.ev_start = (const int64_t *)ctx->ev_start.p;
@@ -216,26 +303,10 @@ PPSource make_source(pp_ctx *ctx)
     return s;
 }
 
-bool has_trace(const pp_ctx *ctx) { return ctx->trace || ctx->trace64 || ctx->trace16; }
-
-// event source of events that are views of the resident trace
-int trace_kind(const pp_ctx *ctx)
-{
-    return ctx->trace64 ? PP_SRC_TRACE64 : ctx->trace16 ? PP_SRC_ADC16 : PP_SRC_TRACE32;
-}
-
-// the resident trace is the buffer `p` of `elem`-byte samples (4: float32, 8: float64, 2: int16 ADC counts)
-void point_trace(pp_ctx *ctx, void *p, size_t elem)
-{
-    ctx->trace = elem == sizeof(float) ? (const float *)p : nullptr;
-    ctx->trace64 = elem == sizeof(double) ? (const double *)p : nullptr;
-    ctx->trace16 = elem == sizeof(int16_t) ? (const int16_t *)p : nullptr;
-}
-
 // float64 samples of the current events and the table that locates an event in them
 const double *f64_samples(pp_ctx *ctx)
 {
-    return ctx->src_kind == PP_SRC_TRACE64 ? ctx->trace64 : (const double *)ctx->flat64.p;
+    return ctx->src_kind == PP_SRC_TRACE64 ? (const double *)ctx->trace : (const double *)ctx->flat64.p;
 }
 const int64_t *f64_bases(pp_ctx *ctx)
 {
@@ -295,10 +366,7 @@ int begin_threshold(pp_ctx *ctx, int64_t scan_len)
     CK(cudaMemsetAsync(ctx->run_maxkey.p, 0, sizeof(unsigned long long) * ctx->cap_runs, ctx->stream));
     ctx->k1_tiles_done = 0;
     ctx->k1_flip = 0;
-    ctx->n_runs = -1;
-    ctx->n_events = ctx->n_event_samples = ctx->n_segments = -1;
-    ctx->stats_valid = false;
-    ctx->prefix_valid = false;
+    drop_from(ctx, LV_RUNS);
     return PP_OK;
 }
 
@@ -337,17 +405,20 @@ int enqueue_threshold_tiles(pp_ctx *ctx, double threshold, int64_t upto, int64_t
 {
     StageRange nvtx_range("pypore:threshold");
     if (ntiles > 0) {
-        if (ctx->trace64) {
-            CKR(launch_threshold_tiles<double>(ctx, ctx->trace64, threshold, 0, upto, ctx->k1_tiles_done, ntiles));
-        } else if (ctx->trace16) {
+        if (ctx->trace_kind == PP_SRC_TRACE64) {
+            CKR(launch_threshold_tiles<double>(ctx, (const double *)ctx->trace, threshold, 0, upto, ctx->k1_tiles_done,
+                                               ntiles));
+        } else if (ctx->trace_kind == PP_SRC_ADC16) {
             int32_t key = 0, kxor = 0;
             pp_adc16_key_threshold(ctx->adc.scale, ctx->adc.offset, threshold, &key, &kxor);
-            CKR(launch_threshold_tiles<int16_t>(ctx, ctx->trace16, key, kxor, upto, ctx->k1_tiles_done, ntiles));
+            CKR(launch_threshold_tiles<int16_t>(ctx, (const int16_t *)ctx->trace, key, kxor, upto, ctx->k1_tiles_done,
+                                                ntiles));
         } else {
             // smallest float32 >= threshold: double(x) < thr  <=>  x < thr_up for every float32 x
             float thr_f = (float)threshold;
             if ((double)thr_f < threshold) thr_f = nextafterf(thr_f, INFINITY);
-            CKR(launch_threshold_tiles<float>(ctx, ctx->trace, thr_f, 0, upto, ctx->k1_tiles_done, ntiles));
+            CKR(launch_threshold_tiles<float>(ctx, (const float *)ctx->trace, thr_f, 0, upto, ctx->k1_tiles_done,
+                                              ntiles));
         }
         ctx->k1_tiles_done += ntiles;
     }
@@ -355,14 +426,14 @@ int enqueue_threshold_tiles(pp_ctx *ctx, double threshold, int64_t upto, int64_t
         upto, ctx->ctr, (const int64_t *)ctx->run_start.p, (const unsigned long long *)ctx->run_minkey.p,
         (const unsigned long long *)ctx->run_maxkey.p, ctx->cap_runs, (int64_t *)ctx->run_len.p,
         (double *)ctx->run_min.p, (double *)ctx->run_max.p, (unsigned char *)ctx->run_below.p,
-        ctx->trace16 != nullptr, ctx->adc);
+        ctx->trace_kind == PP_SRC_ADC16, ctx->adc);
     LAUNCHED(ctx);
     return PP_OK;
 }
 
 int enqueue_threshold(pp_ctx *ctx, double threshold, int64_t scan_len)
 {
-    if (!has_trace(ctx) || ctx->n <= 0) return fail(ctx, PP_ERR_STATE, "no trace resident");
+    if (!ctx->trace || ctx->n <= 0) return fail(ctx, PP_ERR_STATE, "no trace resident");
     if (scan_len < 0 || scan_len > ctx->n) scan_len = ctx->n;
     CKR(begin_threshold(ctx, scan_len));
     return enqueue_threshold_tiles(ctx, threshold, scan_len, (scan_len + K1_TILE - 1) / K1_TILE);
@@ -373,7 +444,7 @@ int enqueue_select(pp_ctx *ctx, int rule_mask, int64_t duration_gt, int64_t dura
                    const long long *dev_plan = nullptr)
 {
     StageRange nvtx_range("pypore:select");
-    ctx->src_kind = trace_kind(ctx);
+    ctx->src_kind = ctx->trace_kind;
     ctx->flat_cap = ctx->n;
     k1_select_events<<<1, SEL_THREADS, 0, ctx->stream>>>(
         ctx->ctr, (const int64_t *)ctx->run_start.p, (const int64_t *)ctx->run_len.p,
@@ -381,9 +452,7 @@ int enqueue_select(pp_ctx *ctx, int rule_mask, int64_t duration_gt, int64_t dura
         duration_gt, duration_lt, min_gt, max_lt, skip_first, skip_last, (int64_t *)ctx->ev_start.p,
         (int64_t *)ctx->ev_len.p, (int64_t *)ctx->ev_off.p, ctx->cap_events, incremental, dev_plan);
     LAUNCHED(ctx);
-    ctx->n_events = ctx->n_event_samples = ctx->n_segments = -1;
-    ctx->stats_valid = false;
-    ctx->prefix_valid = false;
+    drop_from(ctx, LV_EVENTS);
     return PP_OK;
 }
 
@@ -437,11 +506,8 @@ int enqueue_filter(pp_ctx *ctx, const double *b, const double *a, const double *
         LAUNCHED(ctx);
     }
     ctx->src_kind = PP_SRC_FLAT64;  // from here on the events' current is the filtered float64 signal
-    CKR(record_boundary(ctx, ST_FILTER + 1));
-    ctx->stage_ran[ST_FILTER] = true;
-    ctx->n_segments = -1;
-    ctx->stats_valid = false;
-    ctx->prefix_valid = false;
+    CKR(end_stage(ctx, ST_FILTER));
+    drop_from(ctx, LV_PREFIX);
     return PP_OK;
 }
 
@@ -539,8 +605,8 @@ int enqueue_prefix(pp_ctx *ctx, int prefix_mode)
                                                      (int64_t *)ctx->ev_tile_off.p, (K2EventBits *)ctx->k2_bits.p,
                                                      (unsigned *)ctx->inexact.p);
         LAUNCHED(ctx);
-        if (ctx->src_kind == PP_SRC_TRACE32) CKR(enqueue_prefix_tiled<float>(ctx, src, ctx->trace, prefix_mode));
-        else if (ctx->src_kind == PP_SRC_ADC16) CKR(enqueue_prefix_tiled<int16_t>(ctx, src, ctx->trace16, prefix_mode));
+        if (ctx->src_kind == PP_SRC_TRACE32) CKR(enqueue_prefix_tiled<float>(ctx, src, src.trace, prefix_mode));
+        else if (ctx->src_kind == PP_SRC_ADC16) CKR(enqueue_prefix_tiled<int16_t>(ctx, src, src.trace16, prefix_mode));
         else CKR(enqueue_prefix_tiled<double>(ctx, src, f64_samples(ctx), prefix_mode));
         if (prefix_mode != PP_PREFIX_PARALLEL) {
             k2_prefix_sequential<<<ctx->sm_count * 3, K2S_WARPS * 32, 0, ctx->stream>>>(
@@ -644,17 +710,12 @@ int enqueue_split(pp_ctx *ctx, int mw, int MW, int W, double min_gain, int prefi
     CKR(prepare_split(ctx, mw, MW, W));
     CKR(enqueue_prefix(ctx, prefix_mode));
     ctx->prefix_valid = true;
-    CKR(record_boundary(ctx, ST_PREFIX + 1));
-    ctx->stage_ran[ST_PREFIX] = true;
+    drop_from(ctx, LV_SEGMENTS);
+    CKR(end_stage(ctx, ST_PREFIX));
     CKR(enqueue_search(ctx, mw, MW, W, min_gain));
-    CKR(record_boundary(ctx, ST_SPLIT + 1));
-    ctx->stage_ran[ST_SPLIT] = true;
+    CKR(end_stage(ctx, ST_SPLIT));
     CKR(enqueue_compact(ctx));
-    CKR(record_boundary(ctx, ST_COMPACT + 1));
-    ctx->stage_ran[ST_COMPACT] = true;
-    ctx->n_segments = -1;
-    ctx->stats_valid = false;
-    return PP_OK;
+    return end_stage(ctx, ST_COMPACT);
 }
 
 // K4 over the rows of the current event source: segments (flat_start = seg_flat, row_event = seg_event) or whole
@@ -666,12 +727,12 @@ int launch_stats(pp_ctx *ctx, int rows_are_events, const int64_t *flat_start, co
     const int64_t *ev_off = (const int64_t *)ctx->ev_off.p;
     if (ctx->src_kind == PP_SRC_TRACE32)
         k4_segment_stats<float><<<grid, 256, 0, ctx->stream>>>(
-            ctx->trace, (const int64_t *)ctx->ev_start.p, ev_off, ctx->ctr, rows_are_events, flat_start, row_event,
-            cap_rows, mean, sd, mn, mx, ctx->adc);
+            (const float *)ctx->trace, (const int64_t *)ctx->ev_start.p, ev_off, ctx->ctr, rows_are_events, flat_start,
+            row_event, cap_rows, mean, sd, mn, mx, ctx->adc);
     else if (ctx->src_kind == PP_SRC_ADC16)
         k4_segment_stats<int16_t><<<grid, 256, 0, ctx->stream>>>(
-            ctx->trace16, (const int64_t *)ctx->ev_start.p, ev_off, ctx->ctr, rows_are_events, flat_start, row_event,
-            cap_rows, mean, sd, mn, mx, ctx->adc);
+            (const int16_t *)ctx->trace, (const int64_t *)ctx->ev_start.p, ev_off, ctx->ctr, rows_are_events, flat_start,
+            row_event, cap_rows, mean, sd, mn, mx, ctx->adc);
     else
         k4_segment_stats<double><<<grid, 256, 0, ctx->stream>>>(
             f64_samples(ctx), f64_bases(ctx), ev_off, ctx->ctr, rows_are_events, flat_start, row_event, cap_rows,
@@ -686,8 +747,7 @@ int enqueue_stats(pp_ctx *ctx)
     CKR(launch_stats(ctx, 0, (const int64_t *)ctx->seg_flat.p, (const int *)ctx->seg_event.p, ctx->cap_segs,
                      (double *)ctx->seg_mean.p, (double *)ctx->seg_std.p, (double *)ctx->seg_min.p,
                      (double *)ctx->seg_max.p));
-    CKR(record_boundary(ctx, ST_STATS + 1));
-    ctx->stage_ran[ST_STATS] = true;
+    CKR(end_stage(ctx, ST_STATS));
     ctx->stats_valid = true;
     return PP_OK;
 }
@@ -716,6 +776,50 @@ void absorb_counters(pp_ctx *ctx)
     ctx->split_counters[5] = (int64_t)h->n_sure;
     ctx->split_counters[6] = (int64_t)h->n_multi;
     ctx->split_counters[7] = (int64_t)h->n_full;
+}
+
+// End of a pipeline call, counters fetched: the table sizes the device counted, out = runs, events, event samples,
+// segments
+int commit_counters(pp_ctx *ctx, int64_t out[4])
+{
+    absorb_counters(ctx);
+    CKR(check_overflow(ctx));
+    ctx->n_segments = (int64_t)ctx->h_ctr->n_segments;
+    if (out) {
+        out[0] = ctx->n_runs;
+        out[1] = ctx->n_events;
+        out[2] = ctx->n_event_samples;
+        out[3] = ctx->n_segments;
+    }
+    return PP_OK;
+}
+
+// Enqueue a call that begins with a threshold scan, then fetch the counters; a run table that overflowed is regrown
+// to what the scan counted and the call repeats once
+template <typename Enqueue>
+int with_run_retry(pp_ctx *ctx, Enqueue enqueue)
+{
+    for (int attempt = 0; attempt < 2; ++attempt) {
+        CKR(enqueue());
+        CKR(fetch_counters(ctx));
+        const int64_t runs = (int64_t)ctx->h_ctr->n_runs;
+        if (runs <= ctx->cap_runs) {
+            ctx->n_runs = runs;
+            return PP_OK;
+        }
+        CKR(ensure_run_buffers(ctx, runs + 16));
+    }
+    return fail(ctx, PP_ERR_CAPACITY, "run table overflow");
+}
+
+// Copy the rows not exported yet to the host tables and wait for them; tables too small for every row fail with
+// PP_ERR_CAPACITY (the device tables stay whole)
+int export_tables(pp_ctx *ctx, const PPHostTables &H, int with_stats)
+{
+    CKR(enqueue_export(ctx, H, with_stats));
+    CKR(fetch_counters(ctx));
+    if (ctx->h_ctr->overflow & PP_OVF_EXPORT) return fail(ctx, PP_ERR_CAPACITY, "host tables too small");
+    return PP_OK;
 }
 
 }  // namespace
@@ -779,16 +883,6 @@ void pp_destroy(pp_ctx *ctx)
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
     for (int q = 0; q < 64; ++q)
         if (ctx->ctl_ipc[q] && ctx->ctl_peers[q]) cudaIpcCloseMemHandle(ctx->ctl_peers[q]);
-    DevBuf *bufs[] = {&ctx->trace_buf, &ctx->pend[0].buf, &ctx->pend[1].buf, &ctx->trace_spare, &ctx->k1_rec, &ctx->k1_staged, &ctx->k1_blk, &ctx->run_start, &ctx->run_minkey,
-                      &ctx->run_maxkey, &ctx->run_len, &ctx->run_min, &ctx->run_max, &ctx->run_below,
-                      &ctx->ev_start, &ctx->ev_len, &ctx->ev_off, &ctx->flat64, &ctx->cc, &ctx->bits,
-                      &ctx->tasks, &ctx->ready, &ctx->block_count, &ctx->block_off, &ctx->inexact, &ctx->Ttab, &ctx->ev_tile_off, &ctx->k2_bits, &ctx->k2_tiles,
-                      &ctx->seg_flat, &ctx->seg_event, &ctx->seg_start, &ctx->seg_end, &ctx->seg_mean,
-                      &ctx->seg_std, &ctx->seg_min, &ctx->seg_max, &ctx->evs_mean, &ctx->evs_std,
-                      &ctx->evs_min, &ctx->evs_max, &ctx->filt_tmp, &ctx->filt_carry, &ctx->filt_coef, &ctx->hk, &ctx->unpack_flag, &ctx->ctl_buf, &ctx->ctl_peers_dev,
-                      &ctx->hmm_model, &ctx->hmm_x, &ctx->hmm_off, &ctx->hmm_logp, &ctx->hmm_state, &ctx->hmm_bp,
-                      &ctx->hmm_next, &ctx->hmm_old_flat, &ctx->hmm_old_state};
-    for (DevBuf *b : bufs) release(*b);
     if (ctx->ctr) cudaFree(ctx->ctr);
     if (ctx->h_ctr) cudaFreeHost(ctx->h_ctr);
     for (int i = 0; i <= ST_COUNT; ++i)
@@ -804,7 +898,7 @@ void pp_destroy(pp_ctx *ctx)
     }
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
-    delete ctx;
+    delete ctx;   // the device buffers free themselves
 }
 
 const char *pp_last_error(pp_ctx *ctx) { return ctx ? ctx->err : "null context"; }
@@ -875,29 +969,25 @@ int pp_stage_ms(pp_ctx *ctx, int stage, float *ms)
 }
 
 // ---- trace ------------------------------------------------------------------
-static int trace_upload_impl(pp_ctx *ctx, const void *host, int64_t n, int64_t extra_capacity, size_t elem)
+static int trace_upload_impl(pp_ctx *ctx, const void *host, int64_t n, int64_t extra_capacity, int kind)
 {
     if (!ctx || !host || n <= 0 || extra_capacity < 0) return fail(ctx, PP_ERR_ARG, "bad trace");
+    const size_t elem = sample_bytes(kind);
     CKR(set_device(ctx));
     CKR(ensure(ctx, ctx->trace_buf, elem * (size_t)(n + extra_capacity)));
     CK(cudaMemcpyAsync(ctx->trace_buf.p, host, elem * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-    point_trace(ctx, ctx->trace_buf.p, elem);
-    ctx->n = n;
-    ctx->trace_cap = (int64_t)(ctx->trace_buf.cap / elem);
-    ctx->adopted = false;
-    ctx->n_runs = ctx->n_events = ctx->n_event_samples = ctx->n_segments = -1;
-    ctx->prefix_valid = false;
+    set_trace(ctx, ctx->trace_buf.p, kind, n, (int64_t)(ctx->trace_buf.cap / elem));
     return PP_OK;
 }
 
 int pp_trace_upload(pp_ctx *ctx, const float *host, int64_t n, int64_t extra_capacity)
 {
-    return trace_upload_impl(ctx, host, n, extra_capacity, sizeof(float));
+    return trace_upload_impl(ctx, host, n, extra_capacity, PP_SRC_TRACE32);
 }
 
 int pp_trace_upload_f64(pp_ctx *ctx, const double *host, int64_t n)
 {
-    return trace_upload_impl(ctx, host, n, 0, sizeof(double));
+    return trace_upload_impl(ctx, host, n, 0, PP_SRC_TRACE64);
 }
 
 // decode(c) on the host: the product is rounded on its own (no contraction into an FMA), like the device's
@@ -937,7 +1027,7 @@ int pp_trace_upload_adc16(pp_ctx *ctx, const int16_t *host, int64_t n, double sc
 {
     if (pp_adc16_check(scale, offset) != PP_OK)
         return fail(ctx, PP_ERR_ARG, "ADC scale must be finite and non-zero, offset finite, every count decoding finite");
-    CKR(trace_upload_impl(ctx, host, n, 0, sizeof(int16_t)));
+    CKR(trace_upload_impl(ctx, host, n, 0, PP_SRC_ADC16));
     ctx->adc = PPAdc{scale, offset};
     return PP_OK;
 }
@@ -956,7 +1046,7 @@ static int ensure_copy_stream(pp_ctx *ctx)
 int pp_trace_prefetch(pp_ctx *ctx, const float *host, int64_t n, int64_t extra_capacity)
 {
     if (!ctx || !host || n <= 0 || extra_capacity < 0) return fail(ctx, PP_ERR_ARG, "bad trace");
-    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "prefetch takes float32 traces; an ADC trace is resident");
+    CKR(require_trace(ctx, NOT_ADC, "prefetch takes float32 traces"));
     if (ctx->n_pend >= 2) return fail(ctx, PP_ERR_STATE, "two prefetched traces are already waiting for pp_trace_swap");
     CKR(set_device(ctx));
     CKR(ensure_copy_stream(ctx));
@@ -966,10 +1056,7 @@ int pp_trace_prefetch(pp_ctx *ctx, const float *host, int64_t n, int64_t extra_c
         CK(cudaEventCreate(&q.t0));
         CK(cudaEventCreate(&q.t1));
     }
-    if (!q.buf.p && ctx->trace_spare.p) {     // the buffer the last swap retired
-        q.buf = ctx->trace_spare;
-        ctx->trace_spare = DevBuf();
-    }
+    if (!q.buf.p) q.buf = std::move(ctx->trace_spare);     // the buffer the last swap retired, if any
     CKR(ensure(ctx, q.buf, sizeof(float) * (size_t)(n + extra_capacity)));
     // the buffer was the resident trace some swaps ago: whatever still reads it was enqueued before this point
     CK(cudaEventRecord(ctx->compute_ev, ctx->stream));
@@ -1001,28 +1088,17 @@ int pp_trace_swap(pp_ctx *ctx)
     pp_ctx::Pending &q = ctx->pend[0];
     CK(cudaStreamWaitEvent(ctx->stream, q.done, 0));   // stream-level: the host goes on
     // the retired resident buffer becomes the spare one (an older spare is dropped: at most three buffers live)
-    if (ctx->trace_spare.p) release(ctx->trace_spare);
-    ctx->trace_spare = ctx->trace_buf;
-    ctx->trace_buf = q.buf;
-    q.buf = DevBuf();
+    ctx->trace_spare = std::move(ctx->trace_buf);
+    ctx->trace_buf = std::move(q.buf);
     // the timing events of the trace swapped in are what pp_trace_prefetch_ms reads
     cudaEvent_t a = ctx->pf_t0, b = ctx->pf_t1;
     ctx->pf_t0 = q.t0; ctx->pf_t1 = q.t1;
     q.t0 = a; q.t1 = b;
     if (!q.t0) { CK(cudaEventCreate(&q.t0)); CK(cudaEventCreate(&q.t1)); }
-    point_trace(ctx, ctx->trace_buf.p, sizeof(float));
-    ctx->n = q.n;
+    set_trace(ctx, ctx->trace_buf.p, PP_SRC_TRACE32, q.n, (int64_t)(ctx->trace_buf.cap / sizeof(float)));
     q.n = -1;
-    if (ctx->n_pend == 2) {       // the younger one moves up
-        pp_ctx::Pending t = ctx->pend[0];
-        ctx->pend[0] = ctx->pend[1];
-        ctx->pend[1] = t;
-    }
+    if (ctx->n_pend == 2) std::swap(ctx->pend[0], ctx->pend[1]);   // the younger one moves up
     --ctx->n_pend;
-    ctx->trace_cap = (int64_t)(ctx->trace_buf.cap / sizeof(float));
-    ctx->adopted = false;
-    ctx->n_runs = ctx->n_events = ctx->n_event_samples = ctx->n_segments = -1;
-    ctx->prefix_valid = false;
     return PP_OK;
 }
 
@@ -1030,23 +1106,18 @@ int pp_trace_adopt(pp_ctx *ctx, const float *dev, int64_t n, int64_t capacity)
 {
     if (!ctx || !dev || n <= 0 || capacity < n) return fail(ctx, PP_ERR_ARG, "bad trace");
     if (((uintptr_t)dev) & 15) return fail(ctx, PP_ERR_ARG, "device trace must be 16-byte aligned");
-    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "adopt takes float32 traces; an ADC trace is resident");
-    point_trace(ctx, (void *)dev, sizeof(float));
-    ctx->n = n;
-    ctx->trace_cap = capacity;
-    ctx->adopted = true;
-    ctx->n_runs = ctx->n_events = ctx->n_event_samples = ctx->n_segments = -1;
-    ctx->prefix_valid = false;
+    CKR(require_trace(ctx, NOT_ADC, "adopt takes float32 traces"));
+    set_trace(ctx, dev, PP_SRC_TRACE32, n, capacity);
     return PP_OK;
 }
 
 int pp_trace_append(pp_ctx *ctx, const float *src, int64_t n, int src_is_device)
 {
     if (!ctx || !src || n < 0) return fail(ctx, PP_ERR_ARG, "bad append");
-    if (!ctx->trace) return fail(ctx, PP_ERR_STATE, "no float32 trace resident");
+    CKR(require_trace(ctx, TAKES_F32, "append takes float32 traces"));
     if (ctx->n + n > ctx->trace_cap) return fail(ctx, PP_ERR_CAPACITY, "trace capacity exceeded");
     CKR(set_device(ctx));
-    CK(cudaMemcpyAsync((void *)(ctx->trace + ctx->n), src, sizeof(float) * (size_t)n,
+    CK(cudaMemcpyAsync((float *)ctx->trace + ctx->n, src, sizeof(float) * (size_t)n,
                        src_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, ctx->stream));
     ctx->n += n;
     return PP_OK;
@@ -1062,53 +1133,34 @@ int pp_trace_truncate(pp_ctx *ctx, int64_t n)
 int pp_trace_extend(pp_ctx *ctx, int64_t n)
 {
     if (!ctx || n < 0) return fail(ctx, PP_ERR_ARG, "bad extend");
-    if (!ctx->trace) return fail(ctx, PP_ERR_STATE, "no float32 trace resident");
+    CKR(require_trace(ctx, TAKES_F32, "extend takes float32 traces"));
     if (ctx->n + n > ctx->trace_cap) return fail(ctx, PP_ERR_CAPACITY, "trace capacity exceeded");
     ctx->n += n;
     return PP_OK;
 }
 
 int64_t pp_trace_len(pp_ctx *ctx) { return ctx ? ctx->n : 0; }
-const float *pp_trace_device_ptr(pp_ctx *ctx) { return ctx ? ctx->trace : nullptr; }
+const float *pp_trace_device_ptr(pp_ctx *ctx) { return ctx ? trace_as<float>(ctx, PP_SRC_TRACE32) : nullptr; }
 
 // ---- K1 -----------------------------------------------------------------------
 int pp_threshold_scan(pp_ctx *ctx, double threshold, int64_t scan_len, int64_t *n_runs)
 {
     if (!ctx) return PP_ERR_ARG;
-    CKR(set_device(ctx));
-    for (int attempt = 0; attempt < 2; ++attempt) {
-        reset_stages(ctx);
-        CKR(record_boundary(ctx, 0));
+    CKR(with_run_retry(ctx, [&]() -> int {
+        CKR(begin_call(ctx, 0));
         CKR(enqueue_threshold(ctx, threshold, scan_len));
-        CKR(record_boundary(ctx, ST_THRESHOLD + 1));
-        ctx->stage_ran[ST_THRESHOLD] = true;
-        CKR(fetch_counters(ctx));
-        const int64_t runs = (int64_t)ctx->h_ctr->n_runs;
-        if (runs <= ctx->cap_runs) {
-            ctx->n_runs = runs;
-            if (n_runs) *n_runs = runs;
-            return PP_OK;
-        }
-        CKR(ensure_run_buffers(ctx, runs + 16));
-    }
-    return fail(ctx, PP_ERR_CAPACITY, "run table overflow");
+        return end_stage(ctx, ST_THRESHOLD);
+    }));
+    if (n_runs) *n_runs = ctx->n_runs;
+    return PP_OK;
 }
 
 int pp_runs_download(pp_ctx *ctx, int64_t cap, int64_t *start, int64_t *length, double *mn,
                      double *mx, uint8_t *below)
 {
     if (!ctx) return PP_ERR_ARG;
-    if (ctx->n_runs < 0) return fail(ctx, PP_ERR_STATE, "pp_threshold_scan has not run");
     if (cap < ctx->n_runs) return fail(ctx, PP_ERR_CAPACITY, "run buffers too small");
-    CKR(set_device(ctx));
-    const size_t r = (size_t)ctx->n_runs;
-    if (start) CK(cudaMemcpyAsync(start, ctx->run_start.p, 8 * r, cudaMemcpyDeviceToHost, ctx->stream));
-    if (length) CK(cudaMemcpyAsync(length, ctx->run_len.p, 8 * r, cudaMemcpyDeviceToHost, ctx->stream));
-    if (mn) CK(cudaMemcpyAsync(mn, ctx->run_min.p, 8 * r, cudaMemcpyDeviceToHost, ctx->stream));
-    if (mx) CK(cudaMemcpyAsync(mx, ctx->run_max.p, 8 * r, cudaMemcpyDeviceToHost, ctx->stream));
-    if (below) CK(cudaMemcpyAsync(below, ctx->run_below.p, r, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    return PP_OK;
+    return pp_runs_download_range(ctx, 0, ctx->n_runs, start, length, mn, mx, below);
 }
 
 int pp_runs_download_range(pp_ctx *ctx, int64_t first, int64_t count, int64_t *start, int64_t *length,
@@ -1138,8 +1190,7 @@ int pp_select_events(pp_ctx *ctx, int rule_mask, int64_t duration_gt, int64_t du
     if (ctx->n_runs < 0) return fail(ctx, PP_ERR_STATE, "pp_threshold_scan has not run");
     CKR(set_device(ctx));
     CKR(enqueue_select(ctx, rule_mask, duration_gt, duration_lt, min_gt, max_lt, skip_first, skip_last));
-    CKR(record_boundary(ctx, ST_SELECT + 1));
-    ctx->stage_ran[ST_SELECT] = true;
+    CKR(end_stage(ctx, ST_SELECT));
     CKR(fetch_counters(ctx));
     absorb_counters(ctx);
     if (n_events) *n_events = ctx->n_events;
@@ -1151,7 +1202,7 @@ int pp_set_events(pp_ctx *ctx, const int64_t *start, const int64_t *length, int6
 {
     if (!ctx || n_events < 0 || (n_events > 0 && (!start || !length)))
         return fail(ctx, PP_ERR_ARG, "bad events");
-    if (!has_trace(ctx)) return fail(ctx, PP_ERR_STATE, "no trace resident");
+    if (!ctx->trace) return fail(ctx, PP_ERR_STATE, "no trace resident");
     CKR(set_device(ctx));
     for (int64_t i = 0; i < n_events; ++i)
         if (start[i] < 0 || length[i] <= 0 || start[i] + length[i] > ctx->n)
@@ -1164,16 +1215,14 @@ int pp_set_events(pp_ctx *ctx, const int64_t *start, const int64_t *length, int6
     k1_event_offsets<<<1, SEL_THREADS, 0, ctx->stream>>>(ctx->ctr, (const int64_t *)ctx->ev_len.p, n_events,
                                                          (int64_t *)ctx->ev_off.p);
     LAUNCHED(ctx);
-    ctx->src_kind = trace_kind(ctx);
+    ctx->src_kind = ctx->trace_kind;
     int64_t tot = 0;
     for (int64_t i = 0; i < n_events; ++i) tot += length[i];
     ctx->flat_cap = tot > 0 ? tot : 1;
     CK(cudaStreamSynchronize(ctx->stream));  // host arrays may be freed by the caller
+    drop_from(ctx, LV_EVENTS);
     ctx->n_events = n_events;
     ctx->n_event_samples = tot;
-    ctx->n_segments = -1;
-    ctx->stats_valid = false;
-    ctx->prefix_valid = false;
     return PP_OK;
 }
 
@@ -1201,7 +1250,7 @@ int pp_append_event(pp_ctx *ctx, int64_t start, int64_t length)
     LAUNCHED(ctx);
     ctx->n_events += 1;
     ctx->n_event_samples += length;
-    ctx->prefix_valid = false;
+    drop_from(ctx, LV_PREFIX);
     if (ctx->flat_cap < ctx->n) ctx->flat_cap = ctx->n;
     return PP_OK;
 }
@@ -1242,11 +1291,9 @@ int pp_events_upload_f64(pp_ctx *ctx, const double *host, const int64_t *length,
     CK(cudaStreamSynchronize(ctx->stream));
     ctx->src_kind = PP_SRC_FLAT64;
     ctx->flat_cap = tot;
+    drop_from(ctx, LV_EVENTS);
     ctx->n_events = n_events;
     ctx->n_event_samples = tot;
-    ctx->n_segments = -1;
-    ctx->stats_valid = false;
-    ctx->prefix_valid = false;
     return PP_OK;
 }
 
@@ -1256,9 +1303,7 @@ int pp_filter_events(pp_ctx *ctx, const double *b, const double *a, const double
     if (!ctx || !b || !a || ncoef < 2 || ncoef > FILT_MAX_COEF || (ncoef > 1 && !zi))
         return fail(ctx, PP_ERR_ARG, "bad filter coefficients");
     if (ctx->n_events < 0) return fail(ctx, PP_ERR_STATE, "no event table");
-    CKR(set_device(ctx));
-    reset_stages(ctx);
-    CKR(record_boundary(ctx, ST_FILTER));
+    CKR(begin_call(ctx, ST_FILTER));
     CKR(enqueue_filter(ctx, b, a, zi, ncoef));
     CKR(fetch_counters(ctx));
     return check_overflow(ctx);
@@ -1283,14 +1328,10 @@ int pp_statsplit(pp_ctx *ctx, int min_width, int max_width, int window_width, do
 {
     if (!ctx) return PP_ERR_ARG;
     if (ctx->n_events < 0) return fail(ctx, PP_ERR_STATE, "no event table");
-    CKR(set_device(ctx));
-    reset_stages(ctx);
-    CKR(record_boundary(ctx, ST_PREFIX));
+    CKR(begin_call(ctx, ST_PREFIX));
     CKR(enqueue_split(ctx, min_width, max_width, window_width, min_gain, prefix_mode));
     CKR(fetch_counters(ctx));
-    absorb_counters(ctx);
-    CKR(check_overflow(ctx));
-    ctx->n_segments = (int64_t)ctx->h_ctr->n_segments;
+    CKR(commit_counters(ctx, nullptr));
     if (n_segments) *n_segments = ctx->n_segments;
     return PP_OK;
 }
@@ -1317,55 +1358,43 @@ int pp_window_gains(pp_ctx *ctx, int64_t ev, int n_windows, const int32_t *ps, c
     if (!ctx->prefix_valid) return fail(ctx, PP_ERR_STATE, "prefix sums are not resident (pp_prefix / pp_statsplit)");
     if (ev < 0 || ev >= ctx->n_events) return fail(ctx, PP_ERR_ARG, "bad event index");
     CKR(set_device(ctx));
-    int64_t *off = (int64_t *)malloc(sizeof(int64_t) * (size_t)n_windows);
-    if (!off) return fail(ctx, PP_ERR_ARG, "out of host memory");
+    std::vector<int64_t> off;
+    CKR(host_scratch(ctx, off, (size_t)n_windows));
     int64_t total = 0;
     for (int w = 0; w < n_windows; ++w) {
         off[w] = total;
         const int64_t n = (int64_t)pe[w] - ps[w] - 2LL * min_width + 1;
-        if (ps[w] < 0 || pe[w] < ps[w]) { free(off); return fail(ctx, PP_ERR_ARG, "bad window %d", w); }
+        if (ps[w] < 0 || pe[w] < ps[w]) return fail(ctx, PP_ERR_ARG, "bad window %d", w);
         if (n > 0) total += n;
     }
-    if (total > cap) { free(off); return fail(ctx, PP_ERR_CAPACITY, "gain buffer too small"); }
+    if (total > cap) return fail(ctx, PP_ERR_CAPACITY, "gain buffer too small");
     DevBuf d_ps, d_pe, d_off, d_out;
-    // every CUDA call checked; the scratch buffers are released on every path
-    auto run = [&]() -> int {
-        CKR(ensure(ctx, d_ps, 4 * (size_t)n_windows));
-        CKR(ensure(ctx, d_pe, 4 * (size_t)n_windows));
-        CKR(ensure(ctx, d_off, 8 * (size_t)n_windows));
-        CKR(ensure(ctx, d_out, 8 * (size_t)(total > 0 ? total : 1)));
-        CK(cudaMemcpyAsync(d_ps.p, ps, 4 * (size_t)n_windows, cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(d_pe.p, pe, 4 * (size_t)n_windows, cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(d_off.p, off, 8 * (size_t)n_windows, cudaMemcpyHostToDevice, ctx->stream));
-        K3Global G;
-        memset(&G, 0, sizeof G);
-        G.cc = (const double2 *)ctx->cc.p;
-        G.ev_off = (const int64_t *)ctx->ev_off.p;
-        const dim3 grid(32, n_windows < 4096 ? n_windows : 4096);
-        k3_window_gains<<<grid, 256, 0, ctx->stream>>>(G, (int)ev, n_windows, (const int *)d_ps.p,
-                                                       (const int *)d_pe.p, min_width, (const int64_t *)d_off.p,
-                                                       (double *)d_out.p);
-        LAUNCHED(ctx);
-        if (total > 0)
-            CK(cudaMemcpyAsync(out, d_out.p, 8 * (size_t)total, cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-        return PP_OK;
-    };
-    const int rc = run();
-    release(d_ps); release(d_pe); release(d_off); release(d_out);
-    free(off);
-    return rc;
+    CKR(ensure(ctx, d_ps, 4 * (size_t)n_windows));
+    CKR(ensure(ctx, d_pe, 4 * (size_t)n_windows));
+    CKR(ensure(ctx, d_off, 8 * (size_t)n_windows));
+    CKR(ensure(ctx, d_out, 8 * (size_t)(total > 0 ? total : 1)));
+    CK(cudaMemcpyAsync(d_ps.p, ps, 4 * (size_t)n_windows, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_pe.p, pe, 4 * (size_t)n_windows, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_off.p, off.data(), 8 * (size_t)n_windows, cudaMemcpyHostToDevice, ctx->stream));
+    K3Global G;
+    memset(&G, 0, sizeof G);
+    G.cc = (const double2 *)ctx->cc.p;
+    G.ev_off = (const int64_t *)ctx->ev_off.p;
+    const dim3 grid(32, n_windows < 4096 ? n_windows : 4096);
+    k3_window_gains<<<grid, 256, 0, ctx->stream>>>(G, (int)ev, n_windows, (const int *)d_ps.p, (const int *)d_pe.p,
+                                                   min_width, (const int64_t *)d_off.p, (double *)d_out.p);
+    LAUNCHED(ctx);
+    if (total > 0) CK(cudaMemcpyAsync(out, d_out.p, 8 * (size_t)total, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return PP_OK;
 }
 
 int pp_segment_stats(pp_ctx *ctx)
 {
     if (!ctx) return PP_ERR_ARG;
     if (ctx->n_segments < 0) return fail(ctx, PP_ERR_STATE, "pp_statsplit has not run");
-    CKR(set_device(ctx));
-    reset_stages(ctx);
-    CKR(record_boundary(ctx, ST_STATS));
-    CKR(enqueue_stats(ctx));
-    return PP_OK;
+    CKR(begin_call(ctx, ST_STATS));
+    return enqueue_stats(ctx);
 }
 
 int pp_segments_download(pp_ctx *ctx, int64_t cap, int32_t *event, int64_t *start, int64_t *end,
@@ -1462,7 +1491,6 @@ int pp_debug_screen(pp_ctx *ctx, int64_t ev, int ps, int pe, int min_width, doub
     CK(cudaMemcpyAsync(h_exact, b.p, 8 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(ok, c.p, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    release(a); release(b); release(c);
     if (eps) *eps = (double)(pe - ps) * K3_EPS_PER_SAMPLE + K3_EPS_CONST;
     return PP_OK;
 }
@@ -1474,25 +1502,19 @@ int pp_debug_prefix(pp_ctx *ctx, int64_t cap, double *c, double *c2, uint8_t *re
     if (cap < ctx->n_event_samples || cap < ctx->n_events) return fail(ctx, PP_ERR_CAPACITY, "buffers too small");
     CKR(set_device(ctx));
     const size_t n = (size_t)ctx->n_event_samples, e = (size_t)ctx->n_events;
-    double2 *cc = (double2 *)malloc(sizeof(double2) * (n ? n : 1));
-    unsigned *fl = (unsigned *)malloc(sizeof(unsigned) * (e ? e : 1));
-    if (!cc || !fl) { free(cc); free(fl); return fail(ctx, PP_ERR_ARG, "out of host memory"); }
-    auto run = [&]() -> int {
-        if (n) CK(cudaMemcpyAsync(cc, ctx->cc.p, sizeof(double2) * n, cudaMemcpyDeviceToHost, ctx->stream));
-        if (e && ctx->prefix_mode == PP_PREFIX_AUTO)
-            CK(cudaMemcpyAsync(fl, ctx->inexact.p, sizeof(unsigned) * e, cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-        return PP_OK;
-    };
-    const int rc = run();
-    if (rc == PP_OK) {
-        for (size_t i = 0; i < n; ++i) { c[i] = cc[i].x; c2[i] = cc[i].y; }
-        // PARALLEL redoes nothing, SEQUENTIAL runs every event in the strict order
-        for (size_t i = 0; i < e; ++i)
-            redone[i] = ctx->prefix_mode == PP_PREFIX_AUTO ? (fl[i] != 0u) : ctx->prefix_mode == PP_PREFIX_SEQUENTIAL;
-    }
-    free(cc); free(fl);
-    return rc;
+    std::vector<double2> cc;
+    std::vector<unsigned> fl;
+    CKR(host_scratch(ctx, cc, n));
+    CKR(host_scratch(ctx, fl, e));
+    if (n) CK(cudaMemcpyAsync(cc.data(), ctx->cc.p, sizeof(double2) * n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (e && ctx->prefix_mode == PP_PREFIX_AUTO)
+        CK(cudaMemcpyAsync(fl.data(), ctx->inexact.p, sizeof(unsigned) * e, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    for (size_t i = 0; i < n; ++i) { c[i] = cc[i].x; c2[i] = cc[i].y; }
+    // PARALLEL redoes nothing, SEQUENTIAL runs every event in the strict order
+    for (size_t i = 0; i < e; ++i)
+        redone[i] = ctx->prefix_mode == PP_PREFIX_AUTO ? (fl[i] != 0u) : ctx->prefix_mode == PP_PREFIX_SEQUENTIAL;
+    return PP_OK;
 }
 
 int pp_debug_lg2_error(pp_ctx *ctx, double *max_err)
@@ -1506,7 +1528,6 @@ int pp_debug_lg2_error(pp_ctx *ctx, double *max_err)
     LAUNCHED(ctx);
     CK(cudaMemcpyAsync(max_err, a.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    release(a);
     return PP_OK;
 }
 
@@ -1514,52 +1535,29 @@ int pp_debug_lg2_error(pp_ctx *ctx, double *max_err)
 int pp_pipeline(pp_ctx *ctx, const pp_pipeline_params *p, int64_t out[4])
 {
     if (!ctx || !p) return PP_ERR_ARG;
-    CKR(set_device(ctx));
-    for (int attempt = 0; attempt < 2; ++attempt) {
-        reset_stages(ctx);
-        CKR(record_boundary(ctx, 0));
+    CKR(with_run_retry(ctx, [&]() -> int {
+        CKR(begin_call(ctx, 0));
         CKR(enqueue_threshold(ctx, p->threshold, -1));
-        CKR(record_boundary(ctx, ST_THRESHOLD + 1));
-        ctx->stage_ran[ST_THRESHOLD] = true;
+        CKR(end_stage(ctx, ST_THRESHOLD));
         CKR(enqueue_select(ctx, p->rule_mask, p->duration_gt, p->duration_lt, p->min_gt, p->max_lt, 0, 0));
-        CKR(record_boundary(ctx, ST_SELECT + 1));
-        ctx->stage_ran[ST_SELECT] = true;
+        CKR(end_stage(ctx, ST_SELECT));
         if (p->filter_ncoef > 0)
             CKR(enqueue_filter(ctx, p->filter_b, p->filter_a, p->filter_zi, p->filter_ncoef));
         CKR(enqueue_split(ctx, p->min_width, p->max_width, p->window_width, p->min_gain, p->prefix_mode));
         if (p->with_stats) CKR(enqueue_stats(ctx));
-        CKR(fetch_counters(ctx));
-        const int64_t runs = (int64_t)ctx->h_ctr->n_runs;
-        if (runs > ctx->cap_runs) {  // rare: noisy trace with many crossings; grow and redo
-            CKR(ensure_run_buffers(ctx, runs + 16));
-            continue;
-        }
-        absorb_counters(ctx);
-        ctx->n_runs = runs;
-        CKR(check_overflow(ctx));
-        ctx->n_segments = (int64_t)ctx->h_ctr->n_segments;
-        if (out) {
-            out[0] = runs;
-            out[1] = ctx->n_events;
-            out[2] = ctx->n_event_samples;
-            out[3] = ctx->n_segments;
-        }
         return PP_OK;
-    }
-    return fail(ctx, PP_ERR_CAPACITY, "run table overflow");
+    }));
+    return commit_counters(ctx, out);
 }
 
 // ---- multi-GPU (one context per rank; pypore_b200/dist.py drives the exchange) ------------
 int pp_shard_scan(pp_ctx *ctx, double threshold, int64_t scan_len, double *dev_record)
 {
     if (!ctx || !dev_record) return PP_ERR_ARG;
-    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "the sharded path takes float32 traces");
-    CKR(set_device(ctx));
-    reset_stages(ctx);
-    CKR(record_boundary(ctx, 0));
+    CKR(require_trace(ctx, NOT_ADC, "the sharded path takes float32 traces"));
+    CKR(begin_call(ctx, 0));
     CKR(enqueue_threshold(ctx, threshold, scan_len));
-    CKR(record_boundary(ctx, ST_THRESHOLD + 1));
-    ctx->stage_ran[ST_THRESHOLD] = true;
+    CKR(end_stage(ctx, ST_THRESHOLD));
     k1_boundary_record<<<1, 32, 0, ctx->stream>>>(
         ctx->scan_len, ctx->ctr, (const int64_t *)ctx->run_start.p, (const int64_t *)ctx->run_len.p,
         (const double *)ctx->run_min.p, (const double *)ctx->run_max.p, (const unsigned char *)ctx->run_below.p,
@@ -1572,7 +1570,7 @@ int pp_shard_finish(pp_ctx *ctx, const pp_pipeline_params *p, int skip_first, in
                     int64_t ev_start, int64_t ev_len, int64_t *dev_record)
 {
     if (!ctx || !p || !dev_record) return PP_ERR_ARG;
-    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "the sharded path takes float32 traces");
+    CKR(require_trace(ctx, NOT_ADC, "the sharded path takes float32 traces"));
     if (p->filter_ncoef > 0) return fail(ctx, PP_ERR_ARG, "the sharded path does not filter");
     CKR(set_device(ctx));
     CKR(enqueue_select(ctx, p->rule_mask, p->duration_gt, p->duration_lt, p->min_gt, p->max_lt, skip_first,
@@ -1584,8 +1582,7 @@ int pp_shard_finish(pp_ctx *ctx, const pp_pipeline_params *p, int skip_first, in
                                                  (int64_t *)ctx->ev_off.p, ev_start, ev_len);
         LAUNCHED(ctx);
     }
-    CKR(record_boundary(ctx, ST_SELECT + 1));
-    ctx->stage_ran[ST_SELECT] = true;
+    CKR(end_stage(ctx, ST_SELECT));
     CKR(enqueue_split(ctx, p->min_width, p->max_width, p->window_width, p->min_gain, p->prefix_mode));
     if (p->with_stats) CKR(enqueue_stats(ctx));
     k_result_record<<<1, 32, 0, ctx->stream>>>(ctx->ctr, (long long *)dev_record);
@@ -1598,7 +1595,7 @@ int pp_shard_plan(pp_ctx *ctx, const double *dev_infos, int rank, int world, con
 {
     if (!ctx || !p || !dev_infos || !dev_plan || world < 1 || rank < 0 || rank >= world || halo_avail < 0)
         return fail(ctx, PP_ERR_ARG, "bad shard plan arguments");
-    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "the sharded path takes float32 traces");
+    CKR(require_trace(ctx, NOT_ADC, "the sharded path takes float32 traces"));
     CKR(set_device(ctx));
     k_shard_plan<<<1, 32, 0, ctx->stream>>>(dev_infos, rank, world, p->rule_mask, p->duration_gt, p->duration_lt,
                                             p->min_gt, p->max_lt, halo_avail, (long long *)dev_plan);
@@ -1609,7 +1606,7 @@ int pp_shard_plan(pp_ctx *ctx, const double *dev_infos, int rank, int world, con
 int pp_shard_finish_planned(pp_ctx *ctx, const pp_pipeline_params *p, const int64_t *dev_plan, int64_t *dev_record)
 {
     if (!ctx || !p || !dev_plan || !dev_record) return PP_ERR_ARG;
-    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "the sharded path takes float32 traces");
+    CKR(require_trace(ctx, NOT_ADC, "the sharded path takes float32 traces"));
     if (p->filter_ncoef > 0) return fail(ctx, PP_ERR_ARG, "the sharded path does not filter");
     CKR(set_device(ctx));
     CKR(enqueue_select(ctx, p->rule_mask, p->duration_gt, p->duration_lt, p->min_gt, p->max_lt, 0, 0, 0,
@@ -1618,8 +1615,7 @@ int pp_shard_finish_planned(pp_ctx *ctx, const pp_pipeline_params *p, const int6
                                                       (int64_t *)ctx->ev_off.p, ctx->cap_events,
                                                       (const long long *)dev_plan);
     LAUNCHED(ctx);
-    CKR(record_boundary(ctx, ST_SELECT + 1));
-    ctx->stage_ran[ST_SELECT] = true;
+    CKR(end_stage(ctx, ST_SELECT));
     CKR(enqueue_split(ctx, p->min_width, p->max_width, p->window_width, p->min_gain, p->prefix_mode));
     if (p->with_stats) CKR(enqueue_stats(ctx));
     k_result_record<<<1, 32, 0, ctx->stream>>>(ctx->ctr, (long long *)dev_record, (const long long *)dev_plan);
@@ -1630,7 +1626,7 @@ int pp_shard_finish_planned(pp_ctx *ctx, const pp_pipeline_params *p, const int6
 int pp_shard_commit(pp_ctx *ctx, const int64_t rec[8])
 {
     if (!ctx || !rec) return PP_ERR_ARG;
-    if (ctx->trace16) return fail(ctx, PP_ERR_STATE, "the sharded path takes float32 traces");
+    CKR(require_trace(ctx, NOT_ADC, "the sharded path takes float32 traces"));
     ctx->n_runs = rec[0];
     ctx->n_events = rec[1];
     ctx->n_event_samples = rec[2];
@@ -1771,7 +1767,7 @@ static int pipeline_host_impl(pp_ctx *ctx, const void *host, int kind, PPAdc adc
                               const pp_pipeline_params *p, const pp_host_tables *tables, int64_t out[4])
 {
     if (!ctx || !p || !host || n <= 0) return fail(ctx, PP_ERR_ARG, "bad trace");
-    const size_t elem = kind == PP_SRC_ADC16 ? sizeof(int16_t) : sizeof(float);
+    const size_t elem = sample_bytes(kind);
     CKR(set_device(ctx));
     PPHostTables H;
     memset(&H, 0, sizeof H);
@@ -1800,25 +1796,21 @@ static int pipeline_host_impl(pp_ctx *ctx, const void *host, int kind, PPAdc adc
     // every chunk pays a full split-search latency)
     if (chunk_samples <= 0) chunk_samples = (int64_t)16 << 20;
     chunk_samples = (chunk_samples + K1_TILE - 1) / K1_TILE * K1_TILE;
+    // the whole resident trace in one pass, then its rows to the host tables
+    auto whole = [&]() -> int {
+        CKR(pp_pipeline(ctx, p, out));
+        return tables ? export_tables(ctx, H, p->with_stats) : PP_OK;
+    };
     if (p->filter_ncoef > 0 || n <= chunk_samples) {
         // filtering needs every event before the split; a short trace gains nothing from chunking
         if (kind == PP_SRC_ADC16) CKR(pp_trace_upload_adc16(ctx, (const int16_t *)host, n, adc.scale, adc.offset));
         else CKR(pp_trace_upload(ctx, (const float *)host, n, 0));
-        CKR(pp_pipeline(ctx, p, out));
-        if (tables) {
-            CKR(enqueue_export(ctx, H, p->with_stats));
-            CKR(fetch_counters(ctx));
-            if (ctx->h_ctr->overflow & PP_OVF_EXPORT) return fail(ctx, PP_ERR_CAPACITY, "host tables too small");
-        }
-        return PP_OK;
+        return whole();
     }
     CKR(ensure_copy_stream(ctx));
     CKR(ensure(ctx, ctx->trace_buf, elem * (size_t)n));
-    point_trace(ctx, ctx->trace_buf.p, elem);
+    set_trace(ctx, ctx->trace_buf.p, kind, n, (int64_t)(ctx->trace_buf.cap / elem));
     ctx->adc = adc;
-    ctx->n = n;
-    ctx->trace_cap = (int64_t)(ctx->trace_buf.cap / elem);
-    ctx->adopted = false;
     ctx->src_kind = kind;
     ctx->flat_cap = n;
     reset_stages(ctx);
@@ -1852,26 +1844,12 @@ static int pipeline_host_impl(pp_ctx *ctx, const void *host, int kind, PPAdc adc
     const int64_t runs = (int64_t)ctx->h_ctr->n_runs;
     if (runs > ctx->cap_runs) {  // rare: noisy trace with many crossings; the trace is resident now, redo it whole
         CKR(ensure_run_buffers(ctx, runs + 16));
-        CKR(pp_pipeline(ctx, p, out));
-        if (tables) {
-            CKR(enqueue_export(ctx, H, p->with_stats));
-            CKR(fetch_counters(ctx));
-            if (ctx->h_ctr->overflow & PP_OVF_EXPORT) return fail(ctx, PP_ERR_CAPACITY, "host tables too small");
-        }
-        return PP_OK;
+        return whole();
     }
-    absorb_counters(ctx);
     ctx->n_runs = runs;
     ctx->prefix_valid = true;
-    CKR(check_overflow(ctx));
-    ctx->n_segments = (int64_t)ctx->h_ctr->n_segments;
+    CKR(commit_counters(ctx, out));
     ctx->stats_valid = p->with_stats != 0;
-    if (out) {
-        out[0] = runs;
-        out[1] = ctx->n_events;
-        out[2] = ctx->n_event_samples;
-        out[3] = ctx->n_segments;
-    }
     if (ctx->h_ctr->overflow & PP_OVF_EXPORT) return fail(ctx, PP_ERR_CAPACITY, "host tables too small");
     return PP_OK;
 }
@@ -1910,8 +1888,8 @@ static int hmm_upload_model(pp_ctx *ctx, const pp_hmm *m)
     if (!m->mean || !m->inv_std || !m->log_norm || !m->log_start || !m->log_trans)
         return fail(ctx, PP_ERR_ARG, "incomplete model");
     const size_t W = hmm_model_words(S);
-    double *blk = (double *)malloc(sizeof(double) * W);
-    if (!blk) return fail(ctx, PP_ERR_ARG, "out of host memory");
+    std::vector<double> blk;
+    CKR(host_scratch(ctx, blk, W));
     for (int j = 0; j < S; ++j) {
         blk[j] = m->mean[j];
         blk[S + j] = m->inv_std[j];
@@ -1919,15 +1897,11 @@ static int hmm_upload_model(pp_ctx *ctx, const pp_hmm *m)
         blk[3 * S + j] = m->log_start[j];
         blk[4 * S + j] = m->log_end ? m->log_end[j] : 0.0;
     }
-    memcpy(blk + 5 * S, m->log_trans, sizeof(double) * (size_t)S * S);
-    int rc = ensure(ctx, ctx->hmm_model, sizeof(double) * W);
-    if (rc == PP_OK) {
-        cudaError_t e = cudaMemcpyAsync(ctx->hmm_model.p, blk, sizeof(double) * W, cudaMemcpyHostToDevice, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);   // pageable block: consumed before it is freed
-        if (e != cudaSuccess) rc = fail(ctx, PP_ERR_CUDA, "model upload failed: %s", cudaGetErrorString(e));
-    }
-    free(blk);
-    return rc;
+    memcpy(blk.data() + 5 * S, m->log_trans, sizeof(double) * (size_t)S * S);
+    CKR(ensure(ctx, ctx->hmm_model, sizeof(double) * W));
+    CK(cudaMemcpyAsync(ctx->hmm_model.p, blk.data(), sizeof(double) * W, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));   // pageable block: consumed before it is freed
+    return PP_OK;
 }
 
 static int hmm_grid(pp_ctx *ctx, const void *kernel, int threads, size_t smem, int64_t want, int *grid)
@@ -2058,28 +2032,24 @@ int pp_hmm_decode_sequences(pp_ctx *ctx, const pp_hmm *model, int algorithm, con
     if (!ctx) return PP_ERR_ARG;
     if (algorithm != 0 && algorithm != 1) return fail(ctx, PP_ERR_ARG, "algorithm must be 0 (Viterbi) or 1 (forward)");
     if (n < 0 || (n > 0 && (!x || !len))) return fail(ctx, PP_ERR_ARG, "bad sequences");
-    int64_t *off = (int64_t *)malloc(sizeof(int64_t) * (size_t)(n + 1));
-    if (!off) return fail(ctx, PP_ERR_ARG, "out of host memory");
+    std::vector<int64_t> off;
+    CKR(host_scratch(ctx, off, (size_t)(n + 1)));
     off[0] = 0;
     for (int64_t k = 0; k < n; ++k) {
-        if (len[k] <= 0) { free(off); return fail(ctx, PP_ERR_ARG, "sequence %lld is empty", (long long)k); }
+        if (len[k] <= 0) return fail(ctx, PP_ERR_ARG, "sequence %lld is empty", (long long)k);
         off[k + 1] = off[k] + len[k];
     }
     const int64_t total = off[n];
-    auto run = [&]() -> int {
-        CKR(set_device(ctx));
-        CKR(hmm_upload_model(ctx, model));
-        CKR(ensure(ctx, ctx->hmm_off, sizeof(int64_t) * (size_t)(n + 1)));
-        CKR(ensure(ctx, ctx->hmm_x, sizeof(double) * (size_t)(total > 0 ? total : 1)));
-        CK(cudaMemcpyAsync(ctx->hmm_off.p, off, sizeof(int64_t) * (size_t)(n + 1), cudaMemcpyHostToDevice, ctx->stream));
-        if (total) CK(cudaMemcpyAsync(ctx->hmm_x.p, x, sizeof(double) * (size_t)total, cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));   // pageable host memory: consumed before the call returns
-        return hmm_enqueue_decode(ctx, model->n_states, algorithm, (const double *)ctx->hmm_x.p,
-                                  (const int64_t *)ctx->hmm_off.p, n, total);
-    };
-    const int rc = run();
-    free(off);
-    return rc;
+    CKR(set_device(ctx));
+    CKR(hmm_upload_model(ctx, model));
+    CKR(ensure(ctx, ctx->hmm_off, sizeof(int64_t) * (size_t)(n + 1)));
+    CKR(ensure(ctx, ctx->hmm_x, sizeof(double) * (size_t)(total > 0 ? total : 1)));
+    CK(cudaMemcpyAsync(ctx->hmm_off.p, off.data(), sizeof(int64_t) * (size_t)(n + 1), cudaMemcpyHostToDevice,
+                       ctx->stream));
+    if (total) CK(cudaMemcpyAsync(ctx->hmm_x.p, x, sizeof(double) * (size_t)total, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));   // pageable host memory: consumed before the call returns
+    return hmm_enqueue_decode(ctx, model->n_states, algorithm, (const double *)ctx->hmm_x.p,
+                              (const int64_t *)ctx->hmm_off.p, n, total);
 }
 
 int pp_hmm_download(pp_ctx *ctx, int64_t cap_seq, double *log_prob, int64_t cap_states, int32_t *state)
