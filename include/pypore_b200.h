@@ -337,10 +337,13 @@ int pp_hmm_download(pp_ctx *ctx, int64_t cap_seq, double *log_prob, int64_t cap_
  * pp_pack_tables: the tables as 8-byte words in one device buffer for ONE all-gather: event rows {global start,
  *   length} (2 words), then segment rows of 4 words {global event id | event-relative start << 32, mean, std,
  *   min | max << 32 as float32 bit patterns} -- 32 B instead of the table's 56: `end` is the next row's start (or
- *   the event's length) and is rebuilt after the gather, and the sharded path works on float32 traces, whose
- *   extrema are float32 values.  2 E + 4 S words.  Counts and the global event-id base are read on the DEVICE
- *   from the all-gathered result records (8 words per rank), so the call needs no host knowledge of them;
- *   nothing is written if cap_words is too small.
+ *   the event's length) and is rebuilt after the gather, and min / max are stored as float32.  That is exact only
+ *   when the segment table was computed from a float32 trace's own samples: PP_ERR_STATE otherwise (a float64 or
+ *   int16 ADC trace, filtered events, events from pp_events_upload_f64), and nothing is written.  The pp_shard_*
+ *   calls themselves take float64 traces too; their tables stay downloadable, only the packing refuses them.
+ *   2 E + 4 S words.  Counts and the global event-id base are read on the DEVICE from the all-gathered result
+ *   records (8 words per rank), so the call needs no host knowledge of them; nothing is written if cap_words is
+ *   too small.
  */
 int pp_shard_scan(pp_ctx *ctx, double threshold, int64_t scan_len, double *dev_record);
 int pp_shard_finish(pp_ctx *ctx, const pp_pipeline_params *p, int skip_first, int skip_last, int has_event,
@@ -366,9 +369,14 @@ int pp_ctl_exchange(pp_ctx *ctx, const void *dev_src, int n_words, void *dev_dst
  *   events {global start, length}, segments {global event id, start, end (int64), mean, std, min, max (float64)};
  *   E / S = the sums over the all-gathered result records (device memory).  out_is_host = 1: the arrays are
  *   page-locked host memory (pp_host_alloc) and are written by the kernel directly -- the call returns when the
- *   rows are there; 0: device memory.  PP_ERR_CAPACITY if cap_events / cap_segments rows do not suffice.
+ *   rows are there; 0: device memory.  PP_ERR_CAPACITY if cap_events / cap_segments rows do not suffice, and
+ *   PP_ERR_CAPACITY if some rank's 2 E_r + 4 S_r words exceed words_per_rank (its rows would be read from the
+ *   next rank's row, or past the buffer); PP_ERR_ARG for an odd words_per_rank, world outside 1..64 or an empty
+ *   rank range.  Nothing is written when the call refuses.
  *   cuda_stream != NULL: the kernel is only enqueued on that stream (the caller synchronises with it; the copy-out
- *   of one step's tables then overlaps the upload of the next step's trace -- opposite PCIe directions). */
+ *   of one step's tables then overlaps the upload of the next step's trace -- opposite PCIe directions).  The two
+ *   capacity refusals are then not reported, since the call does not wait for the kernel: it writes nothing, and
+ *   the caller sizes the tables and words_per_rank from the records. */
 typedef struct pp_unpacked_tables {
     int64_t cap_events, cap_segments;
     int64_t *ev_start, *ev_len;

@@ -1646,6 +1646,9 @@ int pp_pack_tables(pp_ctx *ctx, const int64_t *dev_records, int rank, int64_t sa
                    int64_t cap_words)
 {
     if (!ctx || !dev_out || !dev_records || rank < 0) return PP_ERR_ARG;
+    // min / max travel as float32: exact only for segments of a float32 trace's own samples
+    if (ctx->src_kind != PP_SRC_TRACE32)
+        return fail(ctx, PP_ERR_STATE, "packed tables hold float32 extrema; the segments are not of a float32 trace");
     CKR(set_device(ctx));
     k_pack_tables<<<ctx->sm_count * 4, 256, 0, ctx->stream>>>(
         (const long long *)dev_records, rank, cap_words, sample_offset, (const int64_t *)ctx->ev_start.p,
@@ -1755,6 +1758,7 @@ int pp_unpack_tables_range(pp_ctx *ctx, const int64_t *dev_gathered, int world, 
     CK(cudaMemcpyAsync(&flag, ctx->unpack_flag.p, sizeof flag, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));   // the rows are in the caller's memory when this returns
     if (flag & 1u) return fail(ctx, PP_ERR_CAPACITY, "unpack tables too small");
+    if (flag & 2u) return fail(ctx, PP_ERR_CAPACITY, "a rank's packed tables are longer than words_per_rank");
     return PP_OK;
 }
 

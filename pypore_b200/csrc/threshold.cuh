@@ -812,8 +812,9 @@ __global__ void k_result_record(const PPCounters *ctr, long long *__restrict__ r
 // n_events rows {global start, length}, then n_segments rows of PP_SEG_WORDS words
 //   { global event id (low 32 bits) | event-relative start (high 32 bits),  mean,  std,  min | max as float32 }
 // -- 32 B instead of the table's 56: `end` is the next row's start (or the event's length) and is rebuilt
-// after the gather, the sharded path works on float32 traces so min / max are float32 values, and an event
-// is shorter than 2^31 samples.  Counts and the global event-id base come from the all-gathered result
+// after the gather, min / max are float32 values because the segments are of a float32 trace's own samples
+// (pp_pack_tables refuses float64 and int16 ADC traces, filtered events and uploaded float64 events), and an
+// event is shorter than 2^31 samples.  Counts and the global event-id base come from the all-gathered result
 // records in DEVICE memory (rec_all[r] = rank r's k_result_record), so the host does not have to know them yet.
 constexpr int PP_SEG_WORDS = 4;
 
@@ -869,16 +870,25 @@ k_unpack_tables(const long long *__restrict__ g, int world, int64_t m, const lon
                 int rank_lo, int rank_hi, PPUnpacked O, unsigned *__restrict__ status)
 {
     __shared__ long long e_base[PP_MAX_WORLD + 1], s_base[PP_MAX_WORLD + 1];
+    __shared__ bool too_long;
     if (threadIdx.x == 0) {
         long long e = 0, sg = 0;
+        bool over = false;
         for (int r = 0; r < world; ++r) {
             e_base[r] = e; s_base[r] = sg;
-            e += rec_all[8 * r + 1];
-            sg += rec_all[8 * r + 3];
+            const long long ne = rec_all[8 * r + 1], ns = rec_all[8 * r + 3];
+            over = over || 2 * ne + PP_SEG_WORDS * ns > m;   // rank r's rows would run into rank r + 1's
+            e += ne;
+            sg += ns;
         }
         e_base[world] = e; s_base[world] = sg;
+        too_long = over;
     }
     __syncthreads();
+    if (too_long) {
+        if (blockIdx.x == 0 && threadIdx.x == 0) atomicOr(status, 2u);
+        return;
+    }
     // rows of the ranks [rank_lo, rank_hi) only, written from index 0 (event ids and starts stay global)
     const long long E0 = e_base[rank_lo], S0 = s_base[rank_lo];
     const long long E = e_base[rank_hi], S = s_base[rank_hi];
