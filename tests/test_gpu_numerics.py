@@ -308,8 +308,9 @@ def join(contents):
 
 
 def stat_batches(make, rng):
-    """The rows of STAT_LENGTHS alone (G = 32 lanes per row: total / rows >= 512), and shuffled among 1000 rows of
-    9 samples (G = 8), so that the rows longer than 65,536 samples share warps with short ones."""
+    """The rows of STAT_LENGTHS alone (a table averaging >= 512 samples per row), and shuffled among 1000 rows of
+    9 samples, so that the rows longer than 65,536 samples share warps with short ones.  Either way a row of fewer
+    than 512 samples is summed by 8 lanes and a longer one by 32."""
     rows = [make(n, rng) for n in STAT_LENGTHS]
     wide = join(rows)
     mixed = rows + [make(9, rng) for _ in range(1000)]

@@ -2,7 +2,11 @@
 pipeline and the oracle, on traces that are longer than one chunk: long events spanning several chunks, crossings and
 non-finite samples on chunk boundaries, every rule shape, every split option, both sample sources, the run-table
 overflow redo and HMM merges after a streamed export.  The cases are built in tests/streamed_cases.py;
-tests/test_streamed_cases_cpu.py checks that each one reaches what it was built for."""
+tests/test_streamed_cases_cpu.py checks that each one reaches what it was built for.
+
+The segment columns are compared bit for bit because every stage computes a row from that row's samples alone: a
+chunk's launches cover other rows than one launch over the whole table, but K4 picks a row's passes and group width
+from the row's own length (tests/test_gpu_rows.py checks this on order-sensitive data)."""
 import numpy as np
 import pytest
 
